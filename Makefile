@@ -16,7 +16,7 @@ $(LIB): $(wildcard $(CSRC)/*.cu $(CSRC)/*.cuh $(CSRC)/*.h) include/wafer_b200.h 
 	@grep -E "error|warning" $(CSRC)/ptxas.log | grep -v "ptxas info" || true
 
 # the reference's driver (main.rs / grid.rs run+solve) over the C ABI; host C++ only
-$(BIN): $(CSRC)/host/wafer_main.cpp $(CSRC)/host/config.hpp include/wafer_b200.h $(LIB)
+$(BIN): $(CSRC)/host/wafer_main.cpp $(CSRC)/host/config.hpp $(CSRC)/host/formats.hpp include/wafer_b200.h $(LIB)
 	/usr/bin/g++ -O2 -std=c++17 -Wall -Wextra -o $@ $(CSRC)/host/wafer_main.cpp -Lwafer_b200 -lwafer_b200 -Wl,-rpath,'$$ORIGIN' -lpthread
 
 oracle:

@@ -14,6 +14,12 @@ step, the host->device copy of psi before evolve, one observables check (grid.rs
 of the evolved psi after it (what a stateless drop-in of the reference's loop body has to do).  `parity` compares
 the measured path bit-for-bit with an independent path of the same library (N = 1: the one-step register-queue
 kernel; N > 1: a single-GPU run of the whole lattice) through wafer_phi_checksum.  Prints ONE JSON line on rank 0.
+
+  python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR
+
+also writes DIR/phi.npy: psi as the last timed step left it, sampled at a fixed set of work sites (see dump_outputs).
+The inputs are generated on the device from the arguments alone, so two builds run with the same arguments can be
+compared output for output.
 """
 import argparse
 import json
@@ -53,8 +59,14 @@ def parse_args():
     ap.add_argument("--cpu-grid", type=int, default=512, help="edge of the CPU sample lattice when the full one does not fit")
     ap.add_argument("--cpu-lattice", default="auto", choices=["auto", "sample"],
                     help="reference arm: auto = the workload's own lattice when 1.5x its five fields fit in free host memory")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="single GPU: after the timed steps write DIR/phi.npy, a fixed float64 sample of the evolved psi")
     a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     world = int(os.environ.get("WORLD_SIZE", "1")) if a.impl == "b200" else max(a.gpus, 1)
+    if a.dump_outputs and (a.impl != "b200" or world > 1):
+        ap.error("--dump-outputs needs the B200 arm on a single GPU")
     if a.workload == "C5":
         a.grid = a.grid or 2048
         a.nx = a.nx or 256 * world
@@ -242,6 +254,29 @@ def measure(lat, args, nsites, dist, steps, warmup, sampler=None):
     return glups, ms, launches, clocks
 
 
+DUMP_SITES = 1 << 22  # 32 MB of float64
+DUMP_SEED = 0
+
+
+def dump_outputs(lat, out_dir):
+    """Writes out_dir/phi.npy: the float64 values of psi (what get_phi hands a caller of evolve) at DUMP_SITES work
+    sites drawn without replacement with seed DUMP_SEED, in C order of the work area (every site when there are
+    fewer).  The sites depend only on the lattice shape, so dumps of two builds line up value for value."""
+    import numpy as np
+    nx, ny, nz = lat.size
+    e = lat.ext
+    total = nx * ny * nz
+    if total <= DUMP_SITES:
+        idx = np.arange(total)
+    else:
+        idx = np.sort(np.random.default_rng(DUMP_SEED).choice(total, DUMP_SITES, replace=False))
+    x, yz = np.divmod(idx, ny * nz)
+    y, z = np.divmod(yz, nz)
+    phi = lat.get_phi()[x + e, y + e, z + e]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "phi.npy"), phi)
+
+
 def hbm_peak():
     try:
         with open(os.path.join(ROOT, "MEASURED_PEAKS.json")) as f:
@@ -417,6 +452,8 @@ def b200_main(args):
 
     sampler = ClockSampler(local_rank) if rank == 0 else None
     glups, ms, launches, clocks = measure(lat, args, nsites, dist, args.steps, args.warmup, sampler)
+    if args.dump_outputs:
+        dump_outputs(lat, args.dump_outputs)  # before the e2e legs below replace psi
     sweeps_total = args.sweeps * args.steps
 
     peak, peak_src = hbm_peak()

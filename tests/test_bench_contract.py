@@ -54,3 +54,65 @@ def test_reference_arm_other_ranks_do_nothing():
 def test_b200_arm_has_no_cpu_fallback():
     r = _run(["--gpus", "1", "--steps", "1", "--warmup", "1", "--grid", "32", "--sweeps", "2", "--no-cpu"])
     assert r.returncode != 0 and "no CUDA device" in r.stderr
+
+
+def _bench_module():
+    import importlib.util
+    spec = importlib.util.spec_from_file_location("bench", os.path.join(ROOT, "bench.py"))
+    mod = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(mod)
+    return mod
+
+
+class _PositionLattice:
+    """stands in for wafer_b200.Lattice: every padded site holds its own C-order index, the padding ring holds -1"""
+
+    def __init__(self, size, ext):
+        self.size, self.ext = size, ext
+
+    def get_phi(self):
+        import numpy as np
+        e = self.ext
+        phi = np.full(tuple(s + 2 * e for s in self.size), -1.0)
+        phi[e:-e, e:-e, e:-e] = np.arange(np.prod(self.size), dtype=np.float64).reshape(self.size)
+        return phi
+
+
+def test_dump_outputs_samples_fixed_work_sites(tmp_path):
+    import numpy as np
+    bench = _bench_module()
+    lat = _PositionLattice((160, 170, 180), 2)  # more work sites than DUMP_SITES: a sample
+    bench.dump_outputs(lat, str(tmp_path / "a"))
+    bench.dump_outputs(lat, str(tmp_path / "b"))
+    got = np.load(tmp_path / "a" / "phi.npy")
+    assert got.dtype == np.float64 and got.shape == (bench.DUMP_SITES,) and got.nbytes <= 64 << 20
+    assert np.array_equal(got, np.load(tmp_path / "b" / "phi.npy"))
+    assert got.min() >= 0 and (np.diff(got) > 0).all()  # distinct work sites, never the ring, in C order
+    small = _PositionLattice((5, 6, 7), 1)  # fewer work sites than DUMP_SITES: all of them
+    bench.dump_outputs(small, str(tmp_path / "c"))
+    assert np.array_equal(np.load(tmp_path / "c" / "phi.npy"), np.arange(5 * 6 * 7))
+    for bad in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", str(tmp_path)]):
+        r = _run(bad)
+        assert r.returncode == 2 and not os.path.exists(tmp_path / "phi.npy"), bad
+
+
+@pytest.mark.gpu
+def test_dump_outputs_is_the_psi_of_the_timed_steps(tmp_path):
+    """the dump equals, bit for bit, psi of a direct run of the same workload: warmup + steps evolve calls"""
+    import numpy as np
+
+    import wafer_b200
+    n, sweeps, steps, warmup = 24, 3, 2, 1
+    r = _run(["--gpus", "1", "--grid", str(n), "--sweeps", str(sweeps), "--steps", str(steps), "--warmup", str(warmup),
+              "--no-e2e", "--no-cpu", "--no-512", "--no-parity", "--dump-outputs", str(tmp_path)])
+    assert r.returncode == 0, r.stderr[-2000:]
+    assert json.loads([l for l in r.stdout.splitlines() if l.startswith("{")][0])["steps"] == steps
+    dn = 10.24 / n
+    with wafer_b200.Lattice((n, n, n), dn=dn, dt=0.3 * dn * dn, mass=1.0) as lat:
+        lat.generate_potential("PoschlTeller")
+        lat.set_initial_conditions("Boolean")
+        lat.check(0)
+        for _ in range(warmup + steps):
+            lat.evolve(0, sweeps)
+        want = lat.get_phi()[1:-1, 1:-1, 1:-1].ravel()
+    assert np.array_equal(np.load(tmp_path / "phi.npy"), want)
