@@ -187,8 +187,14 @@ def test_division_by_invariant(wb):
                 assert lat.selftest_division(den, 1 << 24, seed) == 0, den
 
 
+# tile edges of sweep_tb.cuh (TY = 30, TZ = 60): the tile at y0 = 30, z0 = 60 takes the unmasked path from ny = 61, nz = 122
+TB2_EDGES = [(13, ny, nz) for ny in (60, 61) for nz in (121, 122)]
+DEGENERATE = [(1, 40, 70), (20, 1, 70), (20, 40, 1)]
+
+
 @pytest.mark.parametrize("steps", [1, 2, 3, 4, 7, 10])
-@pytest.mark.parametrize("shape", [(12, 9, 10), (50, 37, 21), (33, 64, 130), (70, 61, 121), (7, 3, 2), (131, 31, 59)])
+@pytest.mark.parametrize("shape", [(12, 9, 10), (50, 37, 21), (33, 64, 130), (70, 61, 121), (7, 3, 2), (131, 31, 59)]
+                         + TB2_EDGES + DEGENERATE)
 def test_time_tiled_sweep_bitwise(wb, oracle, shape, steps):
     """ThreePoint ground state uses the two-steps-per-pass TMA kernel (+ one plain sweep when steps is odd)."""
     g, v, phi = _rand_state(oracle, shape, 1, 29)
@@ -245,9 +251,13 @@ def test_time_tiled_sweep_with_zeros_and_denormals(wb, oracle):
     assert np.array_equal(np.signbit(got), np.signbit(phi))  # signed zeros too
 
 
+# tile edges of sweep_tma1.cuh: TY = 32; TZ = 60 / 60 / 56 for ext 1 / 2 / 3
+TMA1_EDGES = [((9, ny, nz), 3) for ny in (32, 33) for nz in (55, 56, 57, 60, 61)]
+
+
 @pytest.mark.parametrize("ext", [1, 2, 3])
 @pytest.mark.parametrize("shape,steps", [((12, 9, 10), 3), ((50, 37, 21), 4), ((33, 64, 130), 2), ((70, 61, 121), 5),
-                                         ((7, 3, 2), 3), ((131, 31, 59), 2)])
+                                         ((7, 3, 2), 3), ((131, 31, 59), 2)] + TMA1_EDGES + [(s, 3) for s in DEGENERATE])
 def test_tma_one_step_sweep_bitwise(wb, oracle, ext, shape, steps):
     """WAFER_FLAG_TMA_ONE_STEP (8), with the time-tiled kernel switched off (4): every step goes through sweep_tma1."""
     g, v, phi = _rand_state(oracle, shape, ext, 51 + ext)
@@ -342,14 +352,15 @@ def test_sweep_bitwise_256_and_launch_count(wb, oracle):
 
 
 # ---------------------------------------------------------------------------------------------- observables / reductions
+@pytest.mark.parametrize("flags", [0, 1, 4, 12])  # default, A/B arrays, register-queue sweep, TMA one-step only
 @pytest.mark.parametrize("ext", [1, 2, 3])
 @pytest.mark.parametrize("shape", [(9, 11, 10), (40, 33, 70)])
-def test_observables(wb, oracle, ext, shape):
+def test_observables(wb, oracle, ext, shape, flags):
     g, v, phi = _rand_state(oracle, shape, ext, 11, dn=0.1, mass=0.7)
     ps = np.random.default_rng(5).uniform(0.5, 2.0, size=shape)
     oracle.set_sum_mode(1)
     try:
-        with wb.Lattice(shape, CD[ext], dn=g.dn, dt=g.dt, mass=g.mass) as lat:
+        with wb.Lattice(shape, CD[ext], dn=g.dn, dt=g.dt, mass=g.mass, flags=flags) as lat:
             lat.set_potential(v)
             lat.set_phi(phi)
             for potsub in (None, 2.5, ps, -1.0):
@@ -375,7 +386,7 @@ def test_normalise_is_a_true_division(wb, oracle):
     assert np.array_equal(got, phi)
 
 
-def test_orthogonalise_modified_gram_schmidt(wb, oracle):
+def test_orthogonalise_modified_gram_schmidt(wb, oracle, flags=0):
     rng = np.random.default_rng(17)
     shape, ext = (14, 12, 18), 1
     g = oracle.make_grid(*shape, ext=ext)
@@ -388,7 +399,7 @@ def test_orthogonalise_modified_gram_schmidt(wb, oracle):
     npr.work(phi, ext)[...] = rng.normal(size=shape)
     oracle.set_sum_mode(1)
     try:
-        with wb.Lattice(shape) as lat:
+        with wb.Lattice(shape, flags=flags) as lat:
             for q in lowers:
                 lat.push_lower(q)
             for wnum in (1, 2, 3, 7):  # 7 > stored: take(wnum) clamps (grid.rs:478)
@@ -400,9 +411,15 @@ def test_orthogonalise_modified_gram_schmidt(wb, oracle):
     finally:
         oracle.set_sum_mode(0)
 
+@pytest.mark.parametrize("flags", [1, 4, 12])  # A/B arrays, register-queue sweep, TMA one-step only
+def test_orthogonalise_modified_gram_schmidt_under_other_flags(wb, oracle, flags):
+    test_orthogonalise_modified_gram_schmidt(wb, oracle, flags)
 
+
+@pytest.mark.parametrize("flags", [0, 1, 4, 12])  # default, A/B arrays, register-queue sweep, TMA one-step only
+@pytest.mark.parametrize("steps", [1, 2, 6, 7, 8, 9, 16])  # from 8 steps on, pairs of steps replay a CUDA graph
 @pytest.mark.parametrize("ext,nlow", [(1, 1), (1, 3), (2, 2), (3, 1)])
-def test_evolve_excited_state_steps(wb, oracle, ext, nlow):
+def test_evolve_excited_state_steps(wb, oracle, ext, nlow, steps, flags):
     """grid.rs:674-681: every step norm2 -> normalise -> MGS against the stored states"""
     rng = np.random.default_rng(19 + nlow)
     shape = (18, 16, 22)
@@ -419,14 +436,14 @@ def test_evolve_excited_state_steps(wb, oracle, ext, nlow):
     npr.work(phi, ext)[...] = rng.normal(size=shape)
     oracle.set_sum_mode(1)
     try:
-        with wb.Lattice(shape, CD[ext], dn=g.dn, dt=g.dt, mass=g.mass) as lat:
+        with wb.Lattice(shape, CD[ext], dn=g.dn, dt=g.dt, mass=g.mass, flags=flags) as lat:
             lat.set_potential(v)
             for q in lowers:
                 lat.push_lower(q)
             lat.set_phi(phi)
-            lat.evolve(nlow, 6)
+            lat.evolve(nlow, steps)
             got = lat.get_phi()
-        oracle.evolve(g, phi, a, b, 6, lowers=lowers)
+        oracle.evolve(g, phi, a, b, steps, lowers=lowers)
     finally:
         oracle.set_sum_mode(0)
     assert _l2(got, phi) < 1e-12
@@ -434,8 +451,33 @@ def test_evolve_excited_state_steps(wb, oracle, ext, nlow):
         assert abs((q * got).sum()) < 1e-13
 
 
+@pytest.mark.parametrize("flags", [0, 1, 4, 12])
+@pytest.mark.parametrize("steps", [1, 8, 9])
+def test_evolve_excited_with_an_empty_store_still_normalises(wb, oracle, steps, flags):
+    """grid.rs:674: wnum > 0 normalises after every step even when w_store is empty (from 8 steps on through the
+    graph of the wnum = 0 step pair)"""
+    g, v, phi = _rand_state(oracle, (18, 16, 22), 1, 71, dn=0.1, dt=2e-3, mass=1.0)
+    a, b = oracle.build_ab(v, g.dt)
+    oracle.set_sum_mode(1)
+    try:
+        with wb.Lattice(g.work_shape, dn=g.dn, dt=g.dt, mass=g.mass, flags=flags) as lat:
+            lat.set_potential(v)
+            lat.set_phi(phi)
+            lat.evolve(1, steps)
+            assert lat.num_lowers == 0
+            got = lat.get_phi()
+        for _ in range(steps):
+            oracle.evolve(g, phi, a, b, 1)
+            oracle.normalise(phi, oracle.norm2_flat(phi))
+    finally:
+        oracle.set_sum_mode(0)
+    assert _l2(got, phi) < 1e-12
+    assert abs((got * got).sum() - 1.0) < 1e-12
+
+
+@pytest.mark.parametrize("flags", [0, 1, 4, 12])  # default, A/B arrays, register-queue sweep, TMA one-step only
 @pytest.mark.parametrize("nlow", [5, 6])
-def test_evolve_excited_more_states_than_one_pass_takes(wb, oracle, nlow):
+def test_evolve_excited_more_states_than_one_pass_takes(wb, oracle, nlow, flags):
     """more stored states than the sweep fuses (4) / than one projection pass handles (4): the remaining overlaps come
     from extra dot passes; the stored states are deliberately NOT orthogonal, so the Gram-matrix solve of the
     modified-Gram-Schmidt coefficients (kernels.cuh gs_coeff_kernel) is exercised for real"""
@@ -453,7 +495,7 @@ def test_evolve_excited_more_states_than_one_pass_takes(wb, oracle, nlow):
     npr.work(phi, ext)[...] = rng.normal(size=shape)
     oracle.set_sum_mode(1)
     try:
-        with wb.Lattice(shape, CD[ext], dn=g.dn, dt=g.dt, mass=g.mass) as lat:
+        with wb.Lattice(shape, CD[ext], dn=g.dn, dt=g.dt, mass=g.mass, flags=flags) as lat:
             lat.set_potential(v)
             for q in lowers:
                 lat.push_lower(q)
@@ -502,7 +544,7 @@ def test_check_sums_fused_into_the_last_sweep(wb, oracle, ext, potsub):
             assert abs(got[key] - want[key]) <= SUM_TOL * scale, (key, got[key], want[key])
 
 
-def test_check_fuses_observables_normalise_orthogonalise(wb, oracle):
+def test_check_fuses_observables_normalise_orthogonalise(wb, oracle, flags=0):
     """grid.rs:127-135"""
     g, v, phi = _rand_state(oracle, (16, 16, 16), 1, 23, dn=0.1, mass=1.0)
     q = np.zeros(g.padded_shape)
@@ -510,7 +552,7 @@ def test_check_fuses_observables_normalise_orthogonalise(wb, oracle):
     q /= np.sqrt((q * q).sum())
     oracle.set_sum_mode(1)
     try:
-        with wb.Lattice((16, 16, 16), dn=g.dn, dt=g.dt, mass=g.mass) as lat:
+        with wb.Lattice((16, 16, 16), dn=g.dn, dt=g.dt, mass=g.mass, flags=flags) as lat:
             lat.set_potential(v)
             lat.push_lower(q)
             lat.set_phi(phi)
@@ -524,6 +566,10 @@ def test_check_fuses_observables_normalise_orthogonalise(wb, oracle):
     for key in ref:
         assert abs(got[key] - ref[key]) <= SUM_TOL * max(abs(ref["energy"]), ref["norm2"])
     assert _l2(after, phi) < 1e-13
+
+@pytest.mark.parametrize("flags", [1, 4, 12])  # A/B arrays, register-queue sweep, TMA one-step only
+def test_check_fuses_observables_normalise_orthogonalise_under_other_flags(wb, oracle, flags):
+    test_check_fuses_observables_normalise_orthogonalise(wb, oracle, flags)
 
 
 # ---------------------------------------------------------------------------------------------- generators
@@ -629,12 +675,12 @@ def test_excited_state_seed_matches_restatement(wb, oracle):
         assert np.array_equal(lat.get_phi(), oracle.seed_from_state(g, q))
 
 
-def test_max_steps_and_snapshot_semantics(wb, oracle):
+def test_max_steps_and_snapshot_semantics(wb, oracle, flags=0):
     g = oracle.make_grid(8, 8, 8, ext=1, dn=0.1, dt=1e-3, mass=1.0)
     v = oracle.potential(g, "Harmonic")
     a, b = oracle.build_ab(v, g.dt)
     phi = oracle.initial_condition(g, "Boolean")
-    with wb.Lattice((8, 8, 8), dn=0.1, dt=1e-3, mass=1.0) as lat:
+    with wb.Lattice((8, 8, 8), dn=0.1, dt=1e-3, mass=1.0, flags=flags) as lat:
         lat.set_potential(v)
         lat.set_phi(phi)
         conv, rec = lat.solve(0, 1e-300, max_steps=25, screen_update=10)
@@ -647,6 +693,10 @@ def test_max_steps_and_snapshot_semantics(wb, oracle):
         lat.solve(0, float("inf"), screen_update=5, snap_update=5)
         oracle.solve(g, v, a, b, p1, tolerance=float("inf"), screen_update=5, snap_update=5)
         assert _l2(lat.get_phi(), p1) < 1e-14
+
+@pytest.mark.parametrize("flags", [1, 4, 12])  # A/B arrays, register-queue sweep, TMA one-step only
+def test_max_steps_and_snapshot_semantics_under_other_flags(wb, oracle, flags):
+    test_max_steps_and_snapshot_semantics(wb, oracle, flags)
 
 
 # ---------------------------------------------------------------------------------------------- BASELINE full sizes: size-independent properties

@@ -264,7 +264,7 @@ int init_tb(wafer_ctx* ctx) {
 //   * x is cut into chunks of at most 512 planes; per chunk, whole tile columns in tile order form the BULK list that the
 //     CTAs drain through an atomic counter (in-order dispatch keeps neighbouring tiles close in time);
 //   * of the last chunk, the ntiles % G columns that would leave most SMs idle in a last partial wave are cut along x
-//     into G equal shares (even lengths, no stubs shorter than 6 planes): the static TAIL of each CTA.
+//     into at most G equal shares (even lengths, no stubs shorter than 6 planes): the static TAIL of each CTA.
 // 512^3 on 148 SMs: one round of 148 columns + 14 columns cut 148 ways = 516 + ~53 plane-iterations per SM, against
 // 10 waves x 60 for round 1's uniform grid of 162 tiles x 9 chunks.  Measured (gpurun_out/r2f..r2j,
 // profiles/r2_tb2_variants.md): statically assigned rounds +4.8 % at 512^3 and +6 % on a 128-plane slab but -6 % at
@@ -283,10 +283,13 @@ Tb2Plan tb2_plan(int ny, int nz, int xb, int xe, int slots, const std::string& m
     auto seg = [&](int tile, int a, int b) { return tb::Segment{(tile / ntz) * tb::TY, (tile % ntz) * tb::TZ, a, b}; };
     const int MINSEG = 6;
     int G = (int)std::max<long long>(1, std::min<long long>(slots, ((long long)ntiles * P + 7) / 8));
-    // shares of `cols` tile columns starting at tile `t0`, planes [ca, cz), cut into G equal runs -> per[k]
+    // shares of `cols` tile columns starting at tile `t0`, planes [ca, cz), cut into equal runs -> per[k].  At most
+    // Ur / MINSEG shares: a thin slab of a wide plane leaves less than MINSEG planes per CTA, and cutting it G ways would
+    // give stubs of 2-4 planes that are mostly pipeline fill; the CTAs past the last share get no tail.
     auto cut_static = [&](int t0, int cols, int ca, int cz) {
         const int Pc = cz - ca;
         const long long Ur = (long long)cols * Pc;
+        const int S = (int)std::max<long long>(1, std::min<long long>(G, Ur / MINSEG));
         auto snap = [&](long long u) {
             const long long p = u % Pc;
             if (p == 0) return u;
@@ -294,9 +297,9 @@ Tb2Plan tb2_plan(int ny, int nz, int xb, int xe, int slots, const std::string& m
             if (Pc - p < MINSEG) return u + (Pc - p);
             return u - (p & 1);
         };
-        for (int k = 0; k < G && Ur > 0; ++k) {
-            long long u = snap(k * Ur / G);
-            const long long ue = k + 1 == G ? Ur : snap((k + 1) * Ur / G);
+        for (int k = 0; k < S && Ur > 0; ++k) {
+            long long u = snap(k * Ur / S);
+            const long long ue = k + 1 == S ? Ur : snap((k + 1) * Ur / S);
             while (u < ue) {
                 const int p0 = (int)(u % Pc), len = (int)std::min<long long>(Pc - p0, ue - u);
                 per[k].push_back(seg(t0 + (int)(u / Pc), ca + p0, ca + p0 + len));
