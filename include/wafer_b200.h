@@ -123,6 +123,15 @@ uint32_t wafer_num_lowers(const wafer_ctx *ctx);
 int wafer_generate_potential(wafer_ctx *ctx, int32_t kind, double sig);
 /* kind: InitialCondition index (config.rs:153-170): 2 Coulomb, 3 Constant, 4 Boolean */
 int wafer_generate_initial_condition(wafer_ctx *ctx, int32_t kind);
+/* Gaussian initial condition (config.rs:636-642) as a seeded counter-based field: every work site is N(0, sig) from
+   Philox4x32-10 keyed by `seed` at the site's global index (generators.cuh gaussian_site), so the same seed gives the
+   same bits at any world size.  sig must be finite and >= 0. */
+int wafer_generate_gaussian(wafer_ctx *ctx, double sig, uint64_t seed);
+/* symmetrise_wavefunction (config.rs:691-728) on the work area, for every ext: kind = SymmetryConstraint index
+   (config.rs:186-197) 0 NotConstrained (a no-op, no launch), 1 AboutZ, 2 AntisymAboutZ, 3 AboutY, 4 AntisymAboutY.
+   With n the work size of the mirrored axis, psi[.., n-1-t] = +-psi[.., t] for t < n/2; the middle index of an odd n
+   is kept (symmetric) or set to +0 (antisymmetric).  Exact and idempotent; needs no communication when world > 1. */
+int wafer_symmetrise(wafer_ctx *ctx, int32_t kind);
 
 /* -------- the hot path -------------------------------------------------------------------------- */
 int wafer_observables_compute(wafer_ctx *ctx, wafer_observables *out); /* compute_observables        (grid.rs:303-445) */

@@ -51,6 +51,8 @@ extern "C" {
     fn wafer_push_lower_from_phi(ctx: *mut WaferCtx) -> c_int;
     fn wafer_phi_from_lower(ctx: *mut WaferCtx, idx: u32) -> c_int;
     fn wafer_phi_seed_from_lower(ctx: *mut WaferCtx, idx: u32) -> c_int;
+    fn wafer_generate_gaussian(ctx: *mut WaferCtx, sig: f64, seed: u64) -> c_int;
+    fn wafer_symmetrise(ctx: *mut WaferCtx, kind: i32) -> c_int;
     fn wafer_check(ctx: *mut WaferCtx, wnum: u8, out: *mut WaferObservables) -> c_int;
     fn wafer_normalise(ctx: *mut WaferCtx, norm2: f64) -> c_int;
     fn wafer_evolve(ctx: *mut WaferCtx, wnum: u8, steps: u64) -> c_int;
@@ -126,6 +128,14 @@ impl Gpu {
     }
     pub fn phi_seed_from_lower(&self, idx: u32) -> Result<()> {
         self.check(unsafe { wafer_phi_seed_from_lower(self.ctx, idx) })
+    }
+    /// config.rs:636-642 on the device, keyed by `seed` instead of thread_rng: the same seed gives the same start.
+    pub fn generate_gaussian(&self, sig: R64, seed: u64) -> Result<()> {
+        self.check(unsafe { wafer_generate_gaussian(self.ctx, sig.raw(), seed) })
+    }
+    /// symmetrise_wavefunction (config.rs:691-728) for every ext: `kind` = `SymmetryConstraint as i32`.
+    pub fn symmetrise(&self, kind: i32) -> Result<()> {
+        self.check(unsafe { wafer_symmetrise(self.ctx, kind) })
     }
     pub fn check_state(&self, wnum: u8) -> Result<WaferObservables> {
         let mut o = WaferObservables::default();

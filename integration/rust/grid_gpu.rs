@@ -70,7 +70,8 @@ fn solve(config: &Config, log: &Logger, debug_level: usize, gpu: &Gpu, wnum: u8)
         let norm_energy = o.energy / o.norm2;
         let tau = r64(step as f64) * config.grid.dt;
         if config.output.snap_update.is_some() && step % config.output.snap_update.unwrap() == 0 {
-            gpu.normalise(o.norm2)?; // grid.rs:138-139 (NotConstrained)
+            gpu.symmetrise(config.init_symmetry as i32)?; // grid.rs:137-139: symmetrise, normalise, write
+            gpu.normalise(o.norm2)?;
             gpu.get_phi(&mut host_phi)?;
             let work = ::grid::get_work_area(&host_phi, config.central_difference.ext());
             if let Err(err) = output::wavefunction(&work, wnum, false, &config.project_name, &config.output.file_type) {

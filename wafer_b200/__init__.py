@@ -12,16 +12,18 @@ import numpy as np
 from . import _capi
 from ._capi import Observables, Params, Record
 
-__all__ = ["Lattice", "slab_partition", "tb2_plan", "WaferError", "POTENTIALS", "INITIAL_CONDITIONS", "EXT", "nccl_unique_id", "pinned_empty",
-           "pin", "unpin", "FLAG_AB_ARRAYS"]
+__all__ = ["Lattice", "slab_partition", "tb2_plan", "WaferError", "POTENTIALS", "INITIAL_CONDITIONS", "SYMMETRIES", "EXT",
+           "nccl_unique_id", "pinned_empty", "pin", "unpin", "FLAG_AB_ARRAYS"]
 
-# PotentialType (config.rs:74-104), InitialCondition (config.rs:153-170), CentralDifference.ext() (config.rs:232-238)
+# PotentialType (config.rs:74-104), InitialCondition (config.rs:153-170), SymmetryConstraint (config.rs:186-197),
+# CentralDifference.ext() (config.rs:232-238)
 POTENTIALS = {
     "NoPotential": 0, "Cube": 1, "QuadWell": 2, "Periodic": 3, "Coulomb": 4, "ComplexCoulomb": 5,
     "ElipticalCoulomb": 6, "SimpleCornell": 7, "FullCornell": 8, "Harmonic": 9, "ComplexHarmonic": 10,
     "Dodecahedron": 11, "FromFile": 12, "FromScript": 13, "PoschlTeller": 100,
 }
 INITIAL_CONDITIONS = {"FromFile": 0, "Gaussian": 1, "Coulomb": 2, "Constant": 3, "Boolean": 4}
+SYMMETRIES = {"NotConstrained": 0, "AboutZ": 1, "AntisymAboutZ": 2, "AboutY": 3, "AntisymAboutY": 4}
 EXT = {"ThreePoint": 1, "FivePoint": 2, "SevenPoint": 3}
 FLAG_AB_ARRAYS = 0x1
 FLAG_SIMPLE_SWEEP = 0x4
@@ -268,9 +270,20 @@ class Lattice:
         """fault injection: stall this rank's halo stream before every boundary pass (tests of the GPU-GPU ordering)"""
         self._ck(self._lib.wafer_debug_halo_delay(self._h, int(nanoseconds)))
 
-    def set_initial_conditions(self, kind):
-        """config::set_initial_conditions (config.rs:577-627) evaluated on the device."""
-        self._ck(self._lib.wafer_generate_initial_condition(self._h, INITIAL_CONDITIONS[kind]))
+    def set_initial_conditions(self, kind, sig=1.0, seed=0):
+        """config::set_initial_conditions (config.rs:577-627) evaluated on the device.  "Gaussian" is N(0, sig) at every
+        work site from a counter-based generator keyed by `seed` (wafer_generate_gaussian): reproducible, and the same
+        at any world size; sig and seed are unused by the other kinds."""
+        k = INITIAL_CONDITIONS[kind] if isinstance(kind, str) else int(kind)
+        if k == INITIAL_CONDITIONS["Gaussian"]:
+            self._ck(self._lib.wafer_generate_gaussian(self._h, float(sig), int(seed)))
+        else:
+            self._ck(self._lib.wafer_generate_initial_condition(self._h, k))
+
+    def symmetrise_wavefunction(self, kind):
+        """config::symmetrise_wavefunction (config.rs:691-728) on the device: kind is a SYMMETRIES name or index.
+        Mirrors the work area about its centre in y or z, copying the lower half (negated for the Antisym kinds)."""
+        self._ck(self._lib.wafer_symmetrise(self._h, SYMMETRIES[kind] if isinstance(kind, str) else int(kind)))
 
     def push_lower(self, q=None):
         """w_store.push(q); with q=None pushes the current phi (grid.rs:241)."""

@@ -55,6 +55,8 @@ SYMBOLS = {
     "wafer_num_lowers": (C.c_uint32, [_ctx]),
     "wafer_generate_potential": (C.c_int, [_ctx, C.c_int32, C.c_double]),
     "wafer_generate_initial_condition": (C.c_int, [_ctx, C.c_int32]),
+    "wafer_generate_gaussian": (C.c_int, [_ctx, C.c_double, C.c_uint64]),
+    "wafer_symmetrise": (C.c_int, [_ctx, C.c_int32]),
     "wafer_observables_compute": (C.c_int, [_ctx, C.POINTER(Observables)]),
     "wafer_norm2": (C.c_int, [_ctx, _dp]),
     "wafer_normalise": (C.c_int, [_ctx, C.c_double]),

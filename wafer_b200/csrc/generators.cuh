@@ -237,4 +237,101 @@ __global__ void __launch_bounds__(128) seed_from_state_kernel(double* __restrict
     }
 }
 
+// ---- init_symmetry (config.rs:186-197 SymmetryConstraint, applied at config.rs:625 and grid.rs:137-139) ----------------
+// Mirror of the work area about its centre along y (AboutY / AntisymAboutY) or z (AboutZ / AntisymAboutZ): with n the
+// work size of that axis, psi[.., n-1-t] := s * psi[.., t] for t < n/2 (s = +1 / -1); for odd n and s = -1 the middle
+// index becomes +0.  A copy and a sign flip, so the result is exact and applying it twice equals applying it once.
+// Sources (t < n/2) and destinations (t >= n - n/2) never overlap, so the update in place is race-free.  Runs over every
+// plane of the slab inside the global lattice, ghost planes included: a ghost plane gets the bits its owner computes.
+enum SymKind { SYM_NONE = 0, SYM_ABOUT_Z, SYM_ANTI_Z, SYM_ABOUT_Y, SYM_ANTI_Y };
+
+// one CTA per row; the reflected pair (t, t+1) -> (n-2-t, n-1-t) is 16-byte aligned for even nz (rows start 128-byte
+// aligned), so even rows move as double2 and odd ones element by element
+__global__ void __launch_bounds__(128) symmetrise_z_kernel(double* __restrict__ w, Geom g, double s) {
+    const long long rows = (long long)(g.L + 2 * g.gx) * g.ny;
+    const int n = g.nz, half = n / 2;
+    for (long long r = blockIdx.x; r < rows; r += gridDim.x) {
+        const int i = (int)(r / g.ny) - g.gx, j = (int)(r % g.ny);
+        const long long gi = g.x0 + i;
+        if (gi < 0 || gi >= g.gnx) continue;  // outside the lattice: zeros, and nothing maps onto them
+        double* row = w + g.off(i, j, 0);
+        if ((n & 1) == 0) {
+            double2* row2 = reinterpret_cast<double2*>(row);
+            const int pairs = half / 2;  // whole pairs below the centre
+            for (int p = threadIdx.x; p < pairs; p += blockDim.x) {
+                const double2 a = row2[p];
+                row2[n / 2 - 1 - p] = make_double2(s * a.y, s * a.x);
+            }
+            if ((half & 1) && threadIdx.x == 0) row[half] = s * row[half - 1];  // the pair straddling the centre
+        } else {
+            for (int t = threadIdx.x; t < half; t += blockDim.x) row[n - 1 - t] = s * row[t];
+            if (s < 0. && threadIdx.x == 0) row[half] = 0.0;
+        }
+    }
+}
+
+// one CTA per (plane, destination row): whole-row copies, double2 over the 128-byte aligned rows
+__global__ void __launch_bounds__(128) symmetrise_y_kernel(double* __restrict__ w, Geom g, double s) {
+    const int half = g.ny / 2, nrows = g.ny - half;  // destination rows ny-1-t for t < half, plus the middle one if odd
+    const long long rows = (long long)(g.L + 2 * g.gx) * nrows;
+    const int nz2 = g.nz / 2;
+    for (long long r = blockIdx.x; r < rows; r += gridDim.x) {
+        const int i = (int)(r / nrows) - g.gx, t = (int)(r % nrows);
+        const long long gi = g.x0 + i;
+        if (gi < 0 || gi >= g.gnx) continue;
+        double* dst = w + g.off(i, g.ny - 1 - t, 0);
+        if (t < half) {
+            const double2* src2 = reinterpret_cast<const double2*>(w + g.off(i, t, 0));
+            double2* dst2 = reinterpret_cast<double2*>(dst);
+            for (int k = threadIdx.x; k < nz2; k += blockDim.x) {
+                const double2 a = src2[k];
+                dst2[k] = make_double2(s * a.x, s * a.y);
+            }
+            if ((g.nz & 1) && threadIdx.x == 0) dst[g.nz - 1] = s * w[g.off(i, t, g.nz - 1)];  // never the pad column
+        } else if (s < 0.) {  // middle row of an odd ny
+            for (int k = threadIdx.x; k < g.nz; k += blockDim.x) dst[k] = 0.0;
+        }
+    }
+}
+
+// ---- Gaussian initial condition (config.rs:636-642) as a counter-based field ------------------------------------------
+// Philox4x32-10 (Salmon et al., SC'11; the Random123 constants), key = seed, counter = global work site index
+// s = (gi*gny + j)*gnz + k.  Box-Muller on the first two 53-bit uniforms: u1 in (0, 1], u2 in [0, 1);
+// value = sig * (sqrt(-2 log u1) * cos(2 pi u2)).  The value of a site depends on (seed, s) only: not on the slab, the
+// rank count or the launch shape, so ghost planes agree with their owners by construction.
+struct Philox4 { uint32_t v[4]; };
+
+__device__ __host__ inline Philox4 philox4x32_10(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, uint32_t k0,
+                                                 uint32_t k1) {
+    for (int r = 0; r < 10; ++r) {
+        if (r) { k0 += 0x9E3779B9u; k1 += 0xBB67AE85u; }
+        const uint64_t p0 = (uint64_t)0xD2511F53u * c0, p1 = (uint64_t)0xCD9E8D57u * c2;
+        const uint32_t n0 = (uint32_t)(p1 >> 32) ^ c1 ^ k0, n2 = (uint32_t)(p0 >> 32) ^ c3 ^ k1;
+        c0 = n0; c1 = (uint32_t)p1; c2 = n2; c3 = (uint32_t)p0;
+    }
+    return Philox4{{c0, c1, c2, c3}};
+}
+
+__device__ inline double gaussian_site(unsigned long long s, unsigned long long seed, double sig) {
+    const Philox4 r = philox4x32_10((uint32_t)s, (uint32_t)(s >> 32), 0u, 0u, (uint32_t)seed, (uint32_t)(seed >> 32));
+    const double two_m53 = 1.1102230246251565e-16;  // 2^-53
+    const double u1 = ((double)(r.v[0] >> 5) * 67108864.0 + (double)(r.v[1] >> 6) + 1.0) * two_m53;
+    const double u2 = ((double)(r.v[2] >> 5) * 67108864.0 + (double)(r.v[3] >> 6)) * two_m53;
+    return sig * (sqrt(-2.0 * log(u1)) * cos(6.283185307179586 * u2));
+}
+
+// every work site of every slab plane inside the global lattice (ghost planes included), 0 elsewhere, like gen_ic_kernel
+__global__ void __launch_bounds__(128) gen_gaussian_kernel(double* __restrict__ w, Geom g, double sig,
+                                                           unsigned long long seed) {
+    const long long rows = (long long)(g.L + 2 * g.gx) * g.ny;
+    for (long long r = blockIdx.x; r < rows; r += gridDim.x) {
+        const int i = (int)(r / g.ny) - g.gx, j = (int)(r % g.ny);
+        const long long gi = g.x0 + i;
+        double* row = w + g.off(i, j, 0);
+        const bool inside = gi >= 0 && gi < g.gnx;
+        const unsigned long long s0 = ((unsigned long long)gi * g.gny + j) * g.gnz;
+        for (int k = threadIdx.x; k < g.nz; k += blockDim.x) row[k] = inside ? gaussian_site(s0 + k, seed, sig) : 0.0;
+    }
+}
+
 }  // namespace wafer

@@ -63,6 +63,7 @@ struct Config {
     double sig = 0;
     int init_symmetry = 0;
     std::string script_location;  // set from the command line, never from YAML (config.rs:331)
+    uint64_t seed = 0;            // --seed: key of the Gaussian initial condition (the reference draws from thread_rng)
 
     int ext() const { return central_difference + 1; }
     std::string file_extension() const {  // FileType::extentsion (config.rs:280-288)
@@ -190,6 +191,10 @@ inline Config load_config(std::istream& in) {
     if (c.wavenum > c.wavemax) throw ConfigError("LargeWavenum: wavenum can not be larger than wavemax");
     if (c.nx == 0 || c.ny == 0 || c.nz == 0) throw ConfigError("Deserialize: grid.size must be positive");
     if (c.screen_update == 0) throw ConfigError("Deserialize: output.screen_update must be positive");
+    // an antisymmetric state about an axis of one site is identically zero: its first check would divide 0 by 0
+    if ((c.init_symmetry == 2 && c.nz == 1) || (c.init_symmetry == 4 && c.ny == 1))
+        throw ConfigError("init_symmetry " + symmetry_names()[c.init_symmetry] + " needs more than one site along " +
+                          (c.init_symmetry == 2 ? "z" : "y") + ": the constrained state would be zero everywhere");
     return c;
 }
 
@@ -212,7 +217,8 @@ inline std::string config_json(const Config& c) {
     o << ", \"file_type\": \"" << filetype_names()[c.file_type] << "\", \"save_wavefns\": " << (c.save_wavefns ? "true" : "false")
       << ", \"save_potential\": " << (c.save_potential ? "true" : "false") << "}, \"potential\": \""
       << potential_names()[c.potential] << "\", \"mass\": " << c.mass << ", \"init_condition\": \"" << ic_names()[c.init_condition]
-      << "\", \"sig\": " << c.sig << ", \"init_symmetry\": \"" << symmetry_names()[c.init_symmetry] << "\", \"ext\": " << c.ext() << "}";
+      << "\", \"sig\": " << c.sig << ", \"init_symmetry\": \"" << symmetry_names()[c.init_symmetry] << "\", \"ext\": " << c.ext()
+      << ", \"seed\": " << c.seed << "}";
     return o.str();
 }
 

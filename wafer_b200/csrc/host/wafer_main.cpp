@@ -7,10 +7,12 @@
 //
 //   wafer-b200 -c wafer.yaml                 run (one process per GPU; RANK / WORLD_SIZE / LOCAL_RANK select a slab)
 //   wafer-b200 -c wafer.yaml --check-config  parse + validate only, print the configuration as JSON (no GPU needed)
+//   wafer-b200 -c wafer.yaml --seed N        key of the Gaussian initial condition (default 0): same N, same start
 #include <sys/stat.h>
 #include <sys/types.h>
 #include <unistd.h>
 
+#include <cerrno>
 #include <chrono>
 #include <cmath>
 #include <cstdio>
@@ -18,7 +20,6 @@
 #include <ctime>
 #include <fstream>
 #include <iostream>
-#include <random>
 #include <string>
 #include <thread>
 #include <vector>
@@ -207,6 +208,7 @@ bool solve(Run& r, unsigned wnum) {
             throw std::runtime_error("non-finite observables (the reference's R64 would panic here)");
         const double norm_energy = obs.energy / obs.norm2, tau = (double)step * c.dt;
         if (c.snap_update && step % *c.snap_update == 0) {                                               // grid.rs:137-158
+            r.ck(wafer_symmetrise(r.ctx, c.init_symmetry), "wafer_symmetrise");                          // grid.rs:137-139
             r.ck(wafer_normalise(r.ctx, obs.norm2), "wafer_normalise");
             save_wavefunction(r, wnum, false);
         }
@@ -265,6 +267,7 @@ int env_int(const char* k, int dflt) {
 int main(int argc, char** argv) {
     std::string config_file = "wafer.yaml", script = "gen_potential.py", outroot = "output", rdv;
     bool check_only = false, no_output = false, quiet = false;
+    uint64_t seed = 0;  // fixed default: runs are reproducible and every rank of a multi-GPU run draws the same field
     int verbosity = 0;
     for (int i = 1; i < argc; ++i) {
         const std::string a = argv[i];
@@ -276,6 +279,17 @@ int main(int argc, char** argv) {
         else if (a == "-s" || a == "--script") script = next();
         else if (a == "-d" || a == "-dd" || a == "-ddd") verbosity += (int)a.size() - 1;
         else if (a == "--check-config") check_only = true;
+        else if (a == "--seed") {
+            const std::string v = next();
+            char* end = nullptr;
+            errno = 0;
+            const unsigned long long n = strtoull(v.c_str(), &end, 10);
+            if (v.empty() || v[0] == '-' || *end != 0 || errno == ERANGE) {
+                fprintf(stderr, "--seed expects an unsigned 64-bit integer, got %s\n", v.c_str());
+                return 2;
+            }
+            seed = n;
+        }
         else if (a == "--selftest-trilerp") {
             // the reference's `interpolation` unit test input (input.rs:733-748): 2x2x2 [1..8] -> 4x4x4
             Array3 v, out;
@@ -320,7 +334,9 @@ int main(int argc, char** argv) {
         else if (a == "--rendezvous-file") rdv = next();
         else if (a == "-q" || a == "--quiet") quiet = true;
         else if (a == "-h" || a == "--help") {
-            puts("wafer-b200 [-c wafer.yaml] [-s gen_potential.py] [-d] [--check-config] [--no-output] [--output-root DIR] [-q]");
+            puts("wafer-b200 [-c wafer.yaml] [-s gen_potential.py] [-d] [--check-config] [--no-output] [--output-root DIR] [-q]\n"
+                 "           [--seed N]   key of the Gaussian initial condition (default 0); the same N gives the same start\n"
+                 "                        on any number of GPUs");
             return 0;
         } else { fprintf(stderr, "unknown argument %s\n", a.c_str()); return 2; }
     }
@@ -328,6 +344,7 @@ int main(int argc, char** argv) {
     try {
         Run r;
         r.cfg = load_config_file(config_file);
+        r.cfg.seed = seed;
         r.quiet = quiet;
         if (r.cfg.potential == 13) r.cfg.script_location = "./" + script;  // config.rs:344-350
         if (check_only) {
@@ -335,9 +352,6 @@ int main(int argc, char** argv) {
             return 0;
         }
         const Config& c = r.cfg;
-        if (c.init_symmetry != 0)
-            throw std::runtime_error("init_symmetry other than NotConstrained is not supported (the reference's routine "
-                                     "hard-codes the SevenPoint padding, config.rs:702-723)");
         r.rank = env_int("RANK", 0);
         r.world = env_int("WORLD_SIZE", 1);
         uint8_t id[128];
@@ -402,17 +416,12 @@ int main(int argc, char** argv) {
                 std::vector<double> phi(d.padded());
                 if (!read_work("input/wavefunction_0", c.file_type, phi, d)) throw std::runtime_error("LoadWavefunction: input/wavefunction_0.{mpk,csv,json} not found");
                 r.ck(wafer_set_phi(r.ctx, phi.data()), "wafer_set_phi");
-            } else if (c.init_condition == 1) {  // Gaussian (config.rs:636-642): thread_rng there, so any seed is as good
-                std::vector<double> phi(d.padded(), 0.0);
-                std::mt19937_64 gen(std::random_device{}());
-                std::normal_distribution<double> normal(0.0, c.sig);
-                for (size_t i = 0; i < d.nx; ++i)
-                    for (size_t j = 0; j < d.ny; ++j)
-                        for (size_t k = 0; k < d.nz; ++k) phi[d.p(i + d.e, j + d.e, k + d.e)] = normal(gen);
-                r.ck(wafer_set_phi(r.ctx, phi.data()), "wafer_set_phi");
+            } else if (c.init_condition == 1) {  // Gaussian (config.rs:636-642): thread_rng there; seeded on the device here
+                r.ck(wafer_generate_gaussian(r.ctx, c.sig, c.seed), "wafer_generate_gaussian");
             } else {
                 r.ck(wafer_generate_initial_condition(r.ctx, c.init_condition), "wafer_generate_initial_condition");
             }
+            r.ck(wafer_symmetrise(r.ctx, c.init_symmetry), "wafer_symmetrise");                          // config.rs:625
         }
         int rc = 0;
         for (unsigned wnum = c.wavenum; wnum <= c.wavemax; ++wnum) {

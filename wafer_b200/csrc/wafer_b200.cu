@@ -1292,6 +1292,40 @@ int wafer_generate_initial_condition(wafer_ctx* ctx, int32_t kind) {
     return WAFER_OK;
 }
 
+int wafer_generate_gaussian(wafer_ctx* ctx, double sig, uint64_t seed) {
+    if (!ctx) return WAFER_ERR_INVALID;
+    ctx->chk_valid = false;  // psi (or what the check sums depend on) changes
+    REQUIRE(std::isfinite(sig) && sig >= 0., "Gaussian initial condition: sig must be finite and >= 0");
+    CK(cudaSetDevice(ctx->dev));
+    const long long rows = (long long)(ctx->g.L + 2 * ctx->g.gx) * ctx->g.ny;
+    gen_gaussian_kernel<<<(int)std::min<long long>(rows, (long long)ctx->sm_count * 32), 128, 0, ctx->s_main>>>(
+        ctx->psi[ctx->cur], ctx->g, sig, (unsigned long long)seed);
+    TRY(post_launch(ctx));
+    ctx->have_phi = true;
+    return WAFER_OK;
+}
+
+int wafer_symmetrise(wafer_ctx* ctx, int32_t kind) {
+    if (!ctx) return WAFER_ERR_INVALID;
+    REQUIRE(kind >= SYM_NONE && kind <= SYM_ANTI_Y,
+            "init_symmetry: kind must be 0 NotConstrained, 1 AboutZ, 2 AntisymAboutZ, 3 AboutY or 4 AntisymAboutY");
+    if (!ctx->have_phi) { ctx->err = "phi not set (wafer_set_phi / wafer_generate_initial_condition)"; return WAFER_ERR_NOT_READY; }
+    if (kind == SYM_NONE) return WAFER_OK;
+    ctx->chk_valid = false;  // psi (or what the check sums depend on) changes
+    CK(cudaSetDevice(ctx->dev));
+    const Geom& g = ctx->g;
+    const double s = (kind == SYM_ANTI_Z || kind == SYM_ANTI_Y) ? -1. : 1.;
+    const long long planes = (long long)(g.L + 2 * g.gx);
+    if (kind == SYM_ABOUT_Z || kind == SYM_ANTI_Z) {
+        symmetrise_z_kernel<<<(int)std::min<long long>(planes * g.ny, (long long)ctx->sm_count * 32), 128, 0, ctx->s_main>>>(
+            ctx->psi[ctx->cur], g, s);
+    } else {
+        symmetrise_y_kernel<<<(int)std::min<long long>(planes * (g.ny - g.ny / 2), (long long)ctx->sm_count * 32), 128, 0,
+                              ctx->s_main>>>(ctx->psi[ctx->cur], g, s);
+    }
+    return post_launch(ctx);
+}
+
 // ---- the hot path --------------------------------------------------------------------------------------------
 static int ready(wafer_ctx* ctx, bool need_v) {
     if (!ctx->have_phi) { ctx->err = "phi not set (wafer_set_phi / wafer_generate_initial_condition)"; return WAFER_ERR_NOT_READY; }
