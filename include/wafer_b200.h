@@ -132,6 +132,17 @@ int wafer_generate_gaussian(wafer_ctx *ctx, double sig, uint64_t seed);
    With n the work size of the mirrored axis, psi[.., n-1-t] = +-psi[.., t] for t < n/2; the middle index of an odd n
    is kept (symmetric) or set to +0 (antisymmetric).  Exact and idempotent; needs no communication when world > 1. */
 int wafer_symmetrise(wafer_ctx *ctx, int32_t kind);
+/* fill_data (input.rs:149-176) / read_csv (input.rs:641-657) on the device: `src` is the array of an input file as
+   read, dense C order (sx, sy, sz), z contiguous, WORK-area data.  from_csv = 0 (Messagepack / Json): trilinear
+   resample (input.rs:667-716) on a basis of padded-size many points per axis, of which the work area takes the
+   first n; a source of the padded size is refused.  from_csv = 1: a work-sized source is copied, any other size
+   resampled as above.  Resampling needs sx, sy, sz >= 2.  Only the source x-planes this rank's planes need are
+   read, so with world > 1 every rank may pass the whole array; no communication.  Two of its x-planes must fit
+   128 MB (sy*sz*8 <= 64 MB).  Each has the effects of the entry it mirrors (set_phi, set_potential, push_lower);
+   bad arguments are refused with WAFER_ERR_INVALID before anything changes. */
+int wafer_set_phi_resampled(wafer_ctx *ctx, const double *src, uint64_t sx, uint64_t sy, uint64_t sz, uint32_t from_csv);
+int wafer_set_potential_resampled(wafer_ctx *ctx, const double *src, uint64_t sx, uint64_t sy, uint64_t sz, uint32_t from_csv);
+int wafer_push_lower_resampled(wafer_ctx *ctx, const double *src, uint64_t sx, uint64_t sy, uint64_t sz, uint32_t from_csv);
 
 /* -------- the hot path -------------------------------------------------------------------------- */
 int wafer_observables_compute(wafer_ctx *ctx, wafer_observables *out); /* compute_observables        (grid.rs:303-445) */

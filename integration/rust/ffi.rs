@@ -53,6 +53,9 @@ extern "C" {
     fn wafer_phi_seed_from_lower(ctx: *mut WaferCtx, idx: u32) -> c_int;
     fn wafer_generate_gaussian(ctx: *mut WaferCtx, sig: f64, seed: u64) -> c_int;
     fn wafer_symmetrise(ctx: *mut WaferCtx, kind: i32) -> c_int;
+    fn wafer_set_phi_resampled(ctx: *mut WaferCtx, src: *const f64, sx: u64, sy: u64, sz: u64, from_csv: u32) -> c_int;
+    fn wafer_set_potential_resampled(ctx: *mut WaferCtx, src: *const f64, sx: u64, sy: u64, sz: u64, from_csv: u32) -> c_int;
+    fn wafer_push_lower_resampled(ctx: *mut WaferCtx, src: *const f64, sx: u64, sy: u64, sz: u64, from_csv: u32) -> c_int;
     fn wafer_check(ctx: *mut WaferCtx, wnum: u8, out: *mut WaferObservables) -> c_int;
     fn wafer_normalise(ctx: *mut WaferCtx, norm2: f64) -> c_int;
     fn wafer_evolve(ctx: *mut WaferCtx, wnum: u8, steps: u64) -> c_int;
@@ -137,6 +140,21 @@ impl Gpu {
     pub fn symmetrise(&self, kind: i32) -> Result<()> {
         self.check(unsafe { wafer_symmetrise(self.ctx, kind) })
     }
+    /// fill_data / read_csv (input.rs:149-176, 641-657) on the device: `src` is the array of an input file as read (work
+    /// area data, any shape with every axis >= 2, or the work shape for a Csv file), `from_csv` whether it came from a
+    /// Csv file.  Only this rank's source planes are copied.
+    pub fn set_phi_resampled(&self, src: &Array3<R64>, from_csv: bool) -> Result<()> {
+        let (p, x, y, z) = resample_args(src)?;
+        self.check(unsafe { wafer_set_phi_resampled(self.ctx, p, x, y, z, from_csv as u32) })
+    }
+    pub fn set_potential_resampled(&self, src: &Array3<R64>, from_csv: bool) -> Result<()> {
+        let (p, x, y, z) = resample_args(src)?;
+        self.check(unsafe { wafer_set_potential_resampled(self.ctx, p, x, y, z, from_csv as u32) })
+    }
+    pub fn push_lower_resampled(&self, src: &Array3<R64>, from_csv: bool) -> Result<()> {
+        let (p, x, y, z) = resample_args(src)?;
+        self.check(unsafe { wafer_push_lower_resampled(self.ctx, p, x, y, z, from_csv as u32) })
+    }
     pub fn check_state(&self, wnum: u8) -> Result<WaferObservables> {
         let mut o = WaferObservables::default();
         self.check(unsafe { wafer_check(self.ctx, wnum, &mut o) })?;
@@ -166,4 +184,13 @@ impl Drop for Gpu {
             wafer_destroy(self.ctx);
         }
     }
+}
+
+/// pointer and shape of a C-order array for the wafer_*_resampled entries
+fn resample_args(src: &Array3<R64>) -> Result<(*const f64, u64, u64, u64)> {
+    if !src.is_standard_layout() {
+        return Err("input array is not in standard (C) layout".into());
+    }
+    let (x, y, z) = src.dim();
+    Ok((src.as_ptr() as *const f64, x as u64, y as u64, z as u64))
 }

@@ -285,6 +285,27 @@ class Lattice:
         Mirrors the work area about its centre in y or z, copying the lower half (negated for the Antisym kinds)."""
         self._ck(self._lib.wafer_symmetrise(self._h, SYMMETRIES[kind] if isinstance(kind, str) else int(kind)))
 
+    # ---- input files resampled on the device: fill_data (input.rs:149-176) / read_csv (input.rs:641-657)
+    def _resampled(self, fn, arr, from_csv):
+        if arr.ndim != 3:
+            raise ValueError("expected a 3-D array (the array of an input file), got shape %r" % (arr.shape,))
+        sx, sy, sz = arr.shape
+        self._ck(fn(self._h, _p(arr), sx, sy, sz, 1 if from_csv else 0))
+
+    def set_phi_resampled(self, arr, from_csv=False):
+        """phi from the WORK-area array of an input file as read, shape (sx, sy, sz): trilinear resample on the
+        reference's padded-size basis (Messagepack / Json, from_csv=False, always resampled; a padded-size array is
+        refused), or for from_csv=True a straight copy of a work-sized array.  Runs on the device."""
+        self._resampled(self._lib.wafer_set_phi_resampled, arr, from_csv)
+
+    def set_potential_resampled(self, arr, from_csv=False):
+        """V from an input file's array, resampled like set_phi_resampled (the FromFile potential)"""
+        self._resampled(self._lib.wafer_set_potential_resampled, arr, from_csv)
+
+    def push_lower_resampled(self, arr, from_csv=False):
+        """w_store.push of an input file's array, resampled like set_phi_resampled (input::load_wavefunctions)"""
+        self._resampled(self._lib.wafer_push_lower_resampled, arr, from_csv)
+
     def push_lower(self, q=None):
         """w_store.push(q); with q=None pushes the current phi (grid.rs:241)."""
         if q is None:

@@ -57,6 +57,9 @@ SYMBOLS = {
     "wafer_generate_initial_condition": (C.c_int, [_ctx, C.c_int32]),
     "wafer_generate_gaussian": (C.c_int, [_ctx, C.c_double, C.c_uint64]),
     "wafer_symmetrise": (C.c_int, [_ctx, C.c_int32]),
+    "wafer_set_phi_resampled": (C.c_int, [_ctx, _dp, C.c_uint64, C.c_uint64, C.c_uint64, C.c_uint32]),
+    "wafer_set_potential_resampled": (C.c_int, [_ctx, _dp, C.c_uint64, C.c_uint64, C.c_uint64, C.c_uint32]),
+    "wafer_push_lower_resampled": (C.c_int, [_ctx, _dp, C.c_uint64, C.c_uint64, C.c_uint64, C.c_uint32]),
     "wafer_observables_compute": (C.c_int, [_ctx, C.POINTER(Observables)]),
     "wafer_norm2": (C.c_int, [_ctx, _dp]),
     "wafer_normalise": (C.c_int, [_ctx, C.c_double]),

@@ -49,16 +49,19 @@ std::string ordinal(unsigned n) {
     return std::to_string(n) + suf;
 }
 
-// array files: work area out (output.rs:79-216), work area in with optional trilinear resize (input.rs:149-176)
+// array files: work area out (output.rs:79-216); in, the file's array as parsed (input.rs:32-127, 513-662), which the
+// wafer_*_resampled entries embed on the device as fill_data / read_csv do (input.rs:149-176, 641-657; formats.hpp
+// embed_work is the host restatement).  from_csv: the file read was a Csv file.
 void write_work(const std::string& stem, int file_type, const double* padded, const Dims& d) {
     write_array(stem, file_type, extract_work(padded, d.nx, d.ny, d.nz, d.e));
 }
-bool read_work(const std::string& stem, int file_type, std::vector<double>& padded, const Dims& d) {
-    Array3 a;
+bool read_input(const std::string& stem, int file_type, const Dims& d, Array3& a, uint32_t& from_csv) {
     int used = 0;
     if (!read_array(stem, file_type, a, &used)) return false;
     if (a.nx < 2 || a.ny < 2 || a.nz < 2) throw std::runtime_error("ArrayShape: " + stem + " cannot be resized");
-    embed_work(a, padded, d.nx, d.ny, d.nz, d.e, used == 1);
+    from_csv = used == 1 ? 1 : 0;
+    if (!from_csv && a.nx == d.px && a.ny == d.py && a.nz == d.pz)
+        throw std::runtime_error("input array already has the padded size: the reference's fill_data cannot load it (input.rs:167-169)");
     return true;
 }
 
@@ -183,9 +186,10 @@ bool solve(Run& r, unsigned wnum) {
     const Dims d(c);
     if (wnum > 0) {
         // grid.rs:60-96: a wavefunction_{wnum} file in ./input wins, else start from the previous converged state
-        std::vector<double> phi(d.padded());
-        if (read_work("input/wavefunction_" + std::to_string(wnum), c.file_type, phi, d)) {
-            r.ck(wafer_set_phi(r.ctx, phi.data()), "wafer_set_phi");
+        Array3 a;
+        uint32_t csv = 0;
+        if (read_input("input/wavefunction_" + std::to_string(wnum), c.file_type, d, a, csv)) {
+            r.ck(wafer_set_phi_resampled(r.ctx, a.data.data(), a.nx, a.ny, a.nz, csv), "wafer_set_phi_resampled");
         } else {
             // grid.rs:95 clones w_store[wnum-1] and lets rounding noise seed the new state (SURVEY F7); here the
             // clone is multiplied by a fixed symmetry-free polynomial so the start is well defined and reproducible
@@ -380,9 +384,10 @@ int main(int argc, char** argv) {
 
         // potential::load_arrays (potential.rs:75-175)
         if (c.potential == 12) {  // FromFile
-            std::vector<double> v(d.padded());
-            if (!read_work("input/potential", c.file_type, v, d)) throw std::runtime_error("LoadPotential: input/potential.{mpk,csv,json} not found");
-            r.ck(wafer_set_potential(r.ctx, v.data()), "wafer_set_potential");
+            Array3 a;
+            uint32_t csv = 0;
+            if (!read_input("input/potential", c.file_type, d, a, csv)) throw std::runtime_error("LoadPotential: input/potential.{mpk,csv,json} not found");
+            r.ck(wafer_set_potential_resampled(r.ctx, a.data.data(), a.nx, a.ny, a.nz, csv), "wafer_set_potential_resampled");
         } else if (c.potential == 13) {  // FromScript
             std::vector<double> v(d.padded());
             script_potential(c, v, d);
@@ -405,17 +410,19 @@ int main(int argc, char** argv) {
 
         // run (grid.rs:31-47): lower states from ./input when starting above the ground state
         for (unsigned w = 0; w < c.wavenum; ++w) {  // input::load_wavefunctions (input.rs:487-505)
-            std::vector<double> q(d.padded());
-            if (!read_work("input/wavefunction_" + std::to_string(w), c.file_type, q, d))
+            Array3 a;
+            uint32_t csv = 0;
+            if (!read_input("input/wavefunction_" + std::to_string(w), c.file_type, d, a, csv))
                 throw std::runtime_error("LoadWavefunction: input/wavefunction_" + std::to_string(w) + ".{mpk,csv,json} is required when wavenum > 0");
-            r.ck(wafer_push_lower(r.ctx, q.data()), "wafer_push_lower");
+            r.ck(wafer_push_lower_resampled(r.ctx, a.data.data(), a.nx, a.ny, a.nz, csv), "wafer_push_lower_resampled");
         }
         // config::set_initial_conditions (config.rs:577-627)
         if (c.wavenum == 0) {
             if (c.init_condition == 0) {
-                std::vector<double> phi(d.padded());
-                if (!read_work("input/wavefunction_0", c.file_type, phi, d)) throw std::runtime_error("LoadWavefunction: input/wavefunction_0.{mpk,csv,json} not found");
-                r.ck(wafer_set_phi(r.ctx, phi.data()), "wafer_set_phi");
+                Array3 a;
+                uint32_t csv = 0;
+                if (!read_input("input/wavefunction_0", c.file_type, d, a, csv)) throw std::runtime_error("LoadWavefunction: input/wavefunction_0.{mpk,csv,json} not found");
+                r.ck(wafer_set_phi_resampled(r.ctx, a.data.data(), a.nx, a.ny, a.nz, csv), "wafer_set_phi_resampled");
             } else if (c.init_condition == 1) {  // Gaussian (config.rs:636-642): thread_rng there; seeded on the device here
                 r.ck(wafer_generate_gaussian(r.ctx, c.sig, c.seed), "wafer_generate_gaussian");
             } else {

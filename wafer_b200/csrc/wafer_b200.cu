@@ -22,6 +22,7 @@
 #include "generators.cuh"
 #include "kernels.cuh"
 #include "nccl_dyn.h"
+#include "resample.cuh"
 #include "sweep_tb.cuh"
 #include "sweep_tma1.cuh"
 
@@ -75,6 +76,9 @@ struct wafer_ctx {
     // pack / unpack kernel of the other one runs on s_main (lazily allocated, never a field-sized buffer)
     double* stg[2] = {nullptr, nullptr};
     long long stg_planes = 0;       // padded host planes one bounce buffer holds
+    // source staging of the resampling entries when two source planes do not fit a bounce buffer (<= 128 MB each)
+    double* rs_stg[2] = {nullptr, nullptr};
+    long long rs_cap = 0;           // doubles one of them holds
     cudaStream_t s_copy = nullptr;
     cudaEvent_t ev_stg_free[2] = {nullptr, nullptr}, ev_stg_full[2] = {nullptr, nullptr};
     double* partials = nullptr;
@@ -892,6 +896,90 @@ int ensure_ab(wafer_ctx* ctx) {
     return post_launch(ctx);
 }
 
+// fill_data / read_csv on the device (resample.cuh) into the work area of `dst`: only the source x-planes this rank's
+// planes need are copied, run by run, through two device staging buffers (the bounce buffers when two source planes
+// fit one, else two of at most 128 MB); the copy of one run overlaps the kernel of the other.  Synchronises.
+constexpr long long RS_MAX_STG = (128ll << 20) / (long long)sizeof(double);  // doubles in one 128 MB staging buffer
+
+bool resample_copies(const wafer_ctx* ctx, uint64_t sx, uint64_t sy, uint64_t sz, uint32_t from_csv) {
+    return from_csv && sx == (uint64_t)ctx->g.gnx && sy == (uint64_t)ctx->g.gny && sz == (uint64_t)ctx->g.gnz;
+}
+
+int resample_args(wafer_ctx* ctx, const double* src, uint64_t sx, uint64_t sy, uint64_t sz, uint32_t from_csv) {
+    const Geom& g = ctx->g;
+    const uint64_t e2 = 2 * (uint64_t)g.e;
+    REQUIRE(src, "src is NULL");
+    REQUIRE(from_csv <= 1, "from_csv must be 0 (Messagepack / Json) or 1 (Csv)");
+    REQUIRE(sx > 0 && sy > 0 && sz > 0, "ArrayShape: the input array has a zero dimension");
+    REQUIRE(from_csv || !(sx == g.gnx + e2 && sy == g.gny + e2 && sz == g.gnz + e2),
+            "input array already has the padded size: the reference's fill_data cannot load it (input.rs:167-169)");
+    REQUIRE(resample_copies(ctx, sx, sy, sz, from_csv) || (sx >= 2 && sy >= 2 && sz >= 2),
+            "ArrayShape: the input array cannot be resized (needs >= 2 points per axis)");
+    REQUIRE(sy <= (uint64_t)RS_MAX_STG / 2 && sz <= (uint64_t)RS_MAX_STG / 2 / sy,
+            "input array: two of its x-planes (2*sy*sz*8 bytes) exceed the 128 MB staging buffer");
+    return WAFER_OK;
+}
+
+// the arguments passed resample_args
+int resample_into(wafer_ctx* ctx, const double* src, uint64_t sx, uint64_t sy, uint64_t sz, uint32_t from_csv, double* dst) {
+    const Geom& g = ctx->g;
+    const bool copy = resample_copies(ctx, sx, sy, sz, from_csv);
+    const long long splane = (long long)(sy * sz), need = copy ? 1 : 2;
+    // global work planes of the slab inside the lattice (ghosts included) and the source planes [lo, lo + need) of each
+    const long long ga = std::max<long long>(0, g.x0 - g.gx), gb = std::min<long long>(g.gnx, g.x0 + g.L + g.gx);
+    const long long bx = g.gnx + 2 * g.e;
+    auto lo = [&](long long gi) {
+        if (copy) return gi;
+        long long i0;
+        double d;
+        rs_bracket((long long)sx, bx, gi, &i0, &d);
+        return i0;
+    };
+    TRY(ensure_staging(ctx));
+    double* buf[2] = {ctx->stg[0], ctx->stg[1]};
+    long long cap = ctx->stg_planes * (long long)(g.ny + 2 * g.e) * (g.nz + 2 * g.e) / splane;  // source planes per buffer
+    if (cap < need) {
+        cap = std::min<long long>(RS_MAX_STG / splane, gb > ga ? lo(gb - 1) + need - lo(ga) : need);
+        if (ctx->rs_cap < cap * splane) {  // the last call that used them synchronised before returning
+            for (int b = 0; b < 2; ++b) {
+                cudaFree(ctx->rs_stg[b]);
+                ctx->rs_stg[b] = nullptr;
+            }
+            ctx->rs_cap = 0;
+            for (int b = 0; b < 2; ++b) CK(cudaMalloc(&ctx->rs_stg[b], (size_t)(cap * splane) * sizeof(double)));
+            ctx->rs_cap = cap * splane;
+        }
+        buf[0] = ctx->rs_stg[0];
+        buf[1] = ctx->rs_stg[1];
+    }
+    CK(cudaEventRecord(ctx->ev_stg_free[0], ctx->s_main));  // everything queued so far precedes the first refill
+    CK(cudaEventRecord(ctx->ev_stg_free[1], ctx->s_main));
+    const int ztiles = std::min(ceil_div(g.nz, RS_ZTILE), 65535);
+    int k = 0;
+    for (long long a = ga; a < gb; ++k) {
+        const long long s0 = lo(a);
+        long long b = a + 1;
+        while (b < gb && lo(b) + need - s0 <= cap) ++b;  // lo() is non-decreasing: the run's planes are [s0, lo(b-1)+need)
+        const long long s1 = lo(b - 1) + need;
+        const int nb = k & 1;
+        CK(cudaStreamWaitEvent(ctx->s_copy, ctx->ev_stg_free[nb], 0));
+        CK(cudaMemcpyAsync(buf[nb], src + s0 * splane, (size_t)((s1 - s0) * splane) * sizeof(double), cudaMemcpyHostToDevice,
+                           ctx->s_copy));
+        CK(cudaEventRecord(ctx->ev_stg_full[nb], ctx->s_copy));
+        CK(cudaStreamWaitEvent(ctx->s_main, ctx->ev_stg_full[nb], 0));
+        const int i0 = (int)(a - g.x0), i1 = (int)(b - g.x0);
+        const dim3 grid((unsigned)std::min<long long>((long long)(i1 - i0) * g.ny, std::max(1, ctx->sm_count * 8 / ztiles)),
+                        (unsigned)ztiles);
+        if (copy) resample_kernel<true><<<grid, RS_THREADS, 0, ctx->s_main>>>(dst, g, buf[nb], s0, (long long)sx, (long long)sy, (long long)sz, i0, i1);
+        else resample_kernel<false><<<grid, RS_THREADS, 0, ctx->s_main>>>(dst, g, buf[nb], s0, (long long)sx, (long long)sy, (long long)sz, i0, i1);
+        TRY(post_launch(ctx));
+        CK(cudaEventRecord(ctx->ev_stg_free[nb], ctx->s_main));
+        a = b;
+    }
+    CK(cudaStreamSynchronize(ctx->s_main));  // the caller may free `src` on return
+    return WAFER_OK;
+}
+
 int create_impl(const wafer_params* params, wafer_ctx* ctx) {
     const wafer_params& p = *params;
     REQUIRE(p.nx > 0 && p.ny > 0 && p.nz > 0, "grid.size must be positive");
@@ -1023,6 +1111,7 @@ int wafer_destroy(wafer_ctx* ctx) {
     cudaFree(ctx->psi[0]); cudaFree(ctx->psi[1]); cudaFree(ctx->v); cudaFree(ctx->a); cudaFree(ctx->b);
     for (int b = 0; b < 2; ++b) {
         cudaFree(ctx->stg[b]);
+        cudaFree(ctx->rs_stg[b]);
         if (ctx->ev_stg_free[b]) cudaEventDestroy(ctx->ev_stg_free[b]);
         if (ctx->ev_stg_full[b]) cudaEventDestroy(ctx->ev_stg_full[b]);
     }
@@ -1324,6 +1413,61 @@ int wafer_symmetrise(wafer_ctx* ctx, int32_t kind) {
                               ctx->s_main>>>(ctx->psi[ctx->cur], g, s);
     }
     return post_launch(ctx);
+}
+
+// ---- input files resampled on the device (resample.cuh) -------------------------------------------------------
+enum { RS_PHI = 0, RS_POTENTIAL, RS_LOWER };
+
+static int resampled_impl(wafer_ctx* ctx, int which, const double* src, uint64_t sx, uint64_t sy, uint64_t sz,
+                          uint32_t from_csv) {
+    if (!ctx) return WAFER_ERR_INVALID;
+    TRY(resample_args(ctx, src, sx, sy, sz, from_csv));  // before anything is allocated or written
+    CK(cudaSetDevice(ctx->dev));
+    if (which == RS_PHI) {  // the effects of wafer_set_phi; the ring is +0 by construction
+        ctx->chk_valid = false;  // psi (or what the check sums depend on) changes
+        const int rc = resample_into(ctx, src, sx, sy, sz, from_csv, ctx->psi[ctx->cur]);
+        ctx->have_phi = rc == WAFER_OK;
+        return rc;
+    }
+    if (which == RS_POTENTIAL) {  // the effects of wafer_set_potential
+        ctx->chk_valid = false;
+        ctx->h_valid = false;
+        TRY(resample_into(ctx, src, sx, sy, sz, from_csv, ctx->v));
+        TRY(ensure_ab(ctx));
+        ctx->have_v = true;
+        return WAFER_OK;
+    }
+    // the effects of wafer_push_lower
+    REQUIRE(ctx->lowers.size() < 255, "at most 255 lower states (wavenum is a u8, config.rs:308)");
+    double* q = nullptr;
+    TRY(alloc_field(ctx, &q));
+    int rc = resample_into(ctx, src, sx, sy, sz, from_csv, q);
+    if (rc == WAFER_OK) rc = register_lower(ctx, q);
+    if (rc != WAFER_OK) cudaFree(q);
+    return rc;
+}
+
+static int resampled(wafer_ctx* ctx, int which, const char* name, const double* src, uint64_t sx, uint64_t sy,
+                     uint64_t sz, uint32_t from_csv) {
+    try {
+        return resampled_impl(ctx, which, src, sx, sy, sz, from_csv);
+    } catch (const std::exception& e) {  // host-side allocation failures must not unwind through the C ABI
+        if (ctx) ctx->err = std::string(name) + ": " + e.what();
+        return WAFER_ERR_INVALID;
+    }
+}
+
+int wafer_set_phi_resampled(wafer_ctx* ctx, const double* src, uint64_t sx, uint64_t sy, uint64_t sz, uint32_t from_csv) {
+    return resampled(ctx, RS_PHI, "wafer_set_phi_resampled", src, sx, sy, sz, from_csv);
+}
+
+int wafer_set_potential_resampled(wafer_ctx* ctx, const double* src, uint64_t sx, uint64_t sy, uint64_t sz,
+                                  uint32_t from_csv) {
+    return resampled(ctx, RS_POTENTIAL, "wafer_set_potential_resampled", src, sx, sy, sz, from_csv);
+}
+
+int wafer_push_lower_resampled(wafer_ctx* ctx, const double* src, uint64_t sx, uint64_t sy, uint64_t sz, uint32_t from_csv) {
+    return resampled(ctx, RS_LOWER, "wafer_push_lower_resampled", src, sx, sy, sz, from_csv);
 }
 
 // ---- the hot path --------------------------------------------------------------------------------------------
