@@ -2,8 +2,7 @@
 # the CPU oracle under oracle/.  `python -c "import __graft_entry__ as g; g.build()"` runs `make all`.
 NVCC      ?= /usr/local/cuda/bin/nvcc
 ARCH      := -gencode arch=compute_100a,code=sm_100a
-TBFLAGS   ?=
-NVCCFLAGS := $(ARCH) $(TBFLAGS) -O3 -std=c++17 -lineinfo -fmad=false -Xcompiler -fPIC,-Wall,-Wno-unused-function --expt-relaxed-constexpr
+NVCCFLAGS := $(ARCH) -O3 -std=c++17 -lineinfo -fmad=false -Xcompiler -fPIC,-Wall,-Wno-unused-function --expt-relaxed-constexpr
 CSRC      := wafer_b200/csrc
 LIB       := wafer_b200/libwafer_b200.so
 

@@ -189,8 +189,8 @@ int wafer_selftest_division(wafer_ctx *ctx, double den, uint64_t n, uint64_t see
    2^-64 collisions).  This is how multi-GPU runs are compared bit-for-bit with a single-GPU run at full size. */
 int wafer_phi_checksum(wafer_ctx *ctx, uint64_t x_begin, uint64_t x_end, uint64_t out[2]);
 /* Fault injection for the multi-GPU ordering tests: stall this rank by `nanoseconds` (<= 1e9) before the halo handshake
-   of every pass of wafer_evolve (the main stream in the whole-column form, the halo stream in the split form), so that
-   its x-neighbours run ahead of it.  0 switches it off. */
+   of every pass of wafer_evolve (on the main stream before a two-step pass with fused halos, on the halo stream before
+   the boundary launches of every other multi-GPU pass), so that its x-neighbours run ahead of it.  0: no stall. */
 int wafer_debug_halo_delay(wafer_ctx *ctx, uint64_t nanoseconds);
 const char *wafer_version(void);
 const char *wafer_sweep_variant(const wafer_ctx *ctx); /* name of the sweep kernel variant in use */

@@ -1,4 +1,5 @@
-"""Excited-state step rate at 512^3 for k = 3, 4 stored states only (A/B of the prefetch depth WAFER_T1_NPRE3)."""
+"""Excited-state step rate at 512^3 for k = 3, 4 stored states (the modes of the one-step sweep that prefetch one of the
+stored states)."""
 import json
 import os
 import sys

@@ -1,6 +1,6 @@
 #!/bin/bash
-# Round-2 multi-GPU session (gpurun --gpus N): drift/race parity with and without the end-of-evolve wait, NCCL-halo
-# parity, then bench lines at the requested rank counts.   bash scripts/gpu_multi2.sh <label> <N> [bench args]
+# Round-2 multi-GPU session on N GPUs: drift/race parity of the fused halo, NCCL-halo parity, then bench lines
+# at the requested rank counts.   bash scripts/gpu_multi2.sh <label> <N> [bench args]
 set -u
 LABEL=${1:-multi}; N=${2:-2}; shift 2 || true
 EXTRA=${*:-}
@@ -14,7 +14,6 @@ run_check() {  # name, env...
   echo "check $name rc=$?" | tee -a "$OUT/rc.log"; grep '^{' "$OUT/check_$name.log" | tail -1; grep -E "Error|error" "$OUT/check_$name.log" | tail -2 | cut -c1-300
 }
 run_check p2p WAFER_P2P=1
-[ "${SKIP_NEG:-0}" = 1 ] || run_check p2p_nofinalwait WAFER_P2P=1 WAFER_DEBUG_SKIP_FINAL_WAIT=1   # must FAIL: proves the drift test sees the race
 run_check nccl WAFER_P2P=0
 if [ "${EXCITED:-1}" = 1 ]; then
   timeout 600 python -m torch.distributed.run --nnodes=1 --nproc-per-node $N --master-addr 127.0.0.1 --master-port 29555 \

@@ -129,8 +129,7 @@ def main():
     allt = [torch.zeros_like(t) for _ in range(world)]
     dist.all_gather(allt, t)
     allt = torch.stack(allt).cpu().numpy()
-    results["drift"] = dict(shape=list(shape), sweeps=sweeps, bitwise=bool(allt[:, 0].all()), obs_rel=float(allt[:, 1].max()),
-                            final_wait=os.environ.get("WAFER_DEBUG_SKIP_FINAL_WAIT", "0") != "1")
+    results["drift"] = dict(shape=list(shape), sweeps=sweeps, bitwise=bool(allt[:, 0].all()), obs_rel=float(allt[:, 1].max()))
     ok = ok and results["drift"]["bitwise"] and results["drift"]["obs_rel"] < 1e-12
     single.close()
     multi.close()

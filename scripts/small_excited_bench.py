@@ -1,5 +1,5 @@
-"""Excited-state step rate on small lattices (launch-bound regime): microseconds per step for k = 1, 3 at 50^3 .. 256^3.
-Run twice, with WAFER_GRAPHS=1 (default) and WAFER_GRAPHS=0, to see what the CUDA-graph replay of step pairs buys."""
+"""Excited-state step rate on small lattices (launch-bound regime, where the CUDA-graph replay of step pairs matters):
+microseconds per step for k = 1, 3 at 50^3 .. 256^3."""
 import json
 import os
 import sys
@@ -8,7 +8,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 import wafer_b200  # noqa: E402
 
-out = {"graphs": os.environ.get("WAFER_GRAPHS", "1")}
+out = {}
 for n in (50, 128, 256):
     dn = 10.24 / n
     with wafer_b200.Lattice((n,) * 3, "ThreePoint", dn=dn, dt=0.1 * dn * dn, mass=1.0) as lat:

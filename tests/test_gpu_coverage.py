@@ -5,7 +5,8 @@
   boxes of the numpy restatement, and at moderate sizes whose plans have the same structures, against the whole oracle;
 * state cached on a context across calls: the CUDA graphs of excited-state steps, the h field of the time-tiled sweep,
   the check sums fused into the last sweep of an evolve;
-* the A/B switches read from the environment (one worker process per setting), which must not change a single bit.
+* the A/B switch read from the environment (WAFER_T1_HFIELD, one worker process per setting), which must not change a
+  single bit.
 
 Bars as in test_gpu_parity.py: bit for bit where nothing is reduced, 1e-12 relative for sums and excited-state steps.
 """
@@ -57,8 +58,9 @@ PLAN_SHAPES = [((40, 512, 512), 1, 1), ((600, 390, 720), 2, 2), ((160, 600, 1080
 @gpu
 @pytest.mark.parametrize("shape,chunks,rounds", PLAN_SHAPES)
 def test_time_tiled_sweep_with_chunks_rounds_and_tail(wb, oracle, shape, chunks, rounds):
-    """Two evolves on one context (the schedule is cached and its counters re-arm themselves between launches):
-    7 steps = three time-tiled launches, the h field and one one-step tail step, then 6 more."""
+    """Three evolves on one context (the schedule is cached and its counters re-arm themselves between launches):
+    3 steps before the h field exists = one time-tiled launch that reads V and one one-step step; 7 steps = the h field,
+    three time-tiled launches that read it and one one-step tail step; then 6 more."""
     rng = np.random.default_rng(97)
     g = oracle.make_grid(*shape, ext=1, dn=0.05, dt=6.25e-4, mass=1.0)
     v = rng.normal(size=g.padded_shape) * 3.0
@@ -72,10 +74,14 @@ def test_time_tiled_sweep_with_chunks_rounds_and_tail(wb, oracle, shape, chunks,
         assert nc >= 1 and nr >= 1 and len(tail) > 0 and tail.min() >= 6, (nc, nr, tail)
         lat.set_potential(v)
         lat.set_phi(phi)
+        lat.evolve(0, 3)
+        got3 = lat.get_phi()
         lat.evolve(0, 7)
         got7 = lat.get_phi()
         lat.evolve(0, 6)
         got13 = lat.get_phi()
+    oracle.evolve(g, phi, a, b, 3)
+    assert np.array_equal(got3, phi)
     oracle.evolve(g, phi, a, b, 7)
     assert np.array_equal(got7, phi)
     oracle.evolve(g, phi, a, b, 6)
@@ -404,9 +410,8 @@ def test_fused_check_sums_are_dropped_when_their_inputs_change(wb, oracle, chang
                 assert abs(got[key] - want[key]) <= SUM_TOL * scale, (key, got[key], want[key])
 
 
-# ---------------------------------------------------------------------------------------------- environment switches
-ENV_VARIANTS = [{}, {"WAFER_TB_SCHED": "rounds"}, {"WAFER_TB_SCHED": "legacy"}, {"WAFER_TB_SCHED": "contig"},
-                {"WAFER_TB_MAXSEG": "8"}, {"WAFER_TB_HFIELD": "0"}, {"WAFER_T1_HFIELD": "1"}, {"WAFER_GRAPHS": "0"}]
+# ---------------------------------------------------------------------------------------------- environment switch
+ENV_VARIANTS = [{}, {"WAFER_T1_HFIELD": "1"}]
 ENV_KEYS = sorted({k for e in ENV_VARIANTS for k in e})
 
 
@@ -442,7 +447,7 @@ def worker():
 
 @gpu
 def test_environment_switches_give_identical_results():
-    """The switches are read once per process: one worker per setting, each must print the default's checksums."""
+    """The switch is read once per process: one worker per setting, each must print the default's checksums."""
     here = os.path.abspath(__file__)
     results = []
     for extra in ENV_VARIANTS:

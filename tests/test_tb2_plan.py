@@ -40,14 +40,14 @@ def _check(ny, nz, xb, xe, slots):
 @pytest.mark.parametrize("ny,nz,xb,xe,slots", [
     (1024, 1024, 0, 1024, 148),   # C4 on one GPU: 630 columns
     (1024, 1024, 0, 128, 148),    # one rank's slab at N = 8
-    (1024, 1024, 0, 2, 148),      # a boundary launch of the split halo form
+    (1024, 1024, 0, 2, 148),      # a boundary launch of the NCCL-overlap path
     (512, 512, 0, 512, 148),      # 162 columns: one round + 14 columns cut 148 ways
     (2048, 2048, 0, 256, 148),    # C5
     (50, 50, 0, 50, 148), (33, 64, 0, 7, 148), (9, 10, 0, 12, 148), (3, 2, 0, 7, 148), (700, 61, 3, 90, 148),
     (512, 512, 2, 510, 132), (100, 100, 0, 1001, 7), (64, 64, 0, 5000, 148), (480, 512, 0, 512, 148), (300, 512, 0, 600, 148),
     # thin slabs of wide planes: the tail holds fewer than 6 planes per CTA, so only some CTAs get a share
     (512, 512, 0, 40, 148),
-    (512, 512, 2, 62, 148),       # interior launch of the split halo form at 512^3 on 8 GPUs
+    (512, 512, 2, 62, 148),       # interior launch of the NCCL-overlap path at 512^3 on 8 GPUs
     (900, 1200, 0, 70, 148),
 ])
 def test_plan_covers_every_plane_once_and_is_balanced(ny, nz, xb, xe, slots):

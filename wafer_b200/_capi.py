@@ -3,7 +3,7 @@ import ctypes as C
 import os
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-# WAFER_B200_LIB: another build of the same library (kernel-variant A/B runs, scripts/gpu_libs.sh); never a fallback
+# WAFER_B200_LIB: another build of the same library (to compare two builds in one session); never a fallback
 LIB_PATH = os.environ.get("WAFER_B200_LIB") or os.path.join(_HERE, "libwafer_b200.so")
 
 _dp = C.POINTER(C.c_double)

@@ -166,18 +166,10 @@ __global__ void __launch_bounds__(1024) finalize_kernel(const double* __restrict
 // (measured on B200, profiles/: letting ptxas pick the register count — 58..64 — beats forcing 5-6 CTAs/SM for
 // the 5/7-point and norm-fused variants; only the plain 3-point variant gains from 40 registers, and that case is
 // served by the time-tiled kernel anyway)
-#ifdef WAFER_SW_MINBLOCKS
-#define WAFER_SW_BOUNDS __launch_bounds__(SW_BX * SW_BY, WAFER_SW_MINBLOCKS)
-#else
-#define WAFER_SW_BOUNDS __launch_bounds__(SW_BX * SW_BY)
-#endif
-#ifndef WAFER_SW_XCH
-#define WAFER_SW_XCH 32
-#endif
-constexpr int SW_BX = 32, SW_BY = 8, SW_XCH = WAFER_SW_XCH;
+constexpr int SW_BX = 32, SW_BY = 8, SW_XCH = 32;
 
 template <int E, bool ONFLY, bool NORM>
-__global__ void WAFER_SW_BOUNDS
+__global__ void __launch_bounds__(SW_BX * SW_BY)
     sweep_simple_kernel(const double* __restrict__ cur, double* __restrict__ nxt, const double* __restrict__ fa,
                         const double* __restrict__ fb, Geom g, int xb, int xe, double dt, double den,
                         double* __restrict__ partials) {

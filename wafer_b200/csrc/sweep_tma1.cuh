@@ -19,10 +19,6 @@
 #include "kernels.cuh"
 #include "sweep_tb.cuh"
 
-#ifndef WAFER_T1_NPRE3
-#define WAFER_T1_NPRE3 1  // measured at 512^3, k = 3 / 4: 1 -> 65.1 / 58.1 GLUPS, 0 -> 64.7 / 57.8, 2 -> 62.7 / 55.2 (gpurun_out/r2ae)
-#endif
-
 namespace wafer {
 namespace t1 {
 
@@ -116,8 +112,9 @@ __device__ __forceinline__ void iteration(Smem<E>& sm, double2 (&q)[2][Cfg<E>::N
     // arithmetic, consumed after them (loading them at the point of use left the whole DRAM latency exposed: the k = 1
     // sweep took 1.0 ms against 0.6 ms for the plain one at 512^3, ncu r2n)
     constexpr int NQ = (M::nred > 1 && !M::obs && !M::chk) ? M::nred - 1 : 0;
-    // NPRE of the NQ states are fetched early; more than that spills at the 128-register cap (ptxas -v)
-    constexpr int NPRE = E != 1 ? 0 : (NQ <= 2 ? NQ : WAFER_T1_NPRE3);
+    // NPRE of the NQ states are fetched early; more than that spills at the 128-register cap (ptxas -v).  With 3 or 4
+    // states, one early, measured at 512^3, k = 3 / 4: 65.1 / 58.1 GLUPS, against 64.7 / 57.8 for none and 62.7 / 55.2 for two
+    constexpr int NPRE = E != 1 ? 0 : (NQ <= 2 ? NQ : 1);
     double2 ql[2][NQ > 0 ? NQ : 1];
     if (NPRE > 0 && t >= 2 * E) {
 #pragma unroll
@@ -139,7 +136,6 @@ __device__ __forceinline__ void iteration(Smem<E>& sm, double2 (&q)[2][Cfg<E>::N
         const double* vs = sm.st[s_new].v + ln.cb;  // V plane c rides with psi plane c+E
         constexpr int IC = qslot<E>(PHASE, E);
         const bool nofast = !dc.fast;
-        const double hdt = D_MUL(dt, 0.5);
         double xx2 = 0.0;
         if (M::obs || M::chk) {  // (global x of the output plane - centre)^2; the plane is xa - 2E + t
             const double dx = D_ADD(xc0, (double)t);
@@ -205,8 +201,8 @@ __device__ __forceinline__ void iteration(Smem<E>& sm, double2 (&q)[2][Cfg<E>::N
                     tb::ab_fast_h(vv.x, dt, a0, bd0, b0);
                     tb::ab_fast_h(vv.y, dt, a1, bd1, b1);
                 } else {
-                    tb::ab_fast(vv.x, hdt, dt, a0, bd0, b0);
-                    tb::ab_fast(vv.y, hdt, dt, a1, bd1, b1);
+                    tb::ab_fast(vv.x, dt, a0, bd0, b0);
+                    tb::ab_fast(vv.y, dt, a1, bd1, b1);
                 }
                 double2 r;
                 r.x = tb::update_fast(w.x, a0, bd0, s0, dc, b0);

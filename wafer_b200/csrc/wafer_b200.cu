@@ -52,10 +52,10 @@ struct wafer_ctx {
     bool onfly = true;
     bool use_tb = false;            // time-tiled TMA sweep available (ThreePoint, V on the fly)
     CUtensorMap tm_psi[2], tm_v;    // TMA descriptors of the interior of psi[0], psi[1], v
-    double* hfield = nullptr;       // h = (dt*v)/2 for the time-tiled sweep (WAFER_TB_HFIELD), rebuilt when V changes
+    double* hfield = nullptr;       // h = (dt*v)/2 for the time-tiled sweep, rebuilt when V changes
     CUtensorMap tm_h;
     bool h_valid = false;
-    int den_ok = 0;
+    int den_ok = 0;                 // den_in_fast_window(denominator): the sweeps' fast division is exact
     std::map<std::pair<int, int>, Tb2Sched> tb2_sched;  // keyed by the plane range [xb, xe)
     bool use_t1 = false;            // TMA-pipelined one-step sweep (WAFER_FLAG_TMA_ONE_STEP)
     CUtensorMap t1_psi[2], t1_v, t1_h;
@@ -150,6 +150,9 @@ double denominator(const wafer_ctx* c) {
     const double k = c->p.ext == 1 ? 2. : (c->p.ext == 2 ? 24. : 360.);
     return k * c->p.dn * c->p.dn * c->p.mass;
 }
+
+// the exponent window of den in which tb::div_fast is exact (sweep_tb.cuh DivConst): 2^-100 < den < 2^100
+int den_in_fast_window(double den) { return den > 0x1p-100 && den < 0x1p100 ? 1 : 0; }
 
 int post_launch(wafer_ctx* ctx, int n = 1) {
     ctx->launches += n;
@@ -256,8 +259,6 @@ int init_tb(wafer_ctx* ctx) {
     CK(cudaFuncSetAttribute(tb::sweep_tb2_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tb::SMEM_BYTES));
     CK(cudaFuncSetAttribute(tb::sweep_tb2_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tb::SMEM_BYTES));
     CK(cudaFuncSetAttribute(tb::sweep_tb2_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tb::SMEM_BYTES));
-    const double den = denominator(ctx);
-    ctx->den_ok = (den > 7.888609052210118e-31 && den < 1.2676506002282294e30) ? 1 : 0;  // 2^-100 .. 2^100
     ctx->use_tb = true;
     return WAFER_OK;
 }
@@ -269,17 +270,18 @@ int init_tb(wafer_ctx* ctx) {
 //     CTAs drain through an atomic counter (in-order dispatch keeps neighbouring tiles close in time);
 //   * of the last chunk, the ntiles % G columns that would leave most SMs idle in a last partial wave are cut along x
 //     into at most G equal shares (even lengths, no stubs shorter than 6 planes): the static TAIL of each CTA.
+//   * few tile columns on many CTAs (fewer than 3/4 of a column per CTA: small planes, whose halos live in L2 anyway):
+//     no bulk, one contiguous static run of the columns x planes per CTA.
 // 512^3 on 148 SMs: one round of 148 columns + 14 columns cut 148 ways = 516 + ~53 plane-iterations per SM, against
-// 10 waves x 60 for round 1's uniform grid of 162 tiles x 9 chunks.  Measured (gpurun_out/r2f..r2j,
-// profiles/r2_tb2_variants.md): statically assigned rounds +4.8 % at 512^3 and +6 % on a 128-plane slab but -6 % at
-// 1024^3, where CTAs drift apart from round to round and the halo re-reads miss L2 (+17 % DRAM reads, ncu r2g); a fully
-// contiguous static split ("contig") -13 %.  WAFER_TB_SCHED=dynamic|rounds|legacy|contig selects the policy for A/B runs.
+// 10 waves x 60 for round 1's uniform grid of 162 tiles x 9 chunks.  The policies measured against this one (round 1's
+// grid, statically assigned rounds, one contiguous split everywhere) are in profiles/r2_tb2_variants.md.
 // pure host arithmetic (also behind wafer_tb2_plan for the CPU tests): bulk = in-order list, per[k] = static tail of CTA k
 struct Tb2Plan {
     std::vector<tb::Segment> bulk;
     std::vector<std::vector<tb::Segment>> per;
 };
-Tb2Plan tb2_plan(int ny, int nz, int xb, int xe, int slots, const std::string& mode, int MAXSEG) {
+constexpr int TB2_MAXSEG = 512;  // planes per x chunk of the bulk, at most
+Tb2Plan tb2_plan(int ny, int nz, int xb, int xe, int slots) {
     Tb2Plan pl;
     std::vector<tb::Segment>& bulk = pl.bulk;
     std::vector<std::vector<tb::Segment>>& per = pl.per;
@@ -311,61 +313,38 @@ Tb2Plan tb2_plan(int ny, int nz, int xb, int xe, int slots, const std::string& m
             }
         }
     };
-    if (mode == "legacy") {
-        // round 1's grid: tiles x chunks CTAs, one segment each, dispatched in order (here through the counter)
-        int best_nc = 1;
-        double best_cost = 1e300;
-        for (int nc = 1; nc <= std::min(P, 64); ++nc) {
-            const double cost = (double)ceil_div((long long)ntiles * nc, slots) * ((double)ceil_div(P, nc) + 3.0);
-            if (cost < best_cost * 0.999) { best_cost = cost; best_nc = nc; }
-        }
-        const int chunk = ceil_div(P, best_nc);
-        for (int c = 0; c * chunk < P; ++c)
-            for (int t = 0; t < ntiles; ++t) bulk.push_back(seg(t, xb + c * chunk, std::min(xe, xb + (c + 1) * chunk)));
-        G = (int)std::min<size_t>(slots, bulk.size());
-        per.resize(G);
-    } else if (mode == "contig" || (mode == "dynamic" && ntiles * 4 < G * 3)) {
+    if (ntiles * 4 < G * 3) {
         // few tile columns on many CTAs (small planes: every halo lives in L2 anyway): one contiguous static run each
         per.resize(G);
         cut_static(0, ntiles, xb, xe);
-    } else {
-        if (mode == "dynamic" && ntiles < G) G = ntiles;  // nearly one column per CTA: leave the few spare SMs idle, keep lock step
-        per.resize(G);
-        // number of x chunks: at least P / MAXSEG; a few more if that leaves a smaller statically cut tail.  The tail runs
-        // out of lock step (its halo re-reads miss L2), which the estimate charges with an empirical factor of 1.6.
-        int nchunk = ceil_div(P, MAXSEG);
-        if (mode == "dynamic" && ntiles >= G) {
-            double best = 1e300;
-            for (int nc = ceil_div(P, MAXSEG); nc <= ceil_div(P, MAXSEG) + 6 && nc * 32 <= P; ++nc) {
-                const int ch = (ceil_div(P, nc) + 1) & ~1;
-                const long long items = (long long)nc * ntiles, rest = items % G;
-                const double cost = (double)(items / G) * (ch + 4) + (rest ? ((double)rest * ch / G + 4) * 1.6 : 0.0);
-                if (cost < best * 0.999) { best = cost; nchunk = nc; }
-            }
-        }
-        const int chunk = (ceil_div(P, nchunk) + 1) & ~1;
-        const int R = ntiles / G;
-        for (int c = 0; c * chunk < P; ++c) {
-            const int ca = xb + c * chunk, cz = std::min(xe, ca + chunk);
-            if (mode == "rounds") {  // static assignment of whole columns, round by round
-                for (int r = 0; r < R; ++r)
-                    for (int k = 0; k < G; ++k) per[k].push_back(seg(r * G + k, ca, cz));
-                cut_static(R * G, ntiles - R * G, ca, cz);
-            } else {                 // "dynamic": in-order dispatch of whole columns, chunk after chunk
-                for (int t = 0; t < ntiles; ++t) bulk.push_back(seg(t, ca, cz));
-            }
-        }
-        if (mode != "rounds") {
-            // the bulk must come out even — a multiple of G columns — or the CTAs that drew one column more finish a whole
-            // column late: the last bulk.size() % G columns (all in the last chunk) are cut into G equal static shares
-            const int rest = std::min((int)(bulk.size() % G), ntiles);  // (never reaches back into an earlier chunk)
-            if (rest > 0) {
-                const tb::Segment f = bulk[bulk.size() - rest];
-                const int t0 = (f.y0 / tb::TY) * ntz + f.z0 / tb::TZ;
-                bulk.resize(bulk.size() - rest);
-                cut_static(t0, rest, f.xa, f.xz);
-            }
-        }
+        return pl;
+    }
+    if (ntiles < G) G = ntiles;  // nearly one column per CTA: leave the few spare SMs idle, keep lock step
+    per.resize(G);
+    // number of x chunks: at least P / TB2_MAXSEG; a few more if that leaves a smaller statically cut tail.  The tail runs
+    // out of lock step (its halo re-reads miss L2), which the estimate charges with an empirical factor of 1.6.
+    int nchunk = ceil_div(P, TB2_MAXSEG);
+    double best = 1e300;
+    for (int nc = ceil_div(P, TB2_MAXSEG); nc <= ceil_div(P, TB2_MAXSEG) + 6 && nc * 32 <= P; ++nc) {
+        const int ch = (ceil_div(P, nc) + 1) & ~1;
+        const long long items = (long long)nc * ntiles, rest = items % G;
+        const double cost = (double)(items / G) * (ch + 4) + (rest ? ((double)rest * ch / G + 4) * 1.6 : 0.0);
+        if (cost < best * 0.999) { best = cost; nchunk = nc; }
+    }
+    // in-order dispatch of whole columns, chunk after chunk
+    const int chunk = (ceil_div(P, nchunk) + 1) & ~1;
+    for (int c = 0; c * chunk < P; ++c) {
+        const int ca = xb + c * chunk, cz = std::min(xe, ca + chunk);
+        for (int t = 0; t < ntiles; ++t) bulk.push_back(seg(t, ca, cz));
+    }
+    // the bulk must come out even — a multiple of G columns — or the CTAs that drew one column more finish a whole
+    // column late: the last bulk.size() % G columns (all in the last chunk) are cut into G equal static shares
+    const int rest = std::min((int)(bulk.size() % G), ntiles);  // (never reaches back into an earlier chunk)
+    if (rest > 0) {
+        const tb::Segment f = bulk[bulk.size() - rest];
+        const int t0 = (f.y0 / tb::TY) * ntz + f.z0 / tb::TZ;
+        bulk.resize(bulk.size() - rest);
+        cut_static(t0, rest, f.xa, f.xz);
     }
     return pl;
 }
@@ -373,9 +352,7 @@ Tb2Plan tb2_plan(int ny, int nz, int xb, int xe, int slots, const std::string& m
 int tb2_schedule(wafer_ctx* ctx, int xb, int xe, const Tb2Sched** out) {
     auto it = ctx->tb2_sched.find({xb, xe});
     if (it != ctx->tb2_sched.end()) { *out = &it->second; return WAFER_OK; }
-    static const std::string mode = getenv("WAFER_TB_SCHED") ? getenv("WAFER_TB_SCHED") : "dynamic";
-    static const int MAXSEG = getenv("WAFER_TB_MAXSEG") ? std::max(8, atoi(getenv("WAFER_TB_MAXSEG"))) : 512;
-    const Tb2Plan pl = tb2_plan(ctx->g.ny, ctx->g.nz, xb, xe, ctx->sm_count * tb::CTAS_PER_SM, mode, MAXSEG);
+    const Tb2Plan pl = tb2_plan(ctx->g.ny, ctx->g.nz, xb, xe, ctx->sm_count * tb::CTAS_PER_SM);
     const std::vector<tb::Segment>& bulk = pl.bulk;
     std::vector<tb::Segment> flat;
     std::vector<int> first{0};
@@ -399,16 +376,9 @@ int tb2_schedule(wafer_ctx* ctx, int xb, int xe, const Tb2Sched** out) {
     return WAFER_OK;
 }
 
-// two lattice steps: psi[src] -> psi[src^1] for planes [xb, xe).  peer_lo / peer_hi != nullptr: the output planes
-// [xb, lo_end) / [hi_begin, xe) are also stored into the lower / upper neighbour's buffer, at plane + shift_lo / shift_hi.
-struct PeerTargets {
-    double* lo = nullptr;
-    double* hi = nullptr;
-    long long shift_lo = 0, shift_hi = 0;
-    int lo_end = INT_MIN, hi_begin = INT_MAX;
-};
-// The time-tiled sweep can read h = (dt*v)/2 instead of V: same bytes, two DMULs less per site and sweep pair, at the price
-// of one more field in HBM.  Built lazily on the main stream; every launch of the sweep is ordered after it there.
+// The time-tiled sweep reads h = (dt*v)/2 instead of V: same bytes, two DMULs less per site and sweep pair, at the price
+// of one more field in HBM.  Built lazily on the main stream; every launch of the sweep is ordered after it there.  Until
+// h exists (evolves of fewer than 4 steps) or when there is no room for it, the sweep reads V.
 // The one-step TMA sweeps can read h too (WAFER_T1_HFIELD=1); measured: no difference for them (5/7-point, excited
 // steps within 0.5 %, gpurun_out/r2z) — they are not limited by those two multiplications — so it is off by default.
 bool t1_reads_h() {
@@ -417,8 +387,7 @@ bool t1_reads_h() {
 }
 
 int ensure_hfield(wafer_ctx* ctx) {
-    static const bool want = !(getenv("WAFER_TB_HFIELD") && atoi(getenv("WAFER_TB_HFIELD")) == 0);
-    if (!want || ctx->h_valid) return WAFER_OK;
+    if (ctx->h_valid) return WAFER_OK;
     if (!ctx->hfield) {
         if (cudaMalloc(&ctx->hfield, ctx->bytes()) != cudaSuccess) { cudaGetLastError(); ctx->hfield = nullptr; return WAFER_OK; }  // no room: keep V
         TRY(make_tensor_map(ctx, &ctx->tm_h, ctx->hfield, tb::R1));
@@ -434,7 +403,9 @@ int ensure_hfield(wafer_ctx* ctx) {
     return WAFER_OK;
 }
 
-int launch_sweep_tb2(wafer_ctx* ctx, int src, int xb, int xe, cudaStream_t st, const PeerTargets* pt = nullptr) {
+// two lattice steps: psi[src] -> psi[src^1] for planes [xb, xe); pr != nullptr: also store the boundary planes it names
+// into the neighbours' ghost planes (fused halo)
+int launch_sweep_tb2(wafer_ctx* ctx, int src, int xb, int xe, cudaStream_t st, const tb::PeerStores* pr = nullptr) {
     if (xe <= xb) return WAFER_OK;
     const Geom& g = ctx->g;
     const bool hf = ctx->h_valid;
@@ -442,12 +413,9 @@ int launch_sweep_tb2(wafer_ctx* ctx, int src, int xb, int xe, cudaStream_t st, c
     TRY(tb2_schedule(ctx, xb, xe, &sc));
     double* out = ctx->psi[src ^ 1];
     const tb::Sched ks{sc->bulk, sc->nbulk, sc->segs, sc->first, sc->counters};
-    if (pt && (pt->lo || pt->hi)) {
-        tb::PeerStores pr{0, 0, INT_MIN, INT_MAX};
-        if (pt->lo) { pr.delta_lo = (pt->lo - out) + pt->shift_lo * g.plane; pr.lo_end = pt->lo_end; }
-        if (pt->hi) { pr.delta_hi = (pt->hi - out) + pt->shift_hi * g.plane; pr.hi_begin = pt->hi_begin; }
-        if (hf) tb::sweep_tb2_kernel<true, true><<<sc->ncta, tb::THREADS, tb::SMEM_BYTES, st>>>(ctx->tm_psi[src], ctx->tm_h, out, pr, g, ks, ctx->p.dt, denominator(ctx), ctx->den_ok);
-        else tb::sweep_tb2_kernel<true, false><<<sc->ncta, tb::THREADS, tb::SMEM_BYTES, st>>>(ctx->tm_psi[src], ctx->tm_v, out, pr, g, ks, ctx->p.dt, denominator(ctx), ctx->den_ok);
+    if (pr) {
+        if (hf) tb::sweep_tb2_kernel<true, true><<<sc->ncta, tb::THREADS, tb::SMEM_BYTES, st>>>(ctx->tm_psi[src], ctx->tm_h, out, *pr, g, ks, ctx->p.dt, denominator(ctx), ctx->den_ok);
+        else tb::sweep_tb2_kernel<true, false><<<sc->ncta, tb::THREADS, tb::SMEM_BYTES, st>>>(ctx->tm_psi[src], ctx->tm_v, out, *pr, g, ks, ctx->p.dt, denominator(ctx), ctx->den_ok);
     } else {
         const tb::PeerStores none{};
         if (hf) tb::sweep_tb2_kernel<false, true><<<sc->ncta, tb::THREADS, tb::SMEM_BYTES, st>>>(ctx->tm_psi[src], ctx->tm_h, out, none, g, ks, ctx->p.dt, denominator(ctx), ctx->den_ok);
@@ -498,8 +466,6 @@ int init_t1(wafer_ctx* ctx) {
     if (ctx->p.ext == 1) TRY(init_t1_e<1>(ctx));
     else if (ctx->p.ext == 2) TRY(init_t1_e<2>(ctx));
     else TRY(init_t1_e<3>(ctx));
-    const double den = denominator(ctx);
-    ctx->den_ok = (den > 7.888609052210118e-31 && den < 1.2676506002282294e30) ? 1 : 0;
     ctx->use_t1 = true;
     return WAFER_OK;
 }
@@ -1052,6 +1018,7 @@ int create_impl(const wafer_params* params, wafer_ctx* ctx) {
     CK(cudaMemsetAsync(ctx->scal, 0, SL_COUNT * sizeof(double), ctx->s_main));
     CK(cudaMallocHost(&ctx->h_scal, SL_COUNT * sizeof(double)));
     CK(cudaMalloc(&ctx->ring_flag, sizeof(int)));
+    ctx->den_ok = den_in_fast_window(denominator(ctx));
     TRY(init_tb(ctx));
     TRY(init_t1(ctx));
 
@@ -1155,7 +1122,7 @@ int wafer_slab_partition(uint64_t nx, uint32_t world, uint32_t rank, uint64_t* x
 int wafer_tb2_plan(uint32_t ny, uint32_t nz, int32_t xb, int32_t xe, uint32_t slots, int32_t* segments, uint64_t cap, uint64_t* n) {
     if (!n || ny == 0 || nz == 0 || xe <= xb || slots == 0) return WAFER_ERR_INVALID;
     try {
-        const Tb2Plan pl = tb2_plan((int)ny, (int)nz, xb, xe, (int)slots, "dynamic", 512);
+        const Tb2Plan pl = tb2_plan((int)ny, (int)nz, xb, xe, (int)slots);
         uint64_t k = 0;
         auto put = [&](int owner, const tb::Segment& sg) {
             if (segments && k < cap) {
@@ -1536,11 +1503,10 @@ static int excited_step(wafer_ctx* ctx, int wnum) {
 
 
 // `pairs` times two excited-state steps through a captured graph.  Returns WAFER_OK with *ran = false when graphs are not
-// to be used (several ranks, switched off, or the capture failed: the caller then steps the ordinary way).
+// to be used (several ranks, or the capture failed: the caller then steps the ordinary way).
 static int excited_pairs_graph(wafer_ctx* ctx, int wnum, uint64_t pairs, bool* ran) {
     *ran = false;
-    static const bool on = !(getenv("WAFER_GRAPHS") && atoi(getenv("WAFER_GRAPHS")) == 0);
-    if (!on || ctx->world != 1 || pairs == 0) return WAFER_OK;
+    if (ctx->world != 1 || pairs == 0) return WAFER_OK;
     const std::pair<int, int> key{wnum, ctx->cur};
     auto it = ctx->step_graphs.find(key);
     if (it == ctx->step_graphs.end()) {
@@ -1611,14 +1577,13 @@ static int wafer_evolve_impl(wafer_ctx* ctx, uint8_t wnum_in, uint64_t steps) {
         const int src = ctx->cur;
         const double* cur = ctx->psi[src];
         double* nxt = ctx->psi[src ^ 1];
-        // Fused halos, two-step pass, "whole column" form (default): ONE launch on the main stream sweeps all owned planes and
+        // Fused halos, two-step pass, "whole column" form: ONE launch on the main stream sweeps all owned planes and
         // stores its first / last two output planes into the neighbours' ghost planes as it produces them; the neighbours'
         // pass counters are awaited before it and published after it.  No separate boundary launches: those produce 2 planes
         // for 6 plane-iterations of pipeline (140 instead of 132 iterations per tile column at 128 planes per rank, and four
         // small launches that the persistent interior kernel serialises behind itself anyway — 0.894 parallel efficiency at
         // N = 8, profiles/scaling_r2).  The price is a per-pass handshake between neighbours instead of a pass of slack.
-        static const bool split_halo = getenv("WAFER_P2P_SPLIT") && atoi(getenv("WAFER_P2P_SPLIT")) == 1;
-        if (fused && two && !split_halo) {
+        if (fused && two) {
             CK(cudaStreamWaitEvent(ctx->s_main, ctx->ev_halo, 0));  // an earlier pass may have used the halo stream
             if (ctx->dbg_halo_delay_ns) {
                 spin_kernel<<<1, 1, 0, ctx->s_main>>>(ctx->dbg_halo_delay_ns);
@@ -1628,17 +1593,19 @@ static int wafer_evolve_impl(wafer_ctx* ctx, uint8_t wnum_in, uint64_t steps) {
             // and they no longer read the ghost planes (of their `nxt`) that this pass overwrites
             p2p_wait_kernel<<<1, 1, 0, ctx->s_main>>>(ctx->flags, ctx->pass, has_lo, has_hi, ctx->p2p_timeout);
             TRY(post_launch(ctx));
-            PeerTargets pt;
-            if (has_lo) { pt.lo = ctx->peer_psi[0][src ^ 1]; pt.shift_lo = ctx->peer_L[0]; pt.lo_end = b; }
-            if (has_hi) { pt.hi = ctx->peer_psi[1][src ^ 1]; pt.shift_hi = -(long long)g.L; pt.hi_begin = g.L - b; }
-            TRY(launch_sweep_tb2(ctx, src, 0, g.L, ctx->s_main, &pt));
+            // my planes [0,b) are the lower neighbour's ghost planes [L_lo, L_lo+b); my [L-b,L) the upper one's [-b,0)
+            tb::PeerStores pr{0, 0, INT_MIN, INT_MAX};
+            if (has_lo) { pr.delta_lo = (ctx->peer_psi[0][src ^ 1] - nxt) + (long long)ctx->peer_L[0] * g.plane; pr.lo_end = b; }
+            if (has_hi) { pr.delta_hi = (ctx->peer_psi[1][src ^ 1] - nxt) - (long long)g.L * g.plane; pr.hi_begin = g.L - b; }
+            TRY(launch_sweep_tb2(ctx, src, 0, g.L, ctx->s_main, &pr));
             ctx->pass += 1;
             p2p_signal_kernel<<<1, 1, 0, ctx->s_main>>>(has_lo ? ctx->peer_flags[0] : nullptr, has_hi ? ctx->peer_flags[1] : nullptr, ctx->pass);
             TRY(post_launch(ctx));
             CK(cudaEventRecord(ctx->ev_main, ctx->s_main));
             CK(cudaEventRecord(ctx->ev_halo, ctx->s_main));
         } else if (overlap) {
-            // boundary planes + halo on the high-priority stream, interior on the main stream
+            // boundary planes + halo on the high-priority stream, interior on the main stream (a two-step pass gets here only
+            // with the NCCL halo: with fused halos it takes the branch above)
             CK(cudaStreamWaitEvent(ctx->s_halo, ctx->ev_main, 0));
             CK(cudaStreamWaitEvent(ctx->s_main, ctx->ev_halo, 0));
             if (ctx->dbg_halo_delay_ns) {
@@ -1651,15 +1618,9 @@ static int wafer_evolve_impl(wafer_ctx* ctx, uint8_t wnum_in, uint64_t steps) {
                 p2p_wait_kernel<<<1, 1, 0, ctx->s_halo>>>(ctx->flags, ctx->pass, has_lo, has_hi, ctx->p2p_timeout);
                 TRY(post_launch(ctx));
             }
-            double* plo = fused && has_lo ? ctx->peer_psi[0][src ^ 1] : nullptr;
-            double* phi_ = fused && has_hi ? ctx->peer_psi[1][src ^ 1] : nullptr;
             if (two) {
-                // my planes [0,b) are the lower neighbour's ghost planes [L_lo, L_lo+b); my [L-b,L) the upper one's [-b,0)
-                PeerTargets lo_t, hi_t;
-                if (plo) { lo_t.lo = plo; lo_t.shift_lo = ctx->peer_L[0]; lo_t.lo_end = b; }
-                if (phi_) { hi_t.hi = phi_; hi_t.shift_hi = -(long long)g.L; hi_t.hi_begin = g.L - b; }
-                TRY(launch_sweep_tb2(ctx, src, 0, b, ctx->s_halo, &lo_t));
-                TRY(launch_sweep_tb2(ctx, src, g.L - b, g.L, ctx->s_halo, &hi_t));
+                TRY(launch_sweep_tb2(ctx, src, 0, b, ctx->s_halo));
+                TRY(launch_sweep_tb2(ctx, src, g.L - b, g.L, ctx->s_halo));
             } else {
                 // (final step with fused check sums: the three launches share one row of per-CTA partial sums)
                 const int nb_lo = sweep_blocks(ctx, 0, b), nb_hi = sweep_blocks(ctx, g.L - b, g.L);
@@ -1668,8 +1629,8 @@ static int wafer_evolve_impl(wafer_ctx* ctx, uint8_t wnum_in, uint64_t steps) {
                 TRY(launch_sweep(ctx, cur, nxt, g.L - b, g.L, chk_mode, 0, ctx->s_halo, chk_nb, nb_lo));
                 if (fused) {  // rare odd tail step: plain peer copies of the boundary planes
                     const size_t bytes = (size_t)b * g.plane * sizeof(double);
-                    if (plo) CK(cudaMemcpyAsync(plo + g.off(ctx->peer_L[0], -g.e, 0), nxt + g.off(0, -g.e, 0), bytes, cudaMemcpyDeviceToDevice, ctx->s_halo));
-                    if (phi_) CK(cudaMemcpyAsync(phi_ + g.off(-b, -g.e, 0), nxt + g.off(g.L - b, -g.e, 0), bytes, cudaMemcpyDeviceToDevice, ctx->s_halo));
+                    if (has_lo) CK(cudaMemcpyAsync(ctx->peer_psi[0][src ^ 1] + g.off(ctx->peer_L[0], -g.e, 0), nxt + g.off(0, -g.e, 0), bytes, cudaMemcpyDeviceToDevice, ctx->s_halo));
+                    if (has_hi) CK(cudaMemcpyAsync(ctx->peer_psi[1][src ^ 1] + g.off(-b, -g.e, 0), nxt + g.off(g.L - b, -g.e, 0), bytes, cudaMemcpyDeviceToDevice, ctx->s_halo));
                 }
             }
             if (fused) {
@@ -1698,8 +1659,7 @@ static int wafer_evolve_impl(wafer_ctx* ctx, uint8_t wnum_in, uint64_t steps) {
         done += two ? 2 : 1;
     }
     if (overlap) {
-        static const bool skip_final_wait = getenv("WAFER_DEBUG_SKIP_FINAL_WAIT") && atoi(getenv("WAFER_DEBUG_SKIP_FINAL_WAIT")) == 1;
-        if (fused && !skip_final_wait) {  // the env knob exists only so that the drift test can prove it catches the race
+        if (fused) {
             // The neighbours' boundary stores of the LAST pass must have landed in my ghost planes before anything
             // that follows on the main stream reads them (observables, Gram-Schmidt, downloads, w_store.push) or
             // overwrites them (normalise, uploads): wait for their pass counter to reach mine.  Without this a rank
@@ -1911,8 +1871,7 @@ int wafer_selftest_division(wafer_ctx* ctx, double den, uint64_t n, uint64_t see
     unsigned long long* d = nullptr;
     CK(cudaMalloc(&d, sizeof(unsigned long long)));
     CK(cudaMemsetAsync(d, 0, sizeof(unsigned long long), ctx->s_main));
-    const int ok = (den > 7.888609052210118e-31 && den < 1.2676506002282294e30) ? 1 : 0;
-    tb::div_selftest_kernel<<<ctx->sm_count * 8, 256, 0, ctx->s_main>>>(den, ok, n, seed, d);
+    tb::div_selftest_kernel<<<ctx->sm_count * 8, 256, 0, ctx->s_main>>>(den, den_in_fast_window(den), n, seed, d);
     TRY(post_launch(ctx));
     unsigned long long h = 0;
     CK(cudaMemcpyAsync(&h, d, sizeof(h), cudaMemcpyDeviceToHost, ctx->s_main));
