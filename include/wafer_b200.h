@@ -40,7 +40,8 @@ typedef enum {
     WAFER_ERR_RING_NONZERO = 5, /* wafer_set_phi / wafer_push_lower: padding ring not 0 (config.rs:597-622)      */
     WAFER_ERR_NOT_READY = 6,    /* potential or phi not set yet                                                */
     WAFER_ERR_MAX_STEP = 7,     /* wafer_solve: not converged within max_steps (errors.rs MaxStep, grid.rs:244) */
-    WAFER_ERR_NONFINITE = 8     /* NaN/Inf met where the reference's R64 would panic (noisy_float)             */
+    WAFER_ERR_NONFINITE = 8,    /* NaN/Inf met where the reference's R64 would panic (noisy_float)             */
+    WAFER_ERR_IO = 9            /* a file could not be created or written; see wafer_last_error               */
 } wafer_status;
 
 /* flags */
@@ -143,6 +144,24 @@ int wafer_symmetrise(wafer_ctx *ctx, int32_t kind);
 int wafer_set_phi_resampled(wafer_ctx *ctx, const double *src, uint64_t sx, uint64_t sy, uint64_t sz, uint32_t from_csv);
 int wafer_set_potential_resampled(wafer_ctx *ctx, const double *src, uint64_t sx, uint64_t sy, uint64_t sz, uint32_t from_csv);
 int wafer_push_lower_resampled(wafer_ctx *ctx, const double *src, uint64_t sx, uint64_t sy, uint64_t sz, uint32_t from_csv);
+
+/* -------- array files ------------------------------------------------------------------------------ */
+typedef struct {
+    uint64_t bytes;          /* bytes this rank wrote (its sites, plus the preamble on rank 0 and Json's "]}" on the last) */
+    uint64_t file_bytes;     /* size of the whole file                                                                 */
+    uint64_t host_formatted; /* this rank's sites whose %.17g text was made by snprintf on the host (exact ties)        */
+} wafer_write_stats;
+/* output::wavefunction / output::potential (output.rs:79-216): the WORK area of psi (what = 0) or V (what = 1) to `path`
+   (extension included) as file_type 0 Messagepack, 1 Csv, 2 Json, byte for byte formats.hpp's write_mpk / write_csv /
+   write_json (numbers as "%.17g").  The file is encoded on the device, chunk by chunk through the bounce buffers, and
+   written with pwrite while the next chunk is encoded; no field-sized buffer is allocated on either side.  Ordered after
+   the work already queued on the context; psi, V and the fused check sums are left as they are.
+   COLLECTIVE when world > 1: every rank passes the same path and writes its planes at their offset of the one file
+   (the file system must be shared by the ranks, e.g. one host).  If any rank cannot create the file, no rank writes and
+   all return WAFER_ERR_IO; a failed write on one rank makes every rank return WAFER_ERR_IO.
+   WAFER_ERR_INVALID, nothing created: unknown what or file_type (Yaml / Ron), NULL path, Messagepack of more than
+   2^32-1 sites (its array32 header cannot count them).  WAFER_ERR_NOT_READY without psi / V.  stats may be NULL. */
+int wafer_write_array(wafer_ctx *ctx, int32_t what, int32_t file_type, const char *path, wafer_write_stats *stats);
 
 /* -------- the hot path -------------------------------------------------------------------------- */
 int wafer_observables_compute(wafer_ctx *ctx, wafer_observables *out); /* compute_observables        (grid.rs:303-445) */

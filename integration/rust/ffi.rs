@@ -6,7 +6,7 @@
 use errors::*;
 use ndarray::Array3;
 use noisy_float::prelude::*;
-use std::ffi::CStr;
+use std::ffi::{CStr, CString};
 use std::os::raw::{c_char, c_int, c_void};
 use std::ptr;
 
@@ -36,6 +36,14 @@ pub struct WaferObservables {
     pub r2: f64,
 }
 
+#[repr(C)]
+#[derive(Default, Debug, Clone, Copy)]
+pub struct WaferWriteStats {
+    pub bytes: u64,
+    pub file_bytes: u64,
+    pub host_formatted: u64,
+}
+
 pub enum WaferCtx {}
 
 extern "C" {
@@ -59,6 +67,7 @@ extern "C" {
     fn wafer_check(ctx: *mut WaferCtx, wnum: u8, out: *mut WaferObservables) -> c_int;
     fn wafer_normalise(ctx: *mut WaferCtx, norm2: f64) -> c_int;
     fn wafer_evolve(ctx: *mut WaferCtx, wnum: u8, steps: u64) -> c_int;
+    fn wafer_write_array(ctx: *mut WaferCtx, what: i32, file_type: i32, path: *const c_char, stats: *mut WaferWriteStats) -> c_int;
     fn wafer_synchronize(ctx: *mut WaferCtx) -> c_int;
     fn wafer_host_register(ptr: *mut c_void, bytes: usize) -> c_int;
     fn wafer_host_unregister(ptr: *mut c_void) -> c_int;
@@ -165,6 +174,15 @@ impl Gpu {
     }
     pub fn evolve(&self, wnum: u8, steps: u64) -> Result<()> {
         self.check(unsafe { wafer_evolve(self.ctx, wnum, steps) })
+    }
+    /// output::wavefunction / output::potential (output.rs:79-216) encoded on the device: the work area of psi
+    /// (`what` 0) or V (1) to `path` as `file_type` 0 Messagepack, 1 Csv, 2 Json (`FileType as i32`; Yaml / Ron are
+    /// refused).  Collective when world > 1: every rank passes the same path and writes its planes into the one file.
+    pub fn write_array(&self, what: i32, file_type: i32, path: &str) -> Result<WaferWriteStats> {
+        let c = CString::new(path).map_err(|_| Error::from("output path contains a NUL byte"))?;
+        let mut st = WaferWriteStats::default();
+        self.check(unsafe { wafer_write_array(self.ctx, what, file_type, c.as_ptr(), &mut st) })?;
+        Ok(st)
     }
     /// Page-lock the buffer behind `arr` so that set_phi / get_phi run at PCIe speed (54 GB/s measured instead of the
     /// driver's 14 GB/s pageable path).  Call once after allocating the array; `unpin` before it is dropped.

@@ -6,14 +6,15 @@ Arrays are numpy float64 in the reference's padded Array3 layout.  Every call go
 wafer_b200/libwafer_b200.so (include/wafer_b200.h); nothing here computes on the CPU.
 """
 import ctypes as C
+import os
 
 import numpy as np
 
 from . import _capi
-from ._capi import Observables, Params, Record
+from ._capi import Observables, Params, Record, WriteStats
 
 __all__ = ["Lattice", "slab_partition", "tb2_plan", "WaferError", "POTENTIALS", "INITIAL_CONDITIONS", "SYMMETRIES", "EXT",
-           "nccl_unique_id", "pinned_empty", "pin", "unpin", "FLAG_AB_ARRAYS"]
+           "nccl_unique_id", "pinned_empty", "pin", "unpin", "FLAG_AB_ARRAYS", "FILE_TYPES"]
 
 # PotentialType (config.rs:74-104), InitialCondition (config.rs:153-170), SymmetryConstraint (config.rs:186-197),
 # CentralDifference.ext() (config.rs:232-238)
@@ -22,6 +23,7 @@ POTENTIALS = {
     "ElipticalCoulomb": 6, "SimpleCornell": 7, "FullCornell": 8, "Harmonic": 9, "ComplexHarmonic": 10,
     "Dodecahedron": 11, "FromFile": 12, "FromScript": 13, "PoschlTeller": 100,
 }
+FILE_TYPES = {"Messagepack": 0, "Csv": 1, "Json": 2}
 INITIAL_CONDITIONS = {"FromFile": 0, "Gaussian": 1, "Coulomb": 2, "Constant": 3, "Boolean": 4}
 SYMMETRIES = {"NotConstrained": 0, "AboutZ": 1, "AntisymAboutZ": 2, "AboutY": 3, "AntisymAboutY": 4}
 EXT = {"ThreePoint": 1, "FivePoint": 2, "SevenPoint": 3}
@@ -30,7 +32,7 @@ FLAG_SIMPLE_SWEEP = 0x4
 FLAG_TMA_ONE_STEP = 0x8
 
 _STATUS = {1: "INVALID", 2: "NO_DEVICE", 3: "CUDA", 4: "NCCL", 5: "RING_NONZERO", 6: "NOT_READY", 7: "MAX_STEP",
-           8: "NONFINITE"}
+           8: "NONFINITE", 9: "IO"}
 _dp = C.POINTER(C.c_double)
 
 
@@ -331,6 +333,18 @@ class Lattice:
     @property
     def num_lowers(self):
         return int(self._lib.wafer_num_lowers(self._h))
+
+    # ---- array files: output::wavefunction / output::potential (output.rs:79-216), encoded on the device
+    def write_array(self, what, path, file_type):
+        """Write the work area of psi (what="phi" or 0) or V ("potential" or 1) to `path` (extension included) as
+        file_type "Messagepack" / "Csv" / "Json" (or 0 / 1 / 2), byte for byte the front end's formats.hpp writers.
+        Collective when world > 1: every rank passes the same path and writes its planes into the one file.
+        Returns dict(bytes=this rank's bytes, file_bytes=size of the file, host_formatted=sites formatted on the host)."""
+        w = {"phi": 0, "potential": 1}[what] if isinstance(what, str) else int(what)
+        ft = FILE_TYPES[file_type] if isinstance(file_type, str) else int(file_type)
+        st = WriteStats()
+        self._ck(self._lib.wafer_write_array(self._h, w, ft, os.fsencode(path), C.byref(st)))
+        return dict(bytes=st.bytes, file_bytes=st.file_bytes, host_formatted=st.host_formatted)
 
     # ---- the hot path, reference names (grid.rs)
     def compute_observables(self):

@@ -24,6 +24,10 @@ class Record(C.Structure):
     _fields_ = [("step", C.c_uint64), ("tau", C.c_double), ("diff", C.c_double), ("obs", Observables)]
 
 
+class WriteStats(C.Structure):
+    _fields_ = [("bytes", C.c_uint64), ("file_bytes", C.c_uint64), ("host_formatted", C.c_uint64)]
+
+
 # every symbol include/wafer_b200.h declares: name -> (restype, argtypes)
 _ctx = C.c_void_p
 SYMBOLS = {
@@ -60,6 +64,7 @@ SYMBOLS = {
     "wafer_set_phi_resampled": (C.c_int, [_ctx, _dp, C.c_uint64, C.c_uint64, C.c_uint64, C.c_uint32]),
     "wafer_set_potential_resampled": (C.c_int, [_ctx, _dp, C.c_uint64, C.c_uint64, C.c_uint64, C.c_uint32]),
     "wafer_push_lower_resampled": (C.c_int, [_ctx, _dp, C.c_uint64, C.c_uint64, C.c_uint64, C.c_uint32]),
+    "wafer_write_array": (C.c_int, [_ctx, C.c_int32, C.c_int32, C.c_char_p, C.POINTER(WriteStats)]),
     "wafer_observables_compute": (C.c_int, [_ctx, C.POINTER(Observables)]),
     "wafer_norm2": (C.c_int, [_ctx, _dp]),
     "wafer_normalise": (C.c_int, [_ctx, C.c_double]),

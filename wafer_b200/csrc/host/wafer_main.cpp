@@ -2,8 +2,8 @@
 //
 // Same wafer.yaml, same CLI flags (-c/--config, -s/--script, -d), same per-state loop, same table rows
 // (output.rs:497-521) and observables record (output.rs:32-45, 533-547).  Everything numerical happens in
-// libwafer_b200.so on the GPU; this file is host glue: configuration, potential / initial-condition selection,
-// CSV / JSON files (the plain-text members of the reference's five formats), printing.
+// libwafer_b200.so on the GPU, the array files included (wafer_write_array); this file is host glue: configuration,
+// potential / initial-condition selection, the observables files, printing.
 //
 //   wafer-b200 -c wafer.yaml                 run (one process per GPU; RANK / WORLD_SIZE / LOCAL_RANK select a slab)
 //   wafer-b200 -c wafer.yaml --check-config  parse + validate only, print the configuration as JSON (no GPU needed)
@@ -49,12 +49,9 @@ std::string ordinal(unsigned n) {
     return std::to_string(n) + suf;
 }
 
-// array files: work area out (output.rs:79-216); in, the file's array as parsed (input.rs:32-127, 513-662), which the
-// wafer_*_resampled entries embed on the device as fill_data / read_csv do (input.rs:149-176, 641-657; formats.hpp
-// embed_work is the host restatement).  from_csv: the file read was a Csv file.
-void write_work(const std::string& stem, int file_type, const double* padded, const Dims& d) {
-    write_array(stem, file_type, extract_work(padded, d.nx, d.ny, d.nz, d.e));
-}
+// array files in: the file's array as parsed (input.rs:32-127, 513-662), which the wafer_*_resampled entries embed on
+// the device as fill_data / read_csv do (input.rs:149-176, 641-657; formats.hpp embed_work is the host restatement).
+// from_csv: the file read was a Csv file.  Out: wafer_write_array (write_array_file below).
 bool read_input(const std::string& stem, int file_type, const Dims& d, Array3& a, uint32_t& from_csv) {
     int used = 0;
     if (!read_array(stem, file_type, a, &used)) return false;
@@ -170,14 +167,16 @@ void write_observables(const Run& r, unsigned wnum, const wafer_observables& o) 
     fclose(f);
 }
 
+// output.rs:79-216: the work area of psi (what 0) or V (what 1), encoded on the device, formats.hpp's bytes.  With
+// world > 1 every rank calls it and writes its planes into the one file.
+void write_array_file(const Run& r, int what, const std::string& stem) {
+    if (r.cfg.file_type > 2) throw std::runtime_error("output.file_type Yaml / Ron is not supported by this build (use Messagepack, Csv or Json)");
+    r.ck(wafer_write_array(r.ctx, what, r.cfg.file_type, (stem + extension(r.cfg.file_type)).c_str(), nullptr), "wafer_write_array");
+}
+
 void save_wavefunction(const Run& r, unsigned wnum, bool converged) {
     if (r.outdir.empty()) return;
-    const Dims d(r.cfg);
-    std::vector<double> phi(d.padded(), 0.0);
-    r.ck(wafer_get_phi(r.ctx, phi.data()), "wafer_get_phi");
-    std::string name = r.outdir + "/wavefunction_" + std::to_string(wnum) + (converged ? "" : "_partial");
-    if (r.world > 1) name += ".rank" + std::to_string(r.rank);  // each rank holds (and writes) only its slab
-    write_work(name, r.cfg.file_type, phi.data(), d);
+    write_array_file(r, 0, r.outdir + "/wavefunction_" + std::to_string(wnum) + (converged ? "" : "_partial"));
 }
 
 // grid.rs:50-246 for one state; returns true when converged
@@ -227,24 +226,23 @@ bool solve(Run& r, unsigned wnum) {
     if (converged) {
         if (!r.quiet && r.rank == 0) printf("═════╧════════════╧════════════════════╧════════════════╧════════════════╧═════\n");
         if (r.rank == 0) write_observables(r, wnum, obs);
-        if (c.snap_update && !r.outdir.empty()) {                                                        // grid.rs:174-190
-            std::string partial = r.outdir + "/wavefunction_" + std::to_string(wnum) + "_partial";
-            if (r.world > 1) partial += ".rank" + std::to_string(r.rank);
-            unlink((partial + extension(c.file_type)).c_str());
-        }
+        if (c.snap_update && !r.outdir.empty() && r.rank == 0)                                           // grid.rs:174-190
+            unlink((r.outdir + "/wavefunction_" + std::to_string(wnum) + "_partial" + extension(c.file_type)).c_str());
     }
     if (c.save_wavefns) save_wavefunction(r, wnum, converged);                                           // grid.rs:223-237
     if (converged) r.ck(wafer_push_lower_from_phi(r.ctx), "wafer_push_lower_from_phi");                  // grid.rs:241
     return converged;
 }
 
-// rank 0 writes the ncclUniqueId to a file, the others poll for it (no MPI / torch needed)
-void rendezvous(const std::string& path, int rank, uint8_t id[128]) {
+// rank 0 writes the ncclUniqueId and its output directory (empty: none) to a file, the others poll for it (no MPI /
+// torch needed); every rank writes its planes of the array files there
+void rendezvous(const std::string& path, int rank, uint8_t id[128], std::string& outdir) {
     if (rank == 0) {
         if (wafer_nccl_unique_id(id) != WAFER_OK) throw std::runtime_error(std::string("wafer_nccl_unique_id: ") + wafer_last_error(nullptr));
         const std::string tmp = path + ".tmp";
         FILE* f = fopen(tmp.c_str(), "wb");
-        if (!f || fwrite(id, 1, 128, f) != 128) throw std::runtime_error("rendezvous: cannot write " + tmp);
+        if (!f || fwrite(id, 1, 128, f) != 128 || fwrite(outdir.data(), 1, outdir.size(), f) != outdir.size())
+            throw std::runtime_error("rendezvous: cannot write " + tmp);
         fclose(f);
         rename(tmp.c_str(), path.c_str());
     } else {
@@ -252,8 +250,13 @@ void rendezvous(const std::string& path, int rank, uint8_t id[128]) {
             FILE* f = fopen(path.c_str(), "rb");
             if (f) {
                 const size_t n = fread(id, 1, 128, f);
+                char buf[4096];
+                const size_t m = n == 128 ? fread(buf, 1, sizeof buf, f) : 0;
                 fclose(f);
-                if (n == 128) return;
+                if (n == 128) {
+                    outdir.assign(buf, m);
+                    return;
+                }
             }
             std::this_thread::sleep_for(std::chrono::milliseconds(100));
         }
@@ -358,8 +361,6 @@ int main(int argc, char** argv) {
         const Config& c = r.cfg;
         r.rank = env_int("RANK", 0);
         r.world = env_int("WORLD_SIZE", 1);
-        uint8_t id[128];
-        if (r.world > 1) rendezvous(rdv.empty() ? "/tmp/wafer_b200_nccl_id_" + std::to_string(getppid()) : rdv, r.rank, id);
         if (!no_output && r.rank == 0) {
             // output::check_output_dir (output.rs:680-745): ./output/<project>_<date>/ + a copy of the configuration
             char date[64];
@@ -372,6 +373,8 @@ int main(int argc, char** argv) {
             std::ofstream dst(r.outdir + "/wafer.yaml", std::ios::binary);
             dst << src.rdbuf();
         }
+        uint8_t id[128];
+        if (r.world > 1) rendezvous(rdv.empty() ? "/tmp/wafer_b200_nccl_id_" + std::to_string(getppid()) : rdv, r.rank, id, r.outdir);
         wafer_params p{};
         p.nx = c.nx; p.ny = c.ny; p.nz = c.nz; p.ext = (uint32_t)c.ext();
         p.dn = c.dn; p.dt = c.dt; p.mass = c.mass;
@@ -402,11 +405,7 @@ int main(int argc, char** argv) {
             const double ps = c.potential == 6 ? 1. / c.dn : (c.potential == 7 ? 4.0 * c.mass : 0.0);
             r.ck(wafer_set_pot_sub_scalar(r.ctx, ps), "wafer_set_pot_sub_scalar");
         }
-        if (c.save_potential && !r.outdir.empty() && r.rank == 0) {  // potential.rs:163-172
-            std::vector<double> v(d.padded());
-            r.ck(wafer_get_potential(r.ctx, v.data()), "wafer_get_potential");
-            if (r.world == 1) write_work(r.outdir + "/potential", c.file_type, v.data(), d);
-        }
+        if (c.save_potential && !r.outdir.empty()) write_array_file(r, 1, r.outdir + "/potential");  // potential.rs:163-172
 
         // run (grid.rs:31-47): lower states from ./input when starting above the ground state
         for (unsigned w = 0; w < c.wavenum; ++w) {  // input::load_wavefunctions (input.rs:487-505)

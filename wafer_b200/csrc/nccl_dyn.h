@@ -10,7 +10,7 @@ namespace wafer {
 
 struct NcclUniqueId { char internal[128]; };
 typedef struct ncclComm* NcclComm;
-enum { kNcclSuccess = 0, kNcclFloat64 = 8, kNcclSum = 0 };
+enum { kNcclSuccess = 0, kNcclUint64 = 5, kNcclFloat64 = 8, kNcclSum = 0 };
 
 struct NcclApi {
     void* handle = nullptr;

@@ -19,6 +19,11 @@
 #include <utility>
 #include <vector>
 
+#include <errno.h>
+#include <fcntl.h>
+#include <unistd.h>
+
+#include "encode.cuh"
 #include "generators.cuh"
 #include "kernels.cuh"
 #include "nccl_dyn.h"
@@ -36,6 +41,136 @@ std::string g_create_error;
 // SL_CHK: [sum psi^2, sum psi^2 potsub, sum psi^2 r2] left by the last sweep of a ground-state evolve (MODE_CHK)
 enum { SL_OBS = 0, SL_TMP = 5, SL_CHK = 8, SL_RAW = 16, SL_COEF = 16 + 256, SL_COUNT = 16 + 512 };
 constexpr int GRAM_LD = 256;  // at most 255 stored states (wavenum is a u8)
+
+// ---- array files (wafer_write_array): encode kernels over the work sites of this rank's slab -------------------
+// Sites are numbered in file order (x slowest, z fastest) from the slab's first work site; block b of the encoder
+// owns sites [b ENC_BS, (b + 1) ENC_BS).  encode_len_kernel leaves the bytes of each block's certified sites in
+// btot[b] and appends the sites fmt_g17 refuses to a list; the host formats those with snprintf, adds their lengths
+// and scans the block totals into byte offsets; encode_emit_kernel writes every site's bytes at its offset, taking a
+// refused site's text from the sorted table of host-formatted numbers.
+constexpr int ENC_THREADS = 256, ENC_BS = ENC_THREADS * 16;
+constexpr unsigned ENC_FLAG_CAP = 16u * ENC_BS;  // refused sites one launch collects; 16 blocks can never overflow it
+struct EncFlagIn { double v; unsigned long long site; };
+struct EncFlagStr { unsigned long long site; unsigned int len; char s[28]; };
+// The power table lives in a device buffer uploaded once (EncTable layout), not in a __device__ array: a module-scope
+// array would take a slot in front of the math library's tables and change the code of the kernels that read those.
+struct EncTable {
+    uint64_t hilo[2 * enc::NPOW];
+    int16_t shift[enc::NPOW];
+};
+
+// the power table in shared memory: lanes of a warp index different entries
+__device__ __forceinline__ enc::Pow10 enc_load_table(EncTable& s, const EncTable* __restrict__ g) {
+    for (int i = threadIdx.x; i < 2 * enc::NPOW; i += blockDim.x) s.hilo[i] = g->hilo[i];
+    for (int i = threadIdx.x; i < enc::NPOW; i += blockDim.x) s.shift[i] = g->shift[i];
+    __syncthreads();
+    return enc::Pow10{s.hilo, s.shift};
+}
+
+// slab site -> the value and its global (i, j, k)
+__device__ __forceinline__ double enc_site(const double* __restrict__ f, const Geom& g, unsigned long long s,
+                                           unsigned long long* gi, unsigned long long* j, unsigned long long* k) {
+    const unsigned long long plane = (unsigned long long)g.ny * (unsigned long long)g.nz;
+    const unsigned long long li = s / plane, r = s - li * plane;
+    *j = r / (unsigned long long)g.nz;
+    *k = r - *j * (unsigned long long)g.nz;
+    *gi = (unsigned long long)g.x0 + li;
+    return f[g.off((int)li, (int)*j, (int)*k)];
+}
+
+template <int FMT>
+__global__ void __launch_bounds__(ENC_THREADS)
+    encode_len_kernel(const double* __restrict__ f, Geom g, long long b0, unsigned long long nsites, const EncTable* pow10,
+                      unsigned int* __restrict__ btot, EncFlagIn* __restrict__ list, unsigned long long* __restrict__ count) {
+    __shared__ EncTable tab;
+    __shared__ unsigned int warp_sum[ENC_THREADS / 32];
+    const enc::Pow10 t = enc_load_table(tab, pow10);
+    const long long b = b0 + blockIdx.x;
+    const unsigned long long sb = (unsigned long long)b * ENC_BS, se = min(sb + ENC_BS, nsites);
+    unsigned int tot = 0;
+    for (unsigned long long s = sb + threadIdx.x; s < se; s += ENC_THREADS) {
+        unsigned long long gi, j, k;
+        const double v = enc_site(f, g, s, &gi, &j, &k);
+        char buf[enc::SITE_MAX];
+        const int n = enc::encode_site(FMT, v, gi, j, k, g.x0 == 0 && s == 0, nullptr, 0, buf, t);
+        if (n < 0) {
+            const unsigned long long at = atomicAdd(count, 1ull);
+            if (at < ENC_FLAG_CAP) list[at] = EncFlagIn{v, s};
+        } else {
+            tot += (unsigned int)n;
+        }
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) tot += __shfl_down_sync(0xffffffffu, tot, o);
+    if ((threadIdx.x & 31) == 0) warp_sum[threadIdx.x >> 5] = tot;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        unsigned int s = 0;
+        for (int w = 0; w < ENC_THREADS / 32; ++w) s += warp_sum[w];
+        btot[b] = s;
+    }
+}
+
+template <int FMT>
+__global__ void __launch_bounds__(ENC_THREADS)
+    encode_emit_kernel(const double* __restrict__ f, Geom g, long long b0, unsigned long long nsites, const EncTable* pow10,
+                       const unsigned long long* __restrict__ boff, unsigned long long base,
+                       const EncFlagStr* __restrict__ host_txt, int n_host, unsigned char* __restrict__ out,
+                       unsigned long long* __restrict__ missing) {
+    __shared__ EncTable tab;
+    __shared__ unsigned char stage[ENC_THREADS * enc::SITE_MAX];
+    __shared__ unsigned int warp_sum[ENC_THREADS / 32];
+    const enc::Pow10 t = enc_load_table(tab, pow10);
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const long long b = b0 + blockIdx.x;
+    const unsigned long long sb = (unsigned long long)b * ENC_BS, se = min(sb + ENC_BS, nsites);
+    unsigned long long o = boff[b] - base;
+    for (unsigned long long s0 = sb; s0 < se; s0 += ENC_THREADS) {
+        const unsigned long long s = s0 + threadIdx.x;
+        char buf[enc::SITE_MAX];
+        int n = 0;
+        if (s < se) {
+            unsigned long long gi, j, k;
+            const double v = enc_site(f, g, s, &gi, &j, &k);
+            const bool first = g.x0 == 0 && s == 0;
+            n = enc::encode_site(FMT, v, gi, j, k, first, nullptr, 0, buf, t);
+            if (n < 0) {  // refused by fmt_g17: the host's text, found by binary search in the sorted table
+                int lo = 0, hi = n_host;
+                while (lo < hi) {
+                    const int mid = (lo + hi) >> 1;
+                    if (host_txt[mid].site < s) lo = mid + 1;
+                    else hi = mid;
+                }
+                if (lo < n_host && host_txt[lo].site == s) {
+                    n = enc::encode_site(FMT, v, gi, j, k, first, host_txt[lo].s, (int)host_txt[lo].len, buf, t);
+                } else {
+                    n = 0;
+                    atomicAdd(missing, 1ull);
+                }
+            }
+        }
+        // exclusive block scan of the lengths
+        unsigned int incl = (unsigned int)n;
+#pragma unroll
+        for (int d = 1; d < 32; d <<= 1) {
+            const unsigned int y = __shfl_up_sync(0xffffffffu, incl, d);
+            if (lane >= d) incl += y;
+        }
+        if (lane == 31) warp_sum[warp] = incl;
+        __syncthreads();
+        unsigned int before = 0, total = 0;
+        for (int w = 0; w < ENC_THREADS / 32; ++w) {
+            if (w < warp) before += warp_sum[w];
+            total += warp_sum[w];
+        }
+        const unsigned int at = before + incl - (unsigned int)n;
+        for (int c = 0; c < n; ++c) stage[at + c] = (unsigned char)buf[c];
+        __syncthreads();
+        for (unsigned int c = threadIdx.x; c < total; c += ENC_THREADS) out[o + c] = stage[c];
+        o += total;
+        __syncthreads();
+    }
+}
 }  // namespace
 
 struct Tb2Sched {  // work lists of the persistent time-tiled sweep for one plane range (device arrays, sweep_tb.cuh Sched)
@@ -76,6 +211,18 @@ struct wafer_ctx {
     // pack / unpack kernel of the other one runs on s_main (lazily allocated, never a field-sized buffer)
     double* stg[2] = {nullptr, nullptr};
     long long stg_planes = 0;       // padded host planes one bounce buffer holds
+    size_t stg_bytes = 0;           // bytes of one bounce buffer (wafer_write_array may enlarge them on small lattices)
+    // wafer_write_array: pinned host halves of the bounce buffers, the encoder's block totals / offsets, the refused
+    // sites of one launch and the host text of those, the all-reduce vector (all allocated on first use)
+    unsigned char* wr_host[2] = {nullptr, nullptr};
+    unsigned int* wr_btot = nullptr;
+    unsigned long long* wr_boff = nullptr;
+    long long wr_blocks = 0;        // blocks wr_btot / wr_boff hold
+    EncTable* wr_pow10 = nullptr;
+    EncFlagIn* wr_flags = nullptr;
+    EncFlagStr* wr_txt = nullptr;
+    unsigned long long* wr_count = nullptr;  // [0] refused sites collected, [1] refused sites the emit pass did not find
+    unsigned long long* wr_red = nullptr;
     // source staging of the resampling entries when two source planes do not fit a bounce buffer (<= 128 MB each)
     double* rs_stg[2] = {nullptr, nullptr};
     long long rs_cap = 0;           // doubles one of them holds
@@ -757,8 +904,9 @@ int ensure_staging(wafer_ctx* ctx) {
     const long long plane_h = (long long)(g.ny + 2 * g.e) * (g.nz + 2 * g.e);
     const long long want = std::max<long long>(1, (128ll << 20) / (long long)(plane_h * sizeof(double)));
     ctx->stg_planes = std::min<long long>(want, g.L + 2 * g.gx + 2 * g.e);
+    ctx->stg_bytes = (size_t)(ctx->stg_planes * plane_h) * sizeof(double);
     for (int b = 0; b < 2; ++b) {
-        CK(cudaMalloc(&ctx->stg[b], (size_t)(ctx->stg_planes * plane_h) * sizeof(double)));
+        CK(cudaMalloc(&ctx->stg[b], ctx->stg_bytes));
         CK(cudaEventCreateWithFlags(&ctx->ev_stg_free[b], cudaEventDisableTiming));
         CK(cudaEventCreateWithFlags(&ctx->ev_stg_full[b], cudaEventDisableTiming));
     }
@@ -1083,6 +1231,10 @@ int wafer_destroy(wafer_ctx* ctx) {
         if (ctx->ev_stg_full[b]) cudaEventDestroy(ctx->ev_stg_full[b]);
     }
     if (ctx->s_copy) cudaStreamDestroy(ctx->s_copy);
+    for (int b = 0; b < 2; ++b)
+        if (ctx->wr_host[b]) cudaFreeHost(ctx->wr_host[b]);
+    cudaFree(ctx->wr_btot); cudaFree(ctx->wr_boff); cudaFree(ctx->wr_flags); cudaFree(ctx->wr_txt); cudaFree(ctx->wr_count);
+    cudaFree(ctx->wr_red); cudaFree(ctx->wr_pow10);
     cudaFree(ctx->d_cksum); cudaFree(ctx->gram);
     for (auto& kv : ctx->tb2_sched) {
         cudaFree(kv.second.bulk); cudaFree(kv.second.segs); cudaFree(kv.second.first); cudaFree(kv.second.counters);
@@ -1442,6 +1594,319 @@ static int ready(wafer_ctx* ctx, bool need_v) {
     if (!ctx->have_phi) { ctx->err = "phi not set (wafer_set_phi / wafer_generate_initial_condition)"; return WAFER_ERR_NOT_READY; }
     if (need_v && !ctx->have_v) { ctx->err = "potential not set (wafer_set_potential / wafer_generate_potential)"; return WAFER_ERR_NOT_READY; }
     return WAFER_OK;
+}
+
+// ---- array files encoded on the device (encode.cuh) -------------------------------------------------------------
+// Two passes over this rank's work sites.  Pass 1 measures: block totals of the certified sites, the refused sites
+// formatted on the host (their lengths added), an exclusive scan into block offsets.  The ranks then exchange their
+// byte counts in one all-reduce, so each knows where its planes start in the file.  Pass 2 encodes chunk after
+// chunk into a bounce buffer (as many whole blocks as fit), copies it to a pinned host buffer on s_copy and writes it
+// with pwrite while the next chunk is encoded.  Refused sites are collected again per piece of a chunk (a run of
+// blocks with at most ENC_FLAG_CAP of them) rather than kept from pass 1: host memory stays bounded whatever the field.
+static constexpr size_t WR_MIN_STG = 2 * (size_t)ENC_BS * enc::SITE_MAX;  // two blocks of the longest Csv rows
+
+static int wr_buffers(wafer_ctx* ctx, long long nblocks) {
+    TRY(ensure_staging(ctx));
+    if (ctx->stg_bytes < WR_MIN_STG) {  // a small lattice's bounce buffers; upload / download use stg_planes of them
+        for (int b = 0; b < 2; ++b) {
+            double* p = nullptr;
+            CK(cudaMalloc(&p, WR_MIN_STG));
+            cudaFree(ctx->stg[b]);
+            ctx->stg[b] = p;
+        }
+        ctx->stg_bytes = WR_MIN_STG;
+    }
+    for (int b = 0; b < 2; ++b)
+        if (!ctx->wr_host[b]) CK(cudaMallocHost(&ctx->wr_host[b], ctx->stg_bytes));
+    if (ctx->wr_blocks < nblocks) {
+        cudaFree(ctx->wr_btot);
+        cudaFree(ctx->wr_boff);
+        ctx->wr_btot = nullptr;
+        ctx->wr_boff = nullptr;
+        ctx->wr_blocks = 0;
+        CK(cudaMalloc(&ctx->wr_btot, (size_t)nblocks * sizeof(unsigned int)));
+        CK(cudaMalloc(&ctx->wr_boff, (size_t)(nblocks + 1) * sizeof(unsigned long long)));
+        ctx->wr_blocks = nblocks;
+    }
+    if (!ctx->wr_count) {
+        EncTable h;
+        const enc::Pow10 t = enc::host_pow10();
+        memcpy(h.hilo, t.hilo, sizeof h.hilo);
+        memcpy(h.shift, t.shift, sizeof h.shift);
+        CK(cudaMalloc(&ctx->wr_pow10, sizeof(EncTable)));
+        CK(cudaMemcpy(ctx->wr_pow10, &h, sizeof(EncTable), cudaMemcpyHostToDevice));
+        CK(cudaMalloc(&ctx->wr_flags, ENC_FLAG_CAP * sizeof(EncFlagIn)));
+        CK(cudaMalloc(&ctx->wr_txt, ENC_FLAG_CAP * sizeof(EncFlagStr)));
+        CK(cudaMalloc(&ctx->wr_count, 2 * sizeof(unsigned long long)));
+    }
+    if (ctx->world > 1 && !ctx->wr_red) CK(cudaMalloc(&ctx->wr_red, (size_t)(ctx->world + 1) * sizeof(unsigned long long)));
+    return WAFER_OK;
+}
+
+static void wr_host_site(const Geom& g, unsigned long long s, unsigned long long* gi, unsigned long long* j,
+                         unsigned long long* k) {
+    const unsigned long long plane = (unsigned long long)g.ny * (unsigned long long)g.nz, li = s / plane, r = s % plane;
+    *gi = (unsigned long long)g.x0 + li;
+    *j = r / (unsigned long long)g.nz;
+    *k = r % (unsigned long long)g.nz;
+}
+
+struct WrJob {
+    const double* f;
+    int fmt;
+    unsigned long long nsites;
+    long long nblocks;
+    std::vector<unsigned long long> btot;  // bytes of each block
+    std::vector<unsigned int> bflag;       // refused sites in each block
+    unsigned long long host_formatted = 0;
+};
+
+// refused sites of blocks [b0, b1) with their %.17g text, sorted by site; *n = how many the launch met (more than
+// ENC_FLAG_CAP: the list is incomplete and the caller splits the range).  bt: the blocks' certified bytes.
+static int wr_collect(wafer_ctx* ctx, const WrJob& job, long long b0, long long b1, std::vector<EncFlagStr>* txt,
+                      unsigned long long* n, std::vector<unsigned int>* bt) {
+    const Geom& g = ctx->g;
+    CK(cudaMemsetAsync(ctx->wr_count, 0, sizeof(unsigned long long), ctx->s_main));
+    const unsigned grid = (unsigned)(b1 - b0);
+    if (job.fmt == enc::FMT_CSV)
+        encode_len_kernel<enc::FMT_CSV><<<grid, ENC_THREADS, 0, ctx->s_main>>>(job.f, g, b0, job.nsites, ctx->wr_pow10, ctx->wr_btot, ctx->wr_flags, ctx->wr_count);
+    else
+        encode_len_kernel<enc::FMT_JSON><<<grid, ENC_THREADS, 0, ctx->s_main>>>(job.f, g, b0, job.nsites, ctx->wr_pow10, ctx->wr_btot, ctx->wr_flags, ctx->wr_count);
+    TRY(post_launch(ctx));
+    CK(cudaMemcpyAsync(n, ctx->wr_count, sizeof(unsigned long long), cudaMemcpyDeviceToHost, ctx->s_main));
+    if (bt) {
+        bt->resize(grid);
+        CK(cudaMemcpyAsync(bt->data(), ctx->wr_btot + b0, grid * sizeof(unsigned int), cudaMemcpyDeviceToHost, ctx->s_main));
+    }
+    CK(cudaStreamSynchronize(ctx->s_main));
+    txt->clear();
+    if (*n == 0 || *n > ENC_FLAG_CAP) return WAFER_OK;
+    std::vector<EncFlagIn> in(*n);
+    CK(cudaMemcpyAsync(in.data(), ctx->wr_flags, *n * sizeof(EncFlagIn), cudaMemcpyDeviceToHost, ctx->s_main));
+    CK(cudaStreamSynchronize(ctx->s_main));
+    std::sort(in.begin(), in.end(), [](const EncFlagIn& a, const EncFlagIn& b) { return a.site < b.site; });
+    txt->resize(*n);
+    for (size_t i = 0; i < in.size(); ++i) {
+        EncFlagStr& e = (*txt)[i];
+        e.site = in[i].site;
+        e.len = (unsigned int)snprintf(e.s, sizeof e.s, "%.17g", in[i].v);
+    }
+    return WAFER_OK;
+}
+
+// pass 1 over blocks [b0, b1): job.btot / job.bflag
+static int wr_measure(wafer_ctx* ctx, WrJob& job, long long b0, long long b1) {
+    std::vector<EncFlagStr> txt;
+    std::vector<unsigned int> bt;
+    unsigned long long n = 0;
+    TRY(wr_collect(ctx, job, b0, b1, &txt, &n, &bt));
+    if (n > ENC_FLAG_CAP) {  // pieces of ENC_FLAG_CAP sites cannot overflow the list
+        for (long long p = b0; p < b1; p += ENC_FLAG_CAP / ENC_BS)
+            TRY(wr_measure(ctx, job, p, std::min<long long>(b1, p + ENC_FLAG_CAP / ENC_BS)));
+        return WAFER_OK;
+    }
+    for (long long b = b0; b < b1; ++b) job.btot[b] = bt[b - b0];
+    const enc::Pow10 t = enc::host_pow10();
+    for (const EncFlagStr& e : txt) {
+        unsigned long long gi, j, k;
+        wr_host_site(ctx->g, e.site, &gi, &j, &k);
+        char buf[enc::SITE_MAX];
+        const int len = enc::encode_site(job.fmt, 0.0, gi, j, k, ctx->g.x0 == 0 && e.site == 0, e.s, (int)e.len, buf, t);
+        job.btot[e.site / ENC_BS] += (unsigned long long)len;
+        job.bflag[e.site / ENC_BS] += 1;
+        job.host_formatted += 1;
+    }
+    return WAFER_OK;
+}
+
+static int wr_allreduce(wafer_ctx* ctx, std::vector<unsigned long long>& v) {
+    if (ctx->world == 1) return WAFER_OK;
+    CK(cudaMemcpyAsync(ctx->wr_red, v.data(), v.size() * sizeof(unsigned long long), cudaMemcpyHostToDevice, ctx->s_main));
+    NK(nccl_api().AllReduce(ctx->wr_red, ctx->wr_red, v.size(), kNcclUint64, kNcclSum, ctx->comm, ctx->s_main));
+    CK(cudaMemcpyAsync(v.data(), ctx->wr_red, v.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost, ctx->s_main));
+    CK(cudaStreamSynchronize(ctx->s_main));
+    return WAFER_OK;
+}
+
+static bool wr_pwrite(int fd, const void* p, size_t n, unsigned long long off, std::string* err) {
+    const char* c = (const char*)p;
+    while (n > 0) {
+        const ssize_t w = pwrite(fd, c, n, (off_t)off);
+        if (w < 0 && errno == EINTR) continue;
+        if (w <= 0) {
+            *err = std::string("write failed: ") + (w < 0 ? strerror(errno) : "no progress");
+            return false;
+        }
+        c += w;
+        n -= (size_t)w;
+        off += (unsigned long long)w;
+    }
+    return true;
+}
+
+// pass 2: encode, copy and write every chunk; `ok` / `io_err` report the first failed write (the GPU work is still
+// drained so that the buffers are free on return)
+static int wr_emit(wafer_ctx* ctx, const WrJob& job, const std::vector<unsigned long long>& boff, int fd,
+                   unsigned long long data_off, bool* ok, std::string* io_err) {
+    const Geom& g = ctx->g;
+    CK(cudaMemsetAsync(ctx->wr_count + 1, 0, sizeof(unsigned long long), ctx->s_main));
+    CK(cudaEventRecord(ctx->ev_stg_free[0], ctx->s_main));
+    CK(cudaEventRecord(ctx->ev_stg_free[1], ctx->s_main));
+    unsigned long long pend_bytes = 0, pend_off = 0;
+    int k = 0;
+    for (long long cb = 0; cb < job.nblocks; ++k) {
+        long long ce = cb + 1;
+        while (ce < job.nblocks && boff[ce + 1] - boff[cb] <= ctx->stg_bytes) ++ce;
+        const int buf = k & 1;
+        unsigned char* out = (unsigned char*)ctx->stg[buf];
+        CK(cudaStreamWaitEvent(ctx->s_main, ctx->ev_stg_free[buf], 0));  // the copy of chunk k - 2 has left it
+        for (long long pb = cb; pb < ce;) {
+            long long pe = pb;
+            unsigned long long nf = 0;
+            while (pe < ce && nf + job.bflag[pe] <= ENC_FLAG_CAP) nf += job.bflag[pe++];
+            int ntxt = 0;
+            if (nf > 0) {
+                std::vector<EncFlagStr> txt;
+                unsigned long long n = 0;
+                TRY(wr_collect(ctx, job, pb, pe, &txt, &n, nullptr));
+                if (n != nf) { ctx->err = "wafer_write_array: the refused sites differ between the passes"; return WAFER_ERR_CUDA; }
+                CK(cudaMemcpyAsync(ctx->wr_txt, txt.data(), txt.size() * sizeof(EncFlagStr), cudaMemcpyHostToDevice, ctx->s_main));
+                CK(cudaStreamSynchronize(ctx->s_main));
+                ntxt = (int)n;
+            }
+            const unsigned grid = (unsigned)(pe - pb);
+            switch (job.fmt) {
+                case enc::FMT_MPK: encode_emit_kernel<enc::FMT_MPK><<<grid, ENC_THREADS, 0, ctx->s_main>>>(job.f, g, pb, job.nsites, ctx->wr_pow10, ctx->wr_boff, boff[cb], ctx->wr_txt, ntxt, out, ctx->wr_count + 1); break;
+                case enc::FMT_CSV: encode_emit_kernel<enc::FMT_CSV><<<grid, ENC_THREADS, 0, ctx->s_main>>>(job.f, g, pb, job.nsites, ctx->wr_pow10, ctx->wr_boff, boff[cb], ctx->wr_txt, ntxt, out, ctx->wr_count + 1); break;
+                default: encode_emit_kernel<enc::FMT_JSON><<<grid, ENC_THREADS, 0, ctx->s_main>>>(job.f, g, pb, job.nsites, ctx->wr_pow10, ctx->wr_boff, boff[cb], ctx->wr_txt, ntxt, out, ctx->wr_count + 1); break;
+            }
+            TRY(post_launch(ctx));
+            pb = pe;
+        }
+        const unsigned long long bytes = boff[ce] - boff[cb];
+        CK(cudaEventRecord(ctx->ev_stg_full[buf], ctx->s_main));
+        CK(cudaStreamWaitEvent(ctx->s_copy, ctx->ev_stg_full[buf], 0));
+        CK(cudaMemcpyAsync(ctx->wr_host[buf], out, bytes, cudaMemcpyDeviceToHost, ctx->s_copy));
+        CK(cudaEventRecord(ctx->ev_stg_free[buf], ctx->s_copy));
+        if (k > 0) {  // chunk k - 1 is written while chunk k is encoded and copied
+            CK(cudaEventSynchronize(ctx->ev_stg_free[buf ^ 1]));
+            if (*ok) *ok = wr_pwrite(fd, ctx->wr_host[buf ^ 1], pend_bytes, data_off + pend_off, io_err);
+        }
+        pend_bytes = bytes;
+        pend_off = boff[cb];
+        cb = ce;
+    }
+    CK(cudaEventSynchronize(ctx->ev_stg_free[(k - 1) & 1]));
+    if (*ok) *ok = wr_pwrite(fd, ctx->wr_host[(k - 1) & 1], pend_bytes, data_off + pend_off, io_err);
+    unsigned long long missing = 0;
+    CK(cudaMemcpyAsync(&missing, ctx->wr_count + 1, sizeof(missing), cudaMemcpyDeviceToHost, ctx->s_main));
+    CK(cudaStreamSynchronize(ctx->s_main));
+    if (missing) { ctx->err = "wafer_write_array: a refused site had no host text"; return WAFER_ERR_CUDA; }
+    return WAFER_OK;
+}
+
+namespace {
+struct FdGuard {
+    int fd = -1;
+    ~FdGuard() {
+        if (fd >= 0) close(fd);
+    }
+};
+}  // namespace
+
+static int write_array_impl(wafer_ctx* ctx, int32_t what, int32_t file_type, const char* path, wafer_write_stats* stats) {
+    if (!ctx) return WAFER_ERR_INVALID;
+    REQUIRE(what == 0 || what == 1, "what must be 0 (psi) or 1 (V)");
+    REQUIRE(file_type >= 0 && file_type <= 2,
+            "file_type must be 0 (Messagepack), 1 (Csv) or 2 (Json); Yaml and Ron files are not supported");
+    REQUIRE(path, "path is NULL");
+    const Geom& g = ctx->g;
+    char pre[96];
+    int npre = 0;
+    if (file_type == enc::FMT_MPK) {
+        npre = enc::mpk_preamble((uint64_t)g.gnx, (uint64_t)g.gny, (uint64_t)g.gnz, (unsigned char*)pre);
+        REQUIRE(npre >= 0, "Messagepack: an array of more than 2^32-1 elements cannot be written (array32 limit)");
+    } else if (file_type == enc::FMT_JSON) {
+        npre = enc::json_preamble((uint64_t)g.gnx, (uint64_t)g.gny, (uint64_t)g.gnz, pre);
+    }
+    if (what == 0) TRY(ready(ctx, false));
+    else if (!ctx->have_v) { ctx->err = "potential not set (wafer_set_potential / wafer_generate_potential)"; return WAFER_ERR_NOT_READY; }
+    CK(cudaSetDevice(ctx->dev));
+    const int rank = ctx->rank, world = ctx->world;
+
+    WrJob job;
+    job.f = what == 0 ? ctx->psi[ctx->cur] : ctx->v;
+    job.fmt = file_type;
+    job.nsites = (unsigned long long)g.L * (unsigned long long)g.ny * (unsigned long long)g.nz;
+    job.nblocks = (long long)((job.nsites + ENC_BS - 1) / ENC_BS);
+    job.btot.assign(job.nblocks, 0);
+    job.bflag.assign(job.nblocks, 0);
+    TRY(wr_buffers(ctx, job.nblocks));
+    if (file_type == enc::FMT_MPK) {
+        for (long long b = 0; b < job.nblocks; ++b)
+            job.btot[b] = 9ull * (std::min<unsigned long long>(job.nsites, (unsigned long long)(b + 1) * ENC_BS) - (unsigned long long)b * ENC_BS);
+    } else {
+        for (long long b = 0; b < job.nblocks; b += 4096) TRY(wr_measure(ctx, job, b, std::min<long long>(job.nblocks, b + 4096)));
+    }
+    std::vector<unsigned long long> boff(job.nblocks + 1, 0);
+    for (long long b = 0; b < job.nblocks; ++b) boff[b + 1] = boff[b] + job.btot[b];
+    CK(cudaMemcpyAsync(ctx->wr_boff, boff.data(), boff.size() * sizeof(unsigned long long), cudaMemcpyHostToDevice, ctx->s_main));
+
+    // every rank opens the one file; no rank writes unless all could
+    FdGuard fd;
+    fd.fd = open(path, O_WRONLY | O_CREAT | O_CLOEXEC, 0666);
+    std::string io_err = fd.fd < 0 ? std::string("cannot create ") + path + ": " + strerror(errno) : std::string();
+    std::vector<unsigned long long> red(world + 1, 0);
+    red[rank] = boff[job.nblocks];
+    red[world] = fd.fd < 0 ? 1 : 0;
+    TRY(wr_allreduce(ctx, red));
+    if (red[world]) {
+        ctx->err = io_err.empty() ? std::string("another rank cannot create ") + path : io_err;
+        return WAFER_ERR_IO;
+    }
+    unsigned long long before = 0, all = 0;
+    for (int q = 0; q < world; ++q) {
+        if (q < rank) before += red[q];
+        all += red[q];
+    }
+    const unsigned long long trailer = file_type == enc::FMT_JSON ? 2 : 0;
+    const unsigned long long file_bytes = (unsigned long long)npre + all + trailer;
+    bool ok = true;
+    if (rank == 0) {  // a longer file of the same name loses its tail; the ranks write every byte below file_bytes
+        if (ftruncate(fd.fd, (off_t)file_bytes) != 0) {
+            io_err = std::string("cannot truncate ") + path + ": " + strerror(errno);
+            ok = false;
+        }
+        if (ok && npre) ok = wr_pwrite(fd.fd, pre, (size_t)npre, 0, &io_err);
+    }
+    if (ok && rank == world - 1 && trailer) ok = wr_pwrite(fd.fd, "]}", 2, (unsigned long long)npre + all, &io_err);
+    if (ok) TRY(wr_emit(ctx, job, boff, fd.fd, (unsigned long long)npre + before, &ok, &io_err));
+    if (close(fd.fd) != 0 && ok) {
+        io_err = std::string("close failed: ") + strerror(errno);
+        ok = false;
+    }
+    fd.fd = -1;
+    std::vector<unsigned long long> agree(1, ok ? 0 : 1);  // every rank returns the same status
+    TRY(wr_allreduce(ctx, agree));
+    if (agree[0]) {
+        ctx->err = io_err.empty() ? std::string("another rank could not write ") + path : path + std::string(": ") + io_err;
+        return WAFER_ERR_IO;
+    }
+    if (stats) {
+        stats->bytes = boff[job.nblocks] + (rank == 0 ? (unsigned long long)npre : 0) + (rank == world - 1 ? trailer : 0);
+        stats->file_bytes = file_bytes;
+        stats->host_formatted = job.host_formatted;
+    }
+    return WAFER_OK;
+}
+
+int wafer_write_array(wafer_ctx* ctx, int32_t what, int32_t file_type, const char* path, wafer_write_stats* stats) {
+    try {
+        return write_array_impl(ctx, what, file_type, path, stats);
+    } catch (const std::exception& e) {  // host-side allocation failures must not unwind through the C ABI
+        if (ctx) ctx->err = std::string("wafer_write_array: ") + e.what();
+        return WAFER_ERR_INVALID;
+    }
 }
 
 int wafer_observables_compute(wafer_ctx* ctx, wafer_observables* out) {
