@@ -41,7 +41,8 @@ typedef enum {
     WAFER_ERR_NOT_READY = 6,    /* potential or phi not set yet                                                */
     WAFER_ERR_MAX_STEP = 7,     /* wafer_solve: not converged within max_steps (errors.rs MaxStep, grid.rs:244) */
     WAFER_ERR_NONFINITE = 8,    /* NaN/Inf met where the reference's R64 would panic (noisy_float)             */
-    WAFER_ERR_IO = 9            /* a file could not be created or written; see wafer_last_error               */
+    WAFER_ERR_IO = 9,           /* a file could not be created, written, opened or read; see wafer_last_error */
+    WAFER_ERR_FORMAT = 10       /* the file is not in a layout the device decoder reads; nothing changed       */
 } wafer_status;
 
 /* flags */
@@ -162,6 +163,26 @@ typedef struct {
    WAFER_ERR_INVALID, nothing created: unknown what or file_type (Yaml / Ron), NULL path, Messagepack of more than
    2^32-1 sites (its array32 header cannot count them).  WAFER_ERR_NOT_READY without psi / V.  stats may be NULL. */
 int wafer_write_array(wafer_ctx *ctx, int32_t what, int32_t file_type, const char *path, wafer_write_stats *stats);
+
+typedef struct {
+    uint64_t sx, sy, sz;       /* dims of the file's array                                                           */
+    uint64_t bytes_read;       /* bytes this rank read: the whole file                                               */
+    uint64_t sites_converted;  /* sites of the source x-planes this rank's planes need, all converted                  */
+    uint64_t host_converted;   /* of those, numbers strtod converted on the host (the device could not certify them) */
+} wafer_load_stats;
+/* input::load_wavefunctions / fill_data / read_csv (input.rs:113-176, 487-505, 607-662) for a file `path` of file_type
+   0 Messagepack, 1 Csv, 2 Json, decoded on the device: what = 0 sets psi (= wafer_set_phi_resampled of the array that
+   formats.hpp's read_mpk / read_csv / read_json return), 1 sets V (= wafer_set_potential_resampled), 2 pushes a lower
+   state (= wafer_push_lower_resampled), bit for bit.  Only the canonical layouts are read: what formats.hpp's writers
+   (and rmp-serde / serde_json) produce, numbers in the JSON grammar (DESIGN.md section 1.4).  The file is streamed through
+   the bounce buffers with pread and checked whole before anything changes; numbers the device cannot certify are
+   converted with strtod on the host.  Every rank reads the whole file and keeps the source x-planes its planes need,
+   in one device buffer; no communication when world > 1.
+   WAFER_ERR_IO: the file cannot be opened or read.  WAFER_ERR_FORMAT, nothing changed: the file is not canonical, or
+   the rank's source planes cannot be allocated on the device (formats.hpp's readers and wafer_*_resampled still
+   take such a file).  WAFER_ERR_INVALID: unknown what or file_type (Yaml / Ron), NULL path, a shape the resampling
+   entries refuse.  stats may be NULL. */
+int wafer_load_array(wafer_ctx *ctx, int32_t what, int32_t file_type, const char *path, wafer_load_stats *stats);
 
 /* -------- the hot path -------------------------------------------------------------------------- */
 int wafer_observables_compute(wafer_ctx *ctx, wafer_observables *out); /* compute_observables        (grid.rs:303-445) */

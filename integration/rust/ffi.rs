@@ -44,6 +44,20 @@ pub struct WaferWriteStats {
     pub host_formatted: u64,
 }
 
+#[repr(C)]
+#[derive(Default, Debug, Clone, Copy)]
+pub struct WaferLoadStats {
+    pub sx: u64,
+    pub sy: u64,
+    pub sz: u64,
+    pub bytes_read: u64,
+    pub sites_converted: u64,
+    pub host_converted: u64,
+}
+
+/// `WAFER_ERR_FORMAT`: the file is not in a layout the device decoder reads; nothing changed.
+pub const WAFER_ERR_FORMAT: c_int = 10;
+
 pub enum WaferCtx {}
 
 extern "C" {
@@ -68,6 +82,7 @@ extern "C" {
     fn wafer_normalise(ctx: *mut WaferCtx, norm2: f64) -> c_int;
     fn wafer_evolve(ctx: *mut WaferCtx, wnum: u8, steps: u64) -> c_int;
     fn wafer_write_array(ctx: *mut WaferCtx, what: i32, file_type: i32, path: *const c_char, stats: *mut WaferWriteStats) -> c_int;
+    fn wafer_load_array(ctx: *mut WaferCtx, what: i32, file_type: i32, path: *const c_char, stats: *mut WaferLoadStats) -> c_int;
     fn wafer_synchronize(ctx: *mut WaferCtx) -> c_int;
     fn wafer_host_register(ptr: *mut c_void, bytes: usize) -> c_int;
     fn wafer_host_unregister(ptr: *mut c_void) -> c_int;
@@ -182,6 +197,17 @@ impl Gpu {
         let c = CString::new(path).map_err(|_| Error::from("output path contains a NUL byte"))?;
         let mut st = WaferWriteStats::default();
         self.check(unsafe { wafer_write_array(self.ctx, what, file_type, c.as_ptr(), &mut st) })?;
+        Ok(st)
+    }
+    /// input::load_wavefunctions / fill_data / read_csv (input.rs:113-176, 487-505, 607-662) decoded on the device: the
+    /// file `path` of `file_type` 0 Messagepack, 1 Csv, 2 Json into psi (`what` 0), V (1) or a new lower state (2), as
+    /// the `*_resampled` entries would set it from the parsed array.  Only the host writers' layouts are read: any other
+    /// file returns `Err` with status 10 (`WAFER_ERR_FORMAT`) in the message and leaves everything as it was, so the caller parses it
+    /// with `input.rs` and calls the `*_resampled` entry instead.  No communication when world > 1.
+    pub fn load_array(&self, what: i32, file_type: i32, path: &str) -> Result<WaferLoadStats> {
+        let c = CString::new(path).map_err(|_| Error::from("input path contains a NUL byte"))?;
+        let mut st = WaferLoadStats::default();
+        self.check(unsafe { wafer_load_array(self.ctx, what, file_type, c.as_ptr(), &mut st) })?;
         Ok(st)
     }
     /// Page-lock the buffer behind `arr` so that set_phi / get_phi run at PCIe speed (54 GB/s measured instead of the

@@ -11,7 +11,7 @@ import os
 import numpy as np
 
 from . import _capi
-from ._capi import Observables, Params, Record, WriteStats
+from ._capi import LoadStats, Observables, Params, Record, WriteStats
 
 __all__ = ["Lattice", "slab_partition", "tb2_plan", "WaferError", "POTENTIALS", "INITIAL_CONDITIONS", "SYMMETRIES", "EXT",
            "nccl_unique_id", "pinned_empty", "pin", "unpin", "FLAG_AB_ARRAYS", "FILE_TYPES"]
@@ -32,7 +32,7 @@ FLAG_SIMPLE_SWEEP = 0x4
 FLAG_TMA_ONE_STEP = 0x8
 
 _STATUS = {1: "INVALID", 2: "NO_DEVICE", 3: "CUDA", 4: "NCCL", 5: "RING_NONZERO", 6: "NOT_READY", 7: "MAX_STEP",
-           8: "NONFINITE", 9: "IO"}
+           8: "NONFINITE", 9: "IO", 10: "FORMAT"}
 _dp = C.POINTER(C.c_double)
 
 
@@ -345,6 +345,19 @@ class Lattice:
         st = WriteStats()
         self._ck(self._lib.wafer_write_array(self._h, w, ft, os.fsencode(path), C.byref(st)))
         return dict(bytes=st.bytes, file_bytes=st.file_bytes, host_formatted=st.host_formatted)
+
+    def load_array(self, what, path, file_type):
+        """Decode the array file `path` on the device into psi (what="phi" or 0), V ("potential" or 1) or a new lower
+        state ("lower" or 2), as set_phi_resampled / set_potential_resampled / push_lower_resampled of the array the
+        front end's formats.hpp reader returns (from_csv for "Csv"), bit for bit.  file_type: "Messagepack" / "Csv" /
+        "Json" (or 0 / 1 / 2).  Raises WaferError with status 10 (FORMAT), nothing changed, for a file not in the
+        canonical layout of the host writers.  Returns dict(sx, sy, sz, bytes_read, sites_converted, host_converted)."""
+        w = {"phi": 0, "potential": 1, "lower": 2}[what] if isinstance(what, str) else int(what)
+        ft = FILE_TYPES[file_type] if isinstance(file_type, str) else int(file_type)
+        st = LoadStats()
+        self._ck(self._lib.wafer_load_array(self._h, w, ft, os.fsencode(path), C.byref(st)))
+        return dict(sx=st.sx, sy=st.sy, sz=st.sz, bytes_read=st.bytes_read, sites_converted=st.sites_converted,
+                    host_converted=st.host_converted)
 
     # ---- the hot path, reference names (grid.rs)
     def compute_observables(self):

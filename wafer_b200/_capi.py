@@ -28,6 +28,11 @@ class WriteStats(C.Structure):
     _fields_ = [("bytes", C.c_uint64), ("file_bytes", C.c_uint64), ("host_formatted", C.c_uint64)]
 
 
+class LoadStats(C.Structure):
+    _fields_ = [("sx", C.c_uint64), ("sy", C.c_uint64), ("sz", C.c_uint64), ("bytes_read", C.c_uint64),
+                ("sites_converted", C.c_uint64), ("host_converted", C.c_uint64)]
+
+
 # every symbol include/wafer_b200.h declares: name -> (restype, argtypes)
 _ctx = C.c_void_p
 SYMBOLS = {
@@ -65,6 +70,7 @@ SYMBOLS = {
     "wafer_set_potential_resampled": (C.c_int, [_ctx, _dp, C.c_uint64, C.c_uint64, C.c_uint64, C.c_uint32]),
     "wafer_push_lower_resampled": (C.c_int, [_ctx, _dp, C.c_uint64, C.c_uint64, C.c_uint64, C.c_uint32]),
     "wafer_write_array": (C.c_int, [_ctx, C.c_int32, C.c_int32, C.c_char_p, C.POINTER(WriteStats)]),
+    "wafer_load_array": (C.c_int, [_ctx, C.c_int32, C.c_int32, C.c_char_p, C.POINTER(LoadStats)]),
     "wafer_observables_compute": (C.c_int, [_ctx, C.POINTER(Observables)]),
     "wafer_norm2": (C.c_int, [_ctx, _dp]),
     "wafer_normalise": (C.c_int, [_ctx, C.c_double]),

@@ -240,18 +240,26 @@ inline void write_array(const std::string& stem, int file_type, const Array3& a)
     }
 }
 // input.rs:32-111 / 513-578: prefer the configured file type, then whichever of mpk / csv / json exists
-inline bool read_array(const std::string& stem, int preferred, Array3& out, int* used_type = nullptr) {
+inline bool find_array(const std::string& stem, int preferred, int* type) {
     auto exists = [](const std::string& p) { std::ifstream f(p); return (bool)f; };
     const int order[4] = {preferred, 0, 1, 2};
     for (int t : order) {
-        if (t > 2) continue;
-        const std::string path = stem + extension(t);
-        if (!exists(path)) continue;
-        out = t == 0 ? read_mpk(path) : (t == 1 ? read_csv(path) : read_json(path));
-        if (used_type) *used_type = t;
+        if (t > 2 || !exists(stem + extension(t))) continue;
+        *type = t;
         return true;
     }
     return false;
+}
+inline Array3 read_typed(const std::string& stem, int t) {
+    const std::string path = stem + extension(t);
+    return t == 0 ? read_mpk(path) : (t == 1 ? read_csv(path) : read_json(path));
+}
+inline bool read_array(const std::string& stem, int preferred, Array3& out, int* used_type = nullptr) {
+    int t = 0;
+    if (!find_array(stem, preferred, &t)) return false;
+    out = read_typed(stem, t);
+    if (used_type) *used_type = t;
+    return true;
 }
 
 // fill_data (input.rs:149-176) / read_csv (input.rs:641-657): embed the array of a file into the padded one.

@@ -2,7 +2,7 @@
 //
 // Same wafer.yaml, same CLI flags (-c/--config, -s/--script, -d), same per-state loop, same table rows
 // (output.rs:497-521) and observables record (output.rs:32-45, 533-547).  Everything numerical happens in
-// libwafer_b200.so on the GPU, the array files included (wafer_write_array); this file is host glue: configuration,
+// libwafer_b200.so on the GPU, the array files included (wafer_load_array, wafer_write_array); this file is host glue: configuration,
 // potential / initial-condition selection, the observables files, printing.
 //
 //   wafer-b200 -c wafer.yaml                 run (one process per GPU; RANK / WORLD_SIZE / LOCAL_RANK select a slab)
@@ -49,16 +49,25 @@ std::string ordinal(unsigned n) {
     return std::to_string(n) + suf;
 }
 
-// array files in: the file's array as parsed (input.rs:32-127, 513-662), which the wafer_*_resampled entries embed on
-// the device as fill_data / read_csv do (input.rs:149-176, 641-657; formats.hpp embed_work is the host restatement).
-// from_csv: the file read was a Csv file.  Out: wafer_write_array (write_array_file below).
-bool read_input(const std::string& stem, int file_type, const Dims& d, Array3& a, uint32_t& from_csv) {
+// array files in (input.rs:32-127, 513-662), embedded as fill_data / read_csv do (input.rs:149-176, 641-657; formats.hpp
+// embed_work is the host restatement): what 0 psi, 1 V, 2 push a lower state.  The file found is decoded on the device
+// (wafer_load_array); a file it does not take (not in the host writers' layout, or too large for the device) goes
+// through formats.hpp's reader and the wafer_*_resampled entry, with that path's messages and refusals.  Out:
+// wafer_write_array (write_array_file below).
+bool load_input(wafer_ctx* ctx, int what, const std::string& stem, int file_type, const Dims& d) {
     int used = 0;
-    if (!read_array(stem, file_type, a, &used)) return false;
+    if (!find_array(stem, file_type, &used)) return false;
+    if (wafer_load_array(ctx, what, used, (stem + extension(used)).c_str(), nullptr) == WAFER_OK) return true;
+    const Array3 a = read_typed(stem, used);
     if (a.nx < 2 || a.ny < 2 || a.nz < 2) throw std::runtime_error("ArrayShape: " + stem + " cannot be resized");
-    from_csv = used == 1 ? 1 : 0;
+    const uint32_t from_csv = used == 1 ? 1 : 0;
     if (!from_csv && a.nx == d.px && a.ny == d.py && a.nz == d.pz)
         throw std::runtime_error("input array already has the padded size: the reference's fill_data cannot load it (input.rs:167-169)");
+    static const char* entry[3] = {"wafer_set_phi_resampled", "wafer_set_potential_resampled", "wafer_push_lower_resampled"};
+    const int rc = what == 0 ? wafer_set_phi_resampled(ctx, a.data.data(), a.nx, a.ny, a.nz, from_csv)
+                   : what == 1 ? wafer_set_potential_resampled(ctx, a.data.data(), a.nx, a.ny, a.nz, from_csv)
+                               : wafer_push_lower_resampled(ctx, a.data.data(), a.nx, a.ny, a.nz, from_csv);
+    if (rc != WAFER_OK) throw std::runtime_error(std::string(entry[what]) + ": " + wafer_last_error(ctx));
     return true;
 }
 
@@ -185,11 +194,7 @@ bool solve(Run& r, unsigned wnum) {
     const Dims d(c);
     if (wnum > 0) {
         // grid.rs:60-96: a wavefunction_{wnum} file in ./input wins, else start from the previous converged state
-        Array3 a;
-        uint32_t csv = 0;
-        if (read_input("input/wavefunction_" + std::to_string(wnum), c.file_type, d, a, csv)) {
-            r.ck(wafer_set_phi_resampled(r.ctx, a.data.data(), a.nx, a.ny, a.nz, csv), "wafer_set_phi_resampled");
-        } else {
+        if (!load_input(r.ctx, 0, "input/wavefunction_" + std::to_string(wnum), c.file_type, d)) {
             // grid.rs:95 clones w_store[wnum-1] and lets rounding noise seed the new state (SURVEY F7); here the
             // clone is multiplied by a fixed symmetry-free polynomial so the start is well defined and reproducible
             r.ck(wafer_phi_seed_from_lower(r.ctx, wnum - 1), "wafer_phi_seed_from_lower");
@@ -387,10 +392,7 @@ int main(int argc, char** argv) {
 
         // potential::load_arrays (potential.rs:75-175)
         if (c.potential == 12) {  // FromFile
-            Array3 a;
-            uint32_t csv = 0;
-            if (!read_input("input/potential", c.file_type, d, a, csv)) throw std::runtime_error("LoadPotential: input/potential.{mpk,csv,json} not found");
-            r.ck(wafer_set_potential_resampled(r.ctx, a.data.data(), a.nx, a.ny, a.nz, csv), "wafer_set_potential_resampled");
+            if (!load_input(r.ctx, 1, "input/potential", c.file_type, d)) throw std::runtime_error("LoadPotential: input/potential.{mpk,csv,json} not found");
         } else if (c.potential == 13) {  // FromScript
             std::vector<double> v(d.padded());
             script_potential(c, v, d);
@@ -409,19 +411,13 @@ int main(int argc, char** argv) {
 
         // run (grid.rs:31-47): lower states from ./input when starting above the ground state
         for (unsigned w = 0; w < c.wavenum; ++w) {  // input::load_wavefunctions (input.rs:487-505)
-            Array3 a;
-            uint32_t csv = 0;
-            if (!read_input("input/wavefunction_" + std::to_string(w), c.file_type, d, a, csv))
+            if (!load_input(r.ctx, 2, "input/wavefunction_" + std::to_string(w), c.file_type, d))
                 throw std::runtime_error("LoadWavefunction: input/wavefunction_" + std::to_string(w) + ".{mpk,csv,json} is required when wavenum > 0");
-            r.ck(wafer_push_lower_resampled(r.ctx, a.data.data(), a.nx, a.ny, a.nz, csv), "wafer_push_lower_resampled");
         }
         // config::set_initial_conditions (config.rs:577-627)
         if (c.wavenum == 0) {
             if (c.init_condition == 0) {
-                Array3 a;
-                uint32_t csv = 0;
-                if (!read_input("input/wavefunction_0", c.file_type, d, a, csv)) throw std::runtime_error("LoadWavefunction: input/wavefunction_0.{mpk,csv,json} not found");
-                r.ck(wafer_set_phi_resampled(r.ctx, a.data.data(), a.nx, a.ny, a.nz, csv), "wafer_set_phi_resampled");
+                if (!load_input(r.ctx, 0, "input/wavefunction_0", c.file_type, d)) throw std::runtime_error("LoadWavefunction: input/wavefunction_0.{mpk,csv,json} not found");
             } else if (c.init_condition == 1) {  // Gaussian (config.rs:636-642): thread_rng there; seeded on the device here
                 r.ck(wafer_generate_gaussian(r.ctx, c.sig, c.seed), "wafer_generate_gaussian");
             } else {

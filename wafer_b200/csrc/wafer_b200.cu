@@ -21,8 +21,10 @@
 
 #include <errno.h>
 #include <fcntl.h>
+#include <sys/stat.h>
 #include <unistd.h>
 
+#include "decode.cuh"
 #include "encode.cuh"
 #include "generators.cuh"
 #include "kernels.cuh"
@@ -171,6 +173,175 @@ __global__ void __launch_bounds__(ENC_THREADS)
         __syncthreads();
     }
 }
+
+// ---- array files read (wafer_load_array): decode kernels over one chunk of a file's records ---------------------
+// A Csv / Json chunk holds whole records (the host carries a split one into the next chunk); a record starts at byte
+// 0 and after every separator.  Block b owns the records that start in bytes [b DEC_SEG, (b + 1) DEC_SEG):
+// dec_count_kernel counts them, dec_offsets_kernel scans the counts into global record indices, dec_text_kernel lists
+// the block's record starts through a block scan, checks each record's grammar (and a Csv record's indices) and
+// converts the numbers of the source planes [p0, p1) into dst.  Numbers parse_f64 cannot certify are listed (record,
+// offset, length) for strtod on the host.  A Messagepack chunk holds whole 9-byte elements: dec_mpk_kernel.
+constexpr int DEC_THREADS = 256, DEC_BYTES = 32, DEC_SEG = DEC_THREADS * DEC_BYTES;
+constexpr unsigned DEC_FLAG_CAP = 16u * DEC_SEG;  // numbers one launch lists; 16 blocks can never overflow it
+struct DecFlag { unsigned long long rec; unsigned int at, len; double v; };
+struct DecDst {  // the converted source planes [p0, p1) of an array of n sites, `plane` = sy sz sites per x-plane
+    double* dst;
+    unsigned long long n, plane, sz, p0, p1;
+};
+enum { DEC_ERR = 0, DEC_NFLAG = 1, DEC_WORDS = 2 };  // state words of one chunk
+
+__device__ __forceinline__ bool dec_is_start(const unsigned char* __restrict__ c, unsigned long long p, unsigned char sep) {
+    return p == 0 || c[p - 1] == sep;
+}
+
+// record starts in this thread's DEC_BYTES bytes of block b's segment, as a bit mask
+__device__ __forceinline__ unsigned int dec_starts(const unsigned char* __restrict__ c, unsigned long long len, long long b,
+                                                   unsigned char sep, unsigned long long* at) {
+    *at = (unsigned long long)b * DEC_SEG + (unsigned long long)threadIdx.x * DEC_BYTES;
+    unsigned int m = 0;
+    for (int i = 0; i < DEC_BYTES; ++i) {
+        const unsigned long long p = *at + i;
+        if (p < len && dec_is_start(c, p, sep)) m |= 1u << i;
+    }
+    return m;
+}
+
+__global__ void __launch_bounds__(DEC_THREADS)
+    dec_count_kernel(const unsigned char* __restrict__ c, unsigned long long len, unsigned char sep,
+                     unsigned int* __restrict__ bcount) {
+    __shared__ unsigned int warp_sum[DEC_THREADS / 32];
+    unsigned long long at;
+    unsigned int n = __popc(dec_starts(c, len, blockIdx.x, sep, &at));
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) n += __shfl_down_sync(0xffffffffu, n, o);
+    if ((threadIdx.x & 31) == 0) warp_sum[threadIdx.x >> 5] = n;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        unsigned int s = 0;
+        for (int w = 0; w < DEC_THREADS / 32; ++w) s += warp_sum[w];
+        bcount[blockIdx.x] = s;
+    }
+}
+
+// one block: boff[b] = records before block b of this chunk, counting from *base; *base += the chunk's records
+__global__ void __launch_bounds__(1024)
+    dec_offsets_kernel(const unsigned int* __restrict__ bcount, int nb, unsigned long long* __restrict__ boff,
+                       unsigned long long* __restrict__ base) {
+    __shared__ unsigned long long part[1024];
+    const int per = (nb + 1023) / 1024, b0 = threadIdx.x * per, b1 = min(nb, b0 + per);
+    unsigned long long s = 0;
+    for (int b = b0; b < b1; ++b) s += bcount[b];
+    part[threadIdx.x] = s;
+    __syncthreads();
+    for (int d = 1; d < 1024; d <<= 1) {  // inclusive scan of the thread sums
+        const unsigned long long y = threadIdx.x >= d ? part[threadIdx.x - d] : 0;
+        __syncthreads();
+        part[threadIdx.x] += y;
+        __syncthreads();
+    }
+    const unsigned long long first = *base;
+    unsigned long long o = first + part[threadIdx.x] - s;
+    for (int b = b0; b < b1; ++b) {
+        boff[b] = o;
+        o += bcount[b];
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) *base = first + part[1023];
+}
+
+template <int FMT>
+__global__ void __launch_bounds__(DEC_THREADS)
+    dec_text_kernel(const unsigned char* __restrict__ c, unsigned long long len, long long b0,
+                    const unsigned long long* __restrict__ boff, const EncTable* pow10, DecDst d,
+                    DecFlag* __restrict__ list, unsigned long long* __restrict__ st) {
+    __shared__ EncTable tab;
+    __shared__ unsigned short starts[DEC_SEG];
+    __shared__ unsigned int warp_sum[DEC_THREADS / 32];
+    const enc::Pow10 t = enc_load_table(tab, pow10);
+    const unsigned char sep = FMT == enc::FMT_CSV ? '\n' : ',';
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const long long b = b0 + blockIdx.x;
+    unsigned long long at;
+    unsigned int m = dec_starts(c, len, b, sep, &at);
+    // exclusive block scan of the start counts: this thread's starts go to starts[before ..]
+    const unsigned int n = __popc(m);
+    unsigned int incl = n;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const unsigned int y = __shfl_up_sync(0xffffffffu, incl, o);
+        if (lane >= o) incl += y;
+    }
+    if (lane == 31) warp_sum[warp] = incl;
+    __syncthreads();
+    unsigned int before = incl - n, total = 0;
+    for (int w = 0; w < DEC_THREADS / 32; ++w) {
+        if (w < warp) before += warp_sum[w];
+        total += warp_sum[w];
+    }
+    const unsigned long long seg = (unsigned long long)b * DEC_SEG;
+    for (; m; m &= m - 1) starts[before++] = (unsigned short)(at - seg + __ffs(m) - 1);
+    __syncthreads();
+    bool bad = false;
+    for (unsigned int r = threadIdx.x; r < total; r += DEC_THREADS) {
+        const unsigned long long p = seg + starts[r], rec = boff[b] + r;
+        unsigned long long e = p;
+        while (e < len && c[e] != sep) ++e;
+        if (rec >= d.n) {
+            bad = true;
+            continue;
+        }
+        const unsigned char* num = c + p;
+        if (FMT == enc::FMT_CSV) {  // record rec carries the indices of site rec
+            const unsigned long long i = rec / d.plane, jk = rec - i * d.plane, j = jk / d.sz;
+            if (dec::csv_record(c + p, c + e, i, j, jk - j * d.sz, &num) != dec::TOK_OK) {
+                bad = true;
+                continue;
+            }
+        }
+        double v;
+        const int rc = dec::parse_f64(num, c + e, t, &v);
+        if (rc == dec::TOK_BAD) {
+            bad = true;
+            continue;
+        }
+        const unsigned long long plane = rec / d.plane;
+        if (plane < d.p0 || plane >= d.p1) continue;
+        if (rc == dec::TOK_OK) {
+            d.dst[rec - d.p0 * d.plane] = v;
+        } else {
+            const unsigned long long k = atomicAdd(st + DEC_NFLAG, 1ull);
+            if (k < DEC_FLAG_CAP) list[k] = DecFlag{rec, (unsigned int)(num - c), (unsigned int)(c + e - num), 0.0};
+        }
+    }
+    if (bad) atomicOr(st + DEC_ERR, 1ull);
+}
+
+// elements [e0, e0 + nel) of a Messagepack array: 0xcb and the big-endian bits, 9 bytes each
+__global__ void __launch_bounds__(DEC_THREADS)
+    dec_mpk_kernel(const unsigned char* __restrict__ c, unsigned long long nel, unsigned long long e0, DecDst d,
+                   unsigned long long* __restrict__ st) {
+    bool bad = false;
+    for (unsigned long long i = (unsigned long long)blockIdx.x * DEC_THREADS + threadIdx.x; i < nel;
+         i += (unsigned long long)gridDim.x * DEC_THREADS) {
+        const unsigned char* q = c + 9 * i;
+        if (q[0] != 0xcb) {
+            bad = true;
+            continue;
+        }
+        const unsigned long long rec = e0 + i, plane = rec / d.plane;
+        if (plane < d.p0 || plane >= d.p1) continue;
+        unsigned long long u = 0;
+        for (int k = 1; k < 9; ++k) u = (u << 8) | q[k];
+        d.dst[rec - d.p0 * d.plane] = __longlong_as_double((long long)u);
+    }
+    if (bad) atomicOr(st + DEC_ERR, 1ull);
+}
+
+// the numbers converted on the host
+__global__ void dec_scatter_kernel(DecDst d, const DecFlag* __restrict__ list, int n) {
+    for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < n; k += gridDim.x * blockDim.x)
+        d.dst[list[k].rec - d.p0 * d.plane] = list[k].v;
+}
 }  // namespace
 
 struct Tb2Sched {  // work lists of the persistent time-tiled sweep for one plane range (device arrays, sweep_tb.cuh Sched)
@@ -223,6 +394,14 @@ struct wafer_ctx {
     EncFlagStr* wr_txt = nullptr;
     unsigned long long* wr_count = nullptr;  // [0] refused sites collected, [1] refused sites the emit pass did not find
     unsigned long long* wr_red = nullptr;
+    // wafer_load_array, per bounce buffer: the decoder's block counts and record offsets, the uncertified numbers, the
+    // chunk's state words (DEC_ERR, DEC_NFLAG) and their pinned mirror; the running record count
+    unsigned int* rd_bcount[2] = {nullptr, nullptr};
+    unsigned long long* rd_boff[2] = {nullptr, nullptr};
+    DecFlag* rd_flags[2] = {nullptr, nullptr};
+    unsigned long long* rd_st = nullptr;    // 2 x DEC_WORDS, then the running record count
+    unsigned long long* rd_hst = nullptr;   // pinned, 2 x DEC_WORDS
+    long long rd_blocks = 0;                // blocks rd_bcount / rd_boff hold
     // source staging of the resampling entries when two source planes do not fit a bounce buffer (<= 128 MB each)
     double* rs_stg[2] = {nullptr, nullptr};
     long long rs_cap = 0;           // doubles one of them holds
@@ -1019,41 +1198,69 @@ bool resample_copies(const wafer_ctx* ctx, uint64_t sx, uint64_t sy, uint64_t sz
     return from_csv && sx == (uint64_t)ctx->g.gnx && sy == (uint64_t)ctx->g.gny && sz == (uint64_t)ctx->g.gnz;
 }
 
-int resample_args(wafer_ctx* ctx, const double* src, uint64_t sx, uint64_t sy, uint64_t sz, uint32_t from_csv) {
+// What this rank's planes read of an (sx, sy, sz) source: the global work planes [ga, gb) of the slab inside the
+// lattice (ghosts included) and the source x-planes [sp0, sp1) they need.
+struct RsPlan {
+    bool copy;  // a work-sized Csv source, copied straight in
+    long long ga, gb, sp0, sp1;
+};
+
+// lowest source plane behind global work plane gi (the planes [lo, lo + 1 + !copy) are read)
+long long rs_lo(const wafer_ctx* ctx, const RsPlan& pl, uint64_t sx, long long gi) {
+    if (pl.copy) return gi;
+    long long i0;
+    double d;
+    rs_bracket((long long)sx, ctx->g.gnx + 2 * ctx->g.e, gi, &i0, &d);
+    return i0;
+}
+
+// The shape rules of fill_data / read_csv for both the host-staged entries and wafer_load_array
+int resample_shape(wafer_ctx* ctx, uint64_t sx, uint64_t sy, uint64_t sz, uint32_t from_csv, RsPlan* pl) {
     const Geom& g = ctx->g;
     const uint64_t e2 = 2 * (uint64_t)g.e;
-    REQUIRE(src, "src is NULL");
-    REQUIRE(from_csv <= 1, "from_csv must be 0 (Messagepack / Json) or 1 (Csv)");
     REQUIRE(sx > 0 && sy > 0 && sz > 0, "ArrayShape: the input array has a zero dimension");
     REQUIRE(from_csv || !(sx == g.gnx + e2 && sy == g.gny + e2 && sz == g.gnz + e2),
             "input array already has the padded size: the reference's fill_data cannot load it (input.rs:167-169)");
-    REQUIRE(resample_copies(ctx, sx, sy, sz, from_csv) || (sx >= 2 && sy >= 2 && sz >= 2),
-            "ArrayShape: the input array cannot be resized (needs >= 2 points per axis)");
+    pl->copy = resample_copies(ctx, sx, sy, sz, from_csv);
+    REQUIRE(pl->copy || (sx >= 2 && sy >= 2 && sz >= 2), "ArrayShape: the input array cannot be resized (needs >= 2 points per axis)");
+    pl->ga = std::max<long long>(0, g.x0 - g.gx);
+    pl->gb = std::min<long long>(g.gnx, g.x0 + g.L + g.gx);
+    pl->sp0 = rs_lo(ctx, *pl, sx, pl->ga);
+    pl->sp1 = rs_lo(ctx, *pl, sx, pl->gb - 1) + (pl->copy ? 1 : 2);
+    return WAFER_OK;
+}
+
+int resample_args(wafer_ctx* ctx, const double* src, uint64_t sx, uint64_t sy, uint64_t sz, uint32_t from_csv, RsPlan* pl) {
+    REQUIRE(src, "src is NULL");
+    REQUIRE(from_csv <= 1, "from_csv must be 0 (Messagepack / Json) or 1 (Csv)");
+    TRY(resample_shape(ctx, sx, sy, sz, from_csv, pl));
     REQUIRE(sy <= (uint64_t)RS_MAX_STG / 2 && sz <= (uint64_t)RS_MAX_STG / 2 / sy,
             "input array: two of its x-planes (2*sy*sz*8 bytes) exceed the 128 MB staging buffer");
     return WAFER_OK;
 }
 
-// the arguments passed resample_args
-int resample_into(wafer_ctx* ctx, const double* src, uint64_t sx, uint64_t sy, uint64_t sz, uint32_t from_csv, double* dst) {
+void rs_launch(wafer_ctx* ctx, const RsPlan& pl, double* dst, const double* src, long long s0, uint64_t sx, uint64_t sy,
+               uint64_t sz, long long a, long long b) {
     const Geom& g = ctx->g;
-    const bool copy = resample_copies(ctx, sx, sy, sz, from_csv);
-    const long long splane = (long long)(sy * sz), need = copy ? 1 : 2;
-    // global work planes of the slab inside the lattice (ghosts included) and the source planes [lo, lo + need) of each
-    const long long ga = std::max<long long>(0, g.x0 - g.gx), gb = std::min<long long>(g.gnx, g.x0 + g.L + g.gx);
-    const long long bx = g.gnx + 2 * g.e;
-    auto lo = [&](long long gi) {
-        if (copy) return gi;
-        long long i0;
-        double d;
-        rs_bracket((long long)sx, bx, gi, &i0, &d);
-        return i0;
-    };
+    const int ztiles = std::min(ceil_div(g.nz, RS_ZTILE), 65535);
+    const int i0 = (int)(a - g.x0), i1 = (int)(b - g.x0);
+    const dim3 grid((unsigned)std::min<long long>((long long)(i1 - i0) * g.ny, std::max(1, ctx->sm_count * 8 / ztiles)),
+                    (unsigned)ztiles);
+    if (pl.copy) resample_kernel<true><<<grid, RS_THREADS, 0, ctx->s_main>>>(dst, g, src, s0, (long long)sx, (long long)sy, (long long)sz, i0, i1);
+    else resample_kernel<false><<<grid, RS_THREADS, 0, ctx->s_main>>>(dst, g, src, s0, (long long)sx, (long long)sy, (long long)sz, i0, i1);
+}
+
+// the arguments passed resample_args
+int resample_into(wafer_ctx* ctx, const RsPlan& pl, const double* src, uint64_t sx, uint64_t sy, uint64_t sz, double* dst) {
+    const Geom& g = ctx->g;
+    const long long splane = (long long)(sy * sz), need = pl.copy ? 1 : 2;
+    auto lo = [&](long long gi) { return rs_lo(ctx, pl, sx, gi); };
+    const long long ga = pl.ga, gb = pl.gb;
     TRY(ensure_staging(ctx));
     double* buf[2] = {ctx->stg[0], ctx->stg[1]};
     long long cap = ctx->stg_planes * (long long)(g.ny + 2 * g.e) * (g.nz + 2 * g.e) / splane;  // source planes per buffer
     if (cap < need) {
-        cap = std::min<long long>(RS_MAX_STG / splane, gb > ga ? lo(gb - 1) + need - lo(ga) : need);
+        cap = std::min<long long>(RS_MAX_STG / splane, pl.sp1 - pl.sp0);
         if (ctx->rs_cap < cap * splane) {  // the last call that used them synchronised before returning
             for (int b = 0; b < 2; ++b) {
                 cudaFree(ctx->rs_stg[b]);
@@ -1068,7 +1275,6 @@ int resample_into(wafer_ctx* ctx, const double* src, uint64_t sx, uint64_t sy, u
     }
     CK(cudaEventRecord(ctx->ev_stg_free[0], ctx->s_main));  // everything queued so far precedes the first refill
     CK(cudaEventRecord(ctx->ev_stg_free[1], ctx->s_main));
-    const int ztiles = std::min(ceil_div(g.nz, RS_ZTILE), 65535);
     int k = 0;
     for (long long a = ga; a < gb; ++k) {
         const long long s0 = lo(a);
@@ -1081,17 +1287,42 @@ int resample_into(wafer_ctx* ctx, const double* src, uint64_t sx, uint64_t sy, u
                            ctx->s_copy));
         CK(cudaEventRecord(ctx->ev_stg_full[nb], ctx->s_copy));
         CK(cudaStreamWaitEvent(ctx->s_main, ctx->ev_stg_full[nb], 0));
-        const int i0 = (int)(a - g.x0), i1 = (int)(b - g.x0);
-        const dim3 grid((unsigned)std::min<long long>((long long)(i1 - i0) * g.ny, std::max(1, ctx->sm_count * 8 / ztiles)),
-                        (unsigned)ztiles);
-        if (copy) resample_kernel<true><<<grid, RS_THREADS, 0, ctx->s_main>>>(dst, g, buf[nb], s0, (long long)sx, (long long)sy, (long long)sz, i0, i1);
-        else resample_kernel<false><<<grid, RS_THREADS, 0, ctx->s_main>>>(dst, g, buf[nb], s0, (long long)sx, (long long)sy, (long long)sz, i0, i1);
+        rs_launch(ctx, pl, dst, buf[nb], s0, sx, sy, sz, a, b);
         TRY(post_launch(ctx));
         CK(cudaEventRecord(ctx->ev_stg_free[nb], ctx->s_main));
         a = b;
     }
     CK(cudaStreamSynchronize(ctx->s_main));  // the caller may free `src` on return
     return WAFER_OK;
+}
+
+enum { RS_PHI = 0, RS_POTENTIAL, RS_LOWER };
+
+// the effects of wafer_set_phi (which = RS_PHI), wafer_set_potential or wafer_push_lower, with fill(dst) writing the
+// work area of the field
+template <class Fill>
+int set_input(wafer_ctx* ctx, int which, Fill fill) {
+    if (which == RS_PHI) {  // the ring is +0 by construction
+        ctx->chk_valid = false;  // psi (or what the check sums depend on) changes
+        const int rc = fill(ctx->psi[ctx->cur]);
+        ctx->have_phi = rc == WAFER_OK;
+        return rc;
+    }
+    if (which == RS_POTENTIAL) {
+        ctx->chk_valid = false;
+        ctx->h_valid = false;
+        TRY(fill(ctx->v));
+        TRY(ensure_ab(ctx));
+        ctx->have_v = true;
+        return WAFER_OK;
+    }
+    REQUIRE(ctx->lowers.size() < 255, "at most 255 lower states (wavenum is a u8, config.rs:308)");
+    double* q = nullptr;
+    TRY(alloc_field(ctx, &q));
+    int rc = fill(q);
+    if (rc == WAFER_OK) rc = register_lower(ctx, q);
+    if (rc != WAFER_OK) cudaFree(q);
+    return rc;
 }
 
 int create_impl(const wafer_params* params, wafer_ctx* ctx) {
@@ -1235,6 +1466,11 @@ int wafer_destroy(wafer_ctx* ctx) {
         if (ctx->wr_host[b]) cudaFreeHost(ctx->wr_host[b]);
     cudaFree(ctx->wr_btot); cudaFree(ctx->wr_boff); cudaFree(ctx->wr_flags); cudaFree(ctx->wr_txt); cudaFree(ctx->wr_count);
     cudaFree(ctx->wr_red); cudaFree(ctx->wr_pow10);
+    for (int b = 0; b < 2; ++b) {
+        cudaFree(ctx->rd_bcount[b]); cudaFree(ctx->rd_boff[b]); cudaFree(ctx->rd_flags[b]);
+    }
+    cudaFree(ctx->rd_st);
+    if (ctx->rd_hst) cudaFreeHost(ctx->rd_hst);
     cudaFree(ctx->d_cksum); cudaFree(ctx->gram);
     for (auto& kv : ctx->tb2_sched) {
         cudaFree(kv.second.bulk); cudaFree(kv.second.segs); cudaFree(kv.second.first); cudaFree(kv.second.counters);
@@ -1535,35 +1771,13 @@ int wafer_symmetrise(wafer_ctx* ctx, int32_t kind) {
 }
 
 // ---- input files resampled on the device (resample.cuh) -------------------------------------------------------
-enum { RS_PHI = 0, RS_POTENTIAL, RS_LOWER };
-
 static int resampled_impl(wafer_ctx* ctx, int which, const double* src, uint64_t sx, uint64_t sy, uint64_t sz,
                           uint32_t from_csv) {
     if (!ctx) return WAFER_ERR_INVALID;
-    TRY(resample_args(ctx, src, sx, sy, sz, from_csv));  // before anything is allocated or written
+    RsPlan pl;
+    TRY(resample_args(ctx, src, sx, sy, sz, from_csv, &pl));  // before anything is allocated or written
     CK(cudaSetDevice(ctx->dev));
-    if (which == RS_PHI) {  // the effects of wafer_set_phi; the ring is +0 by construction
-        ctx->chk_valid = false;  // psi (or what the check sums depend on) changes
-        const int rc = resample_into(ctx, src, sx, sy, sz, from_csv, ctx->psi[ctx->cur]);
-        ctx->have_phi = rc == WAFER_OK;
-        return rc;
-    }
-    if (which == RS_POTENTIAL) {  // the effects of wafer_set_potential
-        ctx->chk_valid = false;
-        ctx->h_valid = false;
-        TRY(resample_into(ctx, src, sx, sy, sz, from_csv, ctx->v));
-        TRY(ensure_ab(ctx));
-        ctx->have_v = true;
-        return WAFER_OK;
-    }
-    // the effects of wafer_push_lower
-    REQUIRE(ctx->lowers.size() < 255, "at most 255 lower states (wavenum is a u8, config.rs:308)");
-    double* q = nullptr;
-    TRY(alloc_field(ctx, &q));
-    int rc = resample_into(ctx, src, sx, sy, sz, from_csv, q);
-    if (rc == WAFER_OK) rc = register_lower(ctx, q);
-    if (rc != WAFER_OK) cudaFree(q);
-    return rc;
+    return set_input(ctx, which, [&](double* dst) { return resample_into(ctx, pl, src, sx, sy, sz, dst); });
 }
 
 static int resampled(wafer_ctx* ctx, int which, const char* name, const double* src, uint64_t sx, uint64_t sy,
@@ -1905,6 +2119,296 @@ int wafer_write_array(wafer_ctx* ctx, int32_t what, int32_t file_type, const cha
         return write_array_impl(ctx, what, file_type, path, stats);
     } catch (const std::exception& e) {  // host-side allocation failures must not unwind through the C ABI
         if (ctx) ctx->err = std::string("wafer_write_array: ") + e.what();
+        return WAFER_ERR_INVALID;
+    }
+}
+
+// ---- array files decoded on the device (decode.cuh) -----------------------------------------------------------
+// The preamble (and Json's trailer, a Csv file's last record) is read on the host; the shape rules give the source
+// planes this rank needs, converted into one device buffer.  The body is then read with pread into the two pinned
+// buffers, chunk after chunk; each goes to the device through a bounce buffer on s_copy and is decoded on s_main
+// while the next one is read.  A chunk ends after its last separator, the rest is carried into the next.  Once a
+// chunk's kernels are done its uncertified numbers are converted with strtod from the pinned buffer it is still in.
+// The field changes only after the whole file has been read and found canonical: then resample_kernel reads the
+// buffer.
+static int dec_buffers(wafer_ctx* ctx) {
+    TRY(wr_buffers(ctx, 1));  // bounce buffers of at least two blocks of Csv rows, pinned host buffers, the power table
+    const long long nb = (long long)(ctx->stg_bytes / DEC_SEG) + 1;
+    if (ctx->rd_blocks < nb) {
+        for (int b = 0; b < 2; ++b) {
+            cudaFree(ctx->rd_bcount[b]);
+            cudaFree(ctx->rd_boff[b]);
+            ctx->rd_bcount[b] = nullptr;
+            ctx->rd_boff[b] = nullptr;
+        }
+        ctx->rd_blocks = 0;
+        for (int b = 0; b < 2; ++b) {
+            CK(cudaMalloc(&ctx->rd_bcount[b], (size_t)nb * sizeof(unsigned int)));
+            CK(cudaMalloc(&ctx->rd_boff[b], (size_t)nb * sizeof(unsigned long long)));
+        }
+        ctx->rd_blocks = nb;
+    }
+    if (!ctx->rd_st) {
+        for (int b = 0; b < 2; ++b) CK(cudaMalloc(&ctx->rd_flags[b], DEC_FLAG_CAP * sizeof(DecFlag)));
+        CK(cudaMalloc(&ctx->rd_st, (2 * DEC_WORDS + 1) * sizeof(unsigned long long)));
+        CK(cudaMallocHost(&ctx->rd_hst, 2 * DEC_WORDS * sizeof(unsigned long long)));
+    }
+    return WAFER_OK;
+}
+
+static bool rd_pread(int fd, void* p, size_t n, unsigned long long off, std::string* err) {
+    char* c = (char*)p;
+    while (n > 0) {
+        const ssize_t r = pread(fd, c, n, (off_t)off);
+        if (r < 0 && errno == EINTR) continue;
+        if (r <= 0) {
+            *err = std::string("read failed: ") + (r < 0 ? strerror(errno) : "unexpected end of file");
+            return false;
+        }
+        c += r;
+        n -= (size_t)r;
+        off += (unsigned long long)r;
+    }
+    return true;
+}
+
+struct RdChunk {
+    int buf;
+    unsigned long long len;  // bytes of whole records
+    long long nblocks;
+};
+
+struct RdJob {
+    int fmt;
+    DecDst d;
+    unsigned long long host_converted = 0;
+};
+
+static int rd_launch_text(wafer_ctx* ctx, const RdJob& job, const RdChunk& ch, long long b0, long long b1) {
+    unsigned long long* st = ctx->rd_st + DEC_WORDS * ch.buf;
+    const unsigned char* c = (const unsigned char*)ctx->stg[ch.buf];
+    CK(cudaMemsetAsync(st + DEC_NFLAG, 0, sizeof(unsigned long long), ctx->s_main));
+    if (job.fmt == enc::FMT_CSV)
+        dec_text_kernel<enc::FMT_CSV><<<(unsigned)(b1 - b0), DEC_THREADS, 0, ctx->s_main>>>(c, ch.len, b0, ctx->rd_boff[ch.buf], ctx->wr_pow10, job.d, ctx->rd_flags[ch.buf], st);
+    else
+        dec_text_kernel<enc::FMT_JSON><<<(unsigned)(b1 - b0), DEC_THREADS, 0, ctx->s_main>>>(c, ch.len, b0, ctx->rd_boff[ch.buf], ctx->wr_pow10, job.d, ctx->rd_flags[ch.buf], st);
+    TRY(post_launch(ctx));
+    CK(cudaMemcpyAsync(ctx->rd_hst + DEC_WORDS * ch.buf, st, DEC_WORDS * sizeof(unsigned long long), cudaMemcpyDeviceToHost,
+                       ctx->s_main));
+    return WAFER_OK;
+}
+
+// convert the listed numbers of blocks [b0, b1) of the chunk (its kernels done) with strtod and store them
+static int rd_host_convert(wafer_ctx* ctx, RdJob& job, const RdChunk& ch, long long b0, long long b1) {
+    const unsigned long long* hst = ctx->rd_hst + DEC_WORDS * ch.buf;
+    if (hst[DEC_ERR]) return WAFER_ERR_FORMAT;
+    const unsigned long long n = hst[DEC_NFLAG];
+    if (n == 0) return WAFER_OK;
+    if (n > DEC_FLAG_CAP) {  // the list overflowed: again in pieces of 16 blocks, which cannot overflow it
+        for (long long p = b0; p < b1; p += DEC_FLAG_CAP / DEC_SEG) {
+            const long long pe = std::min<long long>(b1, p + DEC_FLAG_CAP / DEC_SEG);
+            TRY(rd_launch_text(ctx, job, ch, p, pe));
+            CK(cudaStreamSynchronize(ctx->s_main));
+            TRY(rd_host_convert(ctx, job, ch, p, pe));
+        }
+        return WAFER_OK;
+    }
+    std::vector<DecFlag> list(n);
+    CK(cudaMemcpyAsync(list.data(), ctx->rd_flags[ch.buf], n * sizeof(DecFlag), cudaMemcpyDeviceToHost, ctx->s_main));
+    CK(cudaStreamSynchronize(ctx->s_main));
+    const char* hb = (const char*)ctx->wr_host[ch.buf];
+    std::string tok;
+    for (DecFlag& f : list) {
+        if ((unsigned long long)f.at + f.len > ch.len) { ctx->err = "wafer_load_array: a listed number lies outside its chunk"; return WAFER_ERR_CUDA; }
+        tok.assign(hb + f.at, f.len);  // the grammar of parse_f64 is a subset of strtod's: it takes the whole token
+        char* end = nullptr;
+        f.v = strtod(tok.c_str(), &end);
+        if (end != tok.c_str() + tok.size()) return WAFER_ERR_FORMAT;
+    }
+    CK(cudaMemcpyAsync(ctx->rd_flags[ch.buf], list.data(), n * sizeof(DecFlag), cudaMemcpyHostToDevice, ctx->s_main));
+    dec_scatter_kernel<<<(unsigned)std::min<unsigned long long>((n + 255) / 256, 1024), 256, 0, ctx->s_main>>>(job.d, ctx->rd_flags[ch.buf], (int)n);
+    TRY(post_launch(ctx));
+    CK(cudaStreamSynchronize(ctx->s_main));  // `list` is freed on return
+    job.host_converted += n;
+    return WAFER_OK;
+}
+
+// a chunk whose kernels are queued: wait for them, then its status and its uncertified numbers
+static int rd_finish(wafer_ctx* ctx, RdJob& job, const RdChunk& ch) {
+    CK(cudaEventSynchronize(ctx->ev_stg_free[ch.buf]));
+    if (ctx->rd_hst[DEC_WORDS * ch.buf + DEC_ERR]) return WAFER_ERR_FORMAT;
+    if (job.fmt == enc::FMT_MPK) return WAFER_OK;
+    return rd_host_convert(ctx, job, ch, 0, ch.nblocks);
+}
+
+// bytes [b0, b1) of the file: every chunk decoded into job.d
+static int rd_stream(wafer_ctx* ctx, RdJob& job, int fd, unsigned long long b0, unsigned long long b1, std::string* io) {
+    const unsigned char sep = job.fmt == enc::FMT_CSV ? '\n' : ',';
+    const unsigned long long cap = job.fmt == enc::FMT_MPK ? ctx->stg_bytes / 9 * 9 : ctx->stg_bytes;
+    unsigned long long off = b0, carry = 0;
+    RdChunk prev{0, 0, 0};
+    CK(cudaMemsetAsync(ctx->rd_st, 0, (2 * DEC_WORDS + 1) * sizeof(unsigned long long), ctx->s_main));
+    CK(cudaEventRecord(ctx->ev_stg_free[0], ctx->s_main));
+    CK(cudaEventRecord(ctx->ev_stg_free[1], ctx->s_main));
+    for (int k = 0; off < b1; ++k) {
+        const int buf = k & 1;
+        unsigned char* hb = ctx->wr_host[buf];
+        const unsigned long long e0 = (off - b0) / 9;  // Messagepack: the chunk's first element
+        if (carry) memcpy(hb, ctx->wr_host[buf ^ 1] + prev.len, carry);  // chunk k - 1's split record
+        const unsigned long long n = std::min(cap - carry, b1 - off);
+        if (!rd_pread(fd, hb + carry, n, off, io)) return WAFER_ERR_IO;
+        off += n;
+        unsigned long long len = carry + n;
+        carry = 0;
+        if (off < b1 && job.fmt != enc::FMT_MPK) {  // end the chunk after its last separator
+            unsigned long long cut = len;
+            while (cut > 0 && hb[cut - 1] != sep) --cut;
+            if (cut == 0) return WAFER_ERR_FORMAT;  // a record longer than a bounce buffer
+            carry = len - cut;
+            len = cut;
+        }
+        RdChunk ch{buf, len, (long long)((len + DEC_SEG - 1) / DEC_SEG)};
+        unsigned char* db = (unsigned char*)ctx->stg[buf];
+        CK(cudaStreamWaitEvent(ctx->s_copy, ctx->ev_stg_free[buf], 0));  // chunk k - 2's kernels are done with it
+        CK(cudaMemcpyAsync(db, hb, len, cudaMemcpyHostToDevice, ctx->s_copy));
+        CK(cudaEventRecord(ctx->ev_stg_full[buf], ctx->s_copy));
+        CK(cudaStreamWaitEvent(ctx->s_main, ctx->ev_stg_full[buf], 0));
+        unsigned long long* st = ctx->rd_st + DEC_WORDS * buf;
+        if (job.fmt == enc::FMT_MPK) {
+            const unsigned long long nel = len / 9;
+            dec_mpk_kernel<<<(unsigned)std::min<unsigned long long>((nel + DEC_THREADS - 1) / DEC_THREADS, (unsigned long long)ctx->sm_count * 16),
+                             DEC_THREADS, 0, ctx->s_main>>>(db, nel, e0, job.d, st);
+            TRY(post_launch(ctx));
+            CK(cudaMemcpyAsync(ctx->rd_hst + DEC_WORDS * buf, st, DEC_WORDS * sizeof(unsigned long long), cudaMemcpyDeviceToHost,
+                               ctx->s_main));
+        } else {
+            dec_count_kernel<<<(unsigned)ch.nblocks, DEC_THREADS, 0, ctx->s_main>>>(db, len, sep, ctx->rd_bcount[buf]);
+            dec_offsets_kernel<<<1, 1024, 0, ctx->s_main>>>(ctx->rd_bcount[buf], (int)ch.nblocks, ctx->rd_boff[buf],
+                                                            ctx->rd_st + 2 * DEC_WORDS);
+            TRY(post_launch(ctx, 2));
+            TRY(rd_launch_text(ctx, job, ch, 0, ch.nblocks));
+        }
+        CK(cudaEventRecord(ctx->ev_stg_free[buf], ctx->s_main));
+        if (k > 0) TRY(rd_finish(ctx, job, prev));  // chunk k - 1, while chunk k is decoded
+        prev = ch;
+    }
+    if (off > b0) TRY(rd_finish(ctx, job, prev));
+    if (job.fmt != enc::FMT_MPK) {  // every site had its record
+        unsigned long long recs = 0;
+        CK(cudaMemcpyAsync(&recs, ctx->rd_st + 2 * DEC_WORDS, sizeof(recs), cudaMemcpyDeviceToHost, ctx->s_main));
+        CK(cudaStreamSynchronize(ctx->s_main));
+        if (recs != job.d.n) return WAFER_ERR_FORMAT;
+    }
+    return WAFER_OK;
+}
+
+namespace {
+struct DevBuf {  // the converted source planes; freed once the work queued on them is done
+    wafer_ctx* ctx;
+    double* p = nullptr;
+    ~DevBuf() {
+        cudaStreamSynchronize(ctx->s_copy);
+        cudaStreamSynchronize(ctx->s_main);
+        cudaFree(p);
+    }
+};
+}  // namespace
+
+static int load_array_impl(wafer_ctx* ctx, int32_t what, int32_t file_type, const char* path, wafer_load_stats* stats) {
+    if (!ctx) return WAFER_ERR_INVALID;
+    REQUIRE(what >= 0 && what <= 2, "what must be 0 (psi), 1 (V) or 2 (push a lower state)");
+    REQUIRE(file_type >= 0 && file_type <= 2,
+            "file_type must be 0 (Messagepack), 1 (Csv) or 2 (Json); Yaml and Ron files are not supported");
+    REQUIRE(path, "path is NULL");
+    CK(cudaSetDevice(ctx->dev));
+    FdGuard fd;
+    fd.fd = open(path, O_RDONLY | O_CLOEXEC);
+    std::string io;
+    struct stat sb;
+    if (fd.fd < 0 || fstat(fd.fd, &sb) != 0) {
+        ctx->err = std::string("wafer_load_array: cannot open ") + path + ": " + strerror(errno);
+        return WAFER_ERR_IO;
+    }
+    const unsigned long long size = (unsigned long long)sb.st_size;
+    auto not_canonical = [&](const char* why) {
+        ctx->err = std::string("wafer_load_array: ") + path + ": " + why + " (not a layout the device decoder reads)";
+        return WAFER_ERR_FORMAT;
+    };
+    auto io_error = [&]() {
+        ctx->err = std::string("wafer_load_array: ") + path + ": " + io;
+        return WAFER_ERR_IO;
+    };
+    // preamble, trailer, dims: the body [b0, b1) holds the records
+    uint64_t dims[3] = {0, 0, 0};
+    unsigned long long b0 = 0, b1 = size;
+    unsigned char head[128], tail[4096];
+    const unsigned long long nh = std::min<unsigned long long>(size, sizeof head);
+    if (!rd_pread(fd.fd, head, nh, 0, &io)) return io_error();
+    if (file_type == enc::FMT_MPK) {
+        uint64_t count = 0;
+        const int h = dec::mpk_header(head, nh, dims, &count);
+        if (h < 0) return not_canonical("Messagepack preamble");
+        b0 = (unsigned long long)h;
+    } else if (file_type == enc::FMT_JSON) {
+        const int h = dec::json_header(head, nh, dims);
+        if (h < 0) return not_canonical("Json preamble");
+        const unsigned long long nt = std::min<unsigned long long>(size - (unsigned long long)h, 8);
+        if (!rd_pread(fd.fd, tail, nt, size - nt, &io)) return io_error();
+        const int tl = dec::json_trailer(tail, nt);
+        if (tl < 0) return not_canonical("Json trailer");
+        b0 = (unsigned long long)h;
+        b1 = size - (unsigned long long)tl;
+    } else {
+        const unsigned long long nt = std::min<unsigned long long>(size, sizeof tail);
+        if (!rd_pread(fd.fd, tail, nt, size - nt, &io)) return io_error();
+        if (!dec::csv_dims(tail, nt, nt == size, dims)) return not_canonical("Csv last record");
+    }
+    if (!dec::body_fits(file_type, dims[0] * dims[1] * dims[2], b1 - b0))
+        return not_canonical("the file is too short for its dims");
+    RsPlan pl;
+    TRY(resample_shape(ctx, dims[0], dims[1], dims[2], file_type == enc::FMT_CSV ? 1 : 0, &pl));
+    TRY(dec_buffers(ctx));
+    RdJob job;
+    job.fmt = file_type;
+    job.d.n = dims[0] * dims[1] * dims[2];
+    job.d.plane = dims[1] * dims[2];
+    job.d.sz = dims[2];
+    job.d.p0 = (unsigned long long)pl.sp0;
+    job.d.p1 = (unsigned long long)pl.sp1;
+    DevBuf src{ctx};
+    const unsigned long long nsrc = (unsigned long long)(pl.sp1 - pl.sp0) * job.d.plane;  // <= n <= file bytes
+    if (nsrc > SIZE_MAX / sizeof(double) || cudaMalloc(&src.p, (size_t)nsrc * sizeof(double)) != cudaSuccess) {
+        cudaGetLastError();
+        src.p = nullptr;
+        return not_canonical("the source planes do not fit the device");
+    }
+    job.d.dst = src.p;
+    const int rc = rd_stream(ctx, job, fd.fd, b0, b1, &io);
+    if (rc == WAFER_ERR_IO) return io_error();
+    if (rc == WAFER_ERR_FORMAT) return not_canonical(file_type == enc::FMT_MPK ? "an element is not a float 64" : "a record is not canonical");
+    TRY(rc);
+    TRY(set_input(ctx, what, [&](double* dst) -> int {
+        rs_launch(ctx, pl, dst, src.p, pl.sp0, dims[0], dims[1], dims[2], pl.ga, pl.gb);
+        TRY(post_launch(ctx));
+        CK(cudaStreamSynchronize(ctx->s_main));
+        return WAFER_OK;
+    }));
+    if (stats) {
+        stats->sx = dims[0];
+        stats->sy = dims[1];
+        stats->sz = dims[2];
+        stats->bytes_read = size;
+        stats->sites_converted = nsrc;
+        stats->host_converted = job.host_converted;
+    }
+    return WAFER_OK;
+}
+
+int wafer_load_array(wafer_ctx* ctx, int32_t what, int32_t file_type, const char* path, wafer_load_stats* stats) {
+    try {
+        return load_array_impl(ctx, what, file_type, path, stats);
+    } catch (const std::exception& e) {  // host-side allocation failures must not unwind through the C ABI
+        if (ctx) ctx->err = std::string("wafer_load_array: ") + e.what();
         return WAFER_ERR_INVALID;
     }
 }
