@@ -400,8 +400,9 @@ def test_large_sources_stream_and_are_exact_at_sampled_sites(wb, n, src_n):
 
 
 @gpu
-def test_large_source_on_a_small_lattice_uses_its_own_staging(wb):
-    """a 256^3 source down-sampled onto 40^3: one source plane pair is larger than the lattice's bounce buffers"""
+def test_large_source_on_a_small_lattice_grows_the_staging_ring(wb):
+    """a 256^3 source down-sampled onto 40^3: one source plane pair is larger than the lattice's staging slots, which
+    grow for it (to at most 128 MB); the next resample, a Csv source, then runs on the grown slots"""
     src = _src((256, 256, 256), 12)
     n = (40, 40, 40)
     with wb.Lattice(n, "SevenPoint", dn=0.1, dt=1e-3, mass=1.0) as lat:

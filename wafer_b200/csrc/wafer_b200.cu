@@ -350,6 +350,18 @@ struct Tb2Sched {  // work lists of the persistent time-tiled sweep for one plan
     int ncta = 0, nbulk = 0;
 };
 
+// The one path between host memory and the device: two device slots, the copy of one on `copy` overlapping the
+// kernels of the other on s_main.  free[b] is recorded when the last user of slot b is done (the kernels that read it,
+// or the copy that drained it), full[b] when its contents are ready for the other side.  The array files also get
+// pinned host halves of the slot size.  Everything is allocated on first use (ring_reserve).
+struct StagingRing {
+    cudaStream_t copy = nullptr;
+    cudaEvent_t free[2] = {nullptr, nullptr}, full[2] = {nullptr, nullptr};
+    void* slot[2] = {nullptr, nullptr};
+    unsigned char* host[2] = {nullptr, nullptr};
+    size_t bytes = 0;  // of one slot (and of one pinned half)
+};
+
 struct wafer_ctx {
     wafer_params p{};
     Geom g{};
@@ -378,23 +390,18 @@ struct wafer_ctx {
     std::map<std::pair<int, int>, std::pair<cudaGraphExec_t, int>> step_graphs;  // exec, kernel launches per replay
     bool chk_valid = false;    // scal[SL_CHK..] holds the point-wise check sums of the CURRENT psi (this rank's share)
     double* gram = nullptr;    // G[i][j] = <q_i, q_j>, j < i, of the stored states (device, GRAM_LD x GRAM_LD)
-    // host <-> device: two small bounce buffers in the host layout, filled / drained on s_copy while the
-    // pack / unpack kernel of the other one runs on s_main (lazily allocated, never a field-sized buffer)
-    double* stg[2] = {nullptr, nullptr};
-    long long stg_planes = 0;       // padded host planes one bounce buffer holds
-    size_t stg_bytes = 0;           // bytes of one bounce buffer (wafer_write_array may enlarge them on small lattices)
-    // wafer_write_array: pinned host halves of the bounce buffers, the encoder's block totals / offsets, the refused
-    // sites of one launch and the host text of those, the all-reduce vector (all allocated on first use)
-    unsigned char* wr_host[2] = {nullptr, nullptr};
+    StagingRing ring;
+    EncTable* pow10 = nullptr;      // the 128-bit power table of the encoder and the decoder (allocated on first use)
+    // wafer_write_array: the encoder's block totals / offsets, the refused sites of one launch and the host text of
+    // those, the all-reduce vector (all allocated on first use)
     unsigned int* wr_btot = nullptr;
     unsigned long long* wr_boff = nullptr;
     long long wr_blocks = 0;        // blocks wr_btot / wr_boff hold
-    EncTable* wr_pow10 = nullptr;
     EncFlagIn* wr_flags = nullptr;
     EncFlagStr* wr_txt = nullptr;
     unsigned long long* wr_count = nullptr;  // [0] refused sites collected, [1] refused sites the emit pass did not find
     unsigned long long* wr_red = nullptr;
-    // wafer_load_array, per bounce buffer: the decoder's block counts and record offsets, the uncertified numbers, the
+    // wafer_load_array, per slot of the ring: the decoder's block counts and record offsets, the uncertified numbers, the
     // chunk's state words (DEC_ERR, DEC_NFLAG) and their pinned mirror; the running record count
     unsigned int* rd_bcount[2] = {nullptr, nullptr};
     unsigned long long* rd_boff[2] = {nullptr, nullptr};
@@ -402,11 +409,6 @@ struct wafer_ctx {
     unsigned long long* rd_st = nullptr;    // 2 x DEC_WORDS, then the running record count
     unsigned long long* rd_hst = nullptr;   // pinned, 2 x DEC_WORDS
     long long rd_blocks = 0;                // blocks rd_bcount / rd_boff hold
-    // source staging of the resampling entries when two source planes do not fit a bounce buffer (<= 128 MB each)
-    double* rs_stg[2] = {nullptr, nullptr};
-    long long rs_cap = 0;           // doubles one of them holds
-    cudaStream_t s_copy = nullptr;
-    cudaEvent_t ev_stg_free[2] = {nullptr, nullptr}, ev_stg_full[2] = {nullptr, nullptr};
     double* partials = nullptr;
     long long partials_cap = 0;
     double* scal = nullptr;
@@ -1075,22 +1077,100 @@ void owned_range(const wafer_ctx* ctx, long long* hp0, long long* hp1) {
     if (ctx->rank == ctx->world - 1) *hp1 = g.gnx + 2 * g.e;
 }
 
-// Bounce buffers: 2 x ~128 MB regardless of the lattice size (a 1024^3 field is 8.8 GB, a full-size staging copy
-// of it was round 1's largest avoidable allocation).
-int ensure_staging(wafer_ctx* ctx) {
-    if (ctx->stg[0]) return WAFER_OK;
+// ---- the staging ring --------------------------------------------------------------------------------------------
+constexpr long long RING_MAX = 128ll << 20;  // no slot grows past it (a field-sized one was 8.8 GB at 1024^3)
+
+long long host_plane(const Geom& g) { return (long long)(g.ny + 2 * g.e) * (g.nz + 2 * g.e); }  // doubles
+
+// Padded planes per chunk of upload / download, and the slots' first size: the smallest of what fits a slot (once there
+// are slots), what fits 128 MB (at least one) and the slab.  So growing the slots changes no chunk here.
+long long ring_planes(const wafer_ctx* ctx) {
     const Geom& g = ctx->g;
-    const long long plane_h = (long long)(g.ny + 2 * g.e) * (g.nz + 2 * g.e);
-    const long long want = std::max<long long>(1, (128ll << 20) / (long long)(plane_h * sizeof(double)));
-    ctx->stg_planes = std::min<long long>(want, g.L + 2 * g.gx + 2 * g.e);
-    ctx->stg_bytes = (size_t)(ctx->stg_planes * plane_h) * sizeof(double);
+    const long long plane = host_plane(g) * (long long)sizeof(double);
+    const long long fit = ctx->ring.bytes ? (long long)ctx->ring.bytes / plane : LLONG_MAX;
+    return std::min({fit, std::max(1ll, RING_MAX / plane), (long long)g.L + 2 * g.gx + 2 * g.e});
+}
+
+// the slots and pinned halves; with `all` (wafer_destroy) the events and the copy stream too
+void ring_free(StagingRing& r, bool all) {
     for (int b = 0; b < 2; ++b) {
-        CK(cudaMalloc(&ctx->stg[b], ctx->stg_bytes));
-        CK(cudaEventCreateWithFlags(&ctx->ev_stg_free[b], cudaEventDisableTiming));
-        CK(cudaEventCreateWithFlags(&ctx->ev_stg_full[b], cudaEventDisableTiming));
+        cudaFree(r.slot[b]);
+        if (r.host[b]) cudaFreeHost(r.host[b]);
+        r.slot[b] = nullptr;
+        r.host[b] = nullptr;
+        if (all && r.free[b]) cudaEventDestroy(r.free[b]);
+        if (all && r.full[b]) cudaEventDestroy(r.full[b]);
     }
-    CK(cudaStreamCreateWithFlags(&ctx->s_copy, cudaStreamNonBlocking));
+    if (all && r.copy) cudaStreamDestroy(r.copy);
+    r.bytes = 0;
+}
+
+// Slots of at least min_bytes and of ring_planes, with pinned halves of the slot size when `pinned` asks for them or
+// they exist.  Every user of the ring synchronises before it returns, so no queued work
+// still uses slots that grow here; the old ones are freed before the new ones are allocated.
+int ring_reserve(wafer_ctx* ctx, size_t min_bytes, bool pinned) {
+    StagingRing& r = ctx->ring;
+    for (cudaEvent_t* e : {&r.free[0], &r.free[1], &r.full[0], &r.full[1]})
+        if (!*e) CK(cudaEventCreateWithFlags(e, cudaEventDisableTiming));
+    if (!r.copy) CK(cudaStreamCreateWithFlags(&r.copy, cudaStreamNonBlocking));
+    const size_t want = std::max(min_bytes, (size_t)(ring_planes(ctx) * host_plane(ctx->g)) * sizeof(double));
+    if (want > r.bytes) {
+        pinned = pinned || r.host[0];
+        ring_free(r, false);
+        for (int b = 0; b < 2; ++b) CK(cudaMalloc(&r.slot[b], want));
+        r.bytes = want;
+    }
+    for (int b = 0; b < 2; ++b)
+        if (pinned && !r.host[b]) CK(cudaMallocHost((void**)&r.host[b], r.bytes));
     return WAFER_OK;
+}
+
+// Once before a loop of ring_in / ring_out: everything queued on s_main so far precedes the first refill of a slot.
+int ring_start(wafer_ctx* ctx) {
+    for (int b = 0; b < 2; ++b) CK(cudaEventRecord(ctx->ring.free[b], ctx->s_main));
+    return WAFER_OK;
+}
+
+// host -> slot b -> s_main: n bytes of `src` are copied on the copy stream once the slot's last users are done with it
+// (nothing when n is 0), then use(slot) queues the kernels that read it; the slot is free again after them.
+template <class Use>
+int ring_in(wafer_ctx* ctx, int b, const void* src, size_t n, Use use) {
+    StagingRing& r = ctx->ring;
+    if (n) {
+        CK(cudaStreamWaitEvent(r.copy, r.free[b], 0));
+        CK(cudaMemcpyAsync(r.slot[b], src, n, cudaMemcpyHostToDevice, r.copy));
+        CK(cudaEventRecord(r.full[b], r.copy));
+        CK(cudaStreamWaitEvent(ctx->s_main, r.full[b], 0));
+    }
+    TRY(use(r.slot[b]));
+    CK(cudaEventRecord(r.free[b], ctx->s_main));
+    return WAFER_OK;
+}
+
+// s_main -> slot b -> host: make(slot) queues the kernels that fill the slot once its last copy has left it, then
+// n bytes of it go to `dst` on the copy stream; the slot is free again (and `dst` written) after that copy.
+template <class Make>
+int ring_out(wafer_ctx* ctx, int b, void* dst, size_t n, Make make) {
+    StagingRing& r = ctx->ring;
+    CK(cudaStreamWaitEvent(ctx->s_main, r.free[b], 0));
+    TRY(make(r.slot[b]));
+    CK(cudaEventRecord(r.full[b], ctx->s_main));
+    CK(cudaStreamWaitEvent(r.copy, r.full[b], 0));
+    CK(cudaMemcpyAsync(dst, r.slot[b], n, cudaMemcpyDeviceToHost, r.copy));
+    CK(cudaEventRecord(r.free[b], r.copy));
+    return WAFER_OK;
+}
+
+// the host waits until slot b is free: its ring_out copy has landed, or the kernels of its ring_in are done
+int ring_wait(wafer_ctx* ctx, int b) {
+    CK(cudaEventSynchronize(ctx->ring.free[b]));
+    return WAFER_OK;
+}
+
+// the host waits for the copy stream and s_main; sets no ctx->err, as DevBuf drains on the way out of failed calls
+cudaError_t ring_drain(wafer_ctx* ctx) {
+    const cudaError_t e = cudaStreamSynchronize(ctx->ring.copy), m = cudaStreamSynchronize(ctx->s_main);
+    return e != cudaSuccess ? e : m;
 }
 
 // host -> device.  `host` points at plane `host_p0` of the reference array; planes [hp0, hp1) of it are read.
@@ -1100,27 +1180,22 @@ int upload(wafer_ctx* ctx, const double* host, long long host_p0, long long hp0,
     const Geom& g = ctx->g;
     const long long py = worksized ? g.ny : g.ny + 2 * g.e, pz = worksized ? g.nz : g.nz + 2 * g.e;
     const int hoff = worksized ? 0 : g.e;
-    TRY(ensure_staging(ctx));
+    TRY(ring_reserve(ctx, 0, false));
+    const long long planes = ring_planes(ctx);
     if (check_ring) CK(cudaMemsetAsync(ctx->ring_flag, 0, sizeof(int), ctx->s_main));
-    CK(cudaEventRecord(ctx->ev_stg_free[0], ctx->s_main));  // everything queued so far precedes the first refill
-    CK(cudaEventRecord(ctx->ev_stg_free[1], ctx->s_main));
+    TRY(ring_start(ctx));
     int k = 0;
-    for (int i0 = -g.gx; i0 < g.L + g.gx; i0 += (int)ctx->stg_planes, ++k) {
-        const int i1 = (int)std::min<long long>(i0 + ctx->stg_planes, g.L + g.gx), b = k & 1;
+    for (int i0 = -g.gx; i0 < g.L + g.gx; i0 += (int)planes, ++k) {
+        const int i1 = (int)std::min<long long>(i0 + planes, g.L + g.gx);
         // host planes behind device planes [i0, i1), clipped to what the caller handed over
         const long long sp0 = std::max<long long>(hp0, g.x0 + i0 + hoff), sp1 = std::min<long long>(hp1, g.x0 + i1 + hoff);
-        if (sp1 > sp0) {
-            CK(cudaStreamWaitEvent(ctx->s_copy, ctx->ev_stg_free[b], 0));
-            CK(cudaMemcpyAsync(ctx->stg[b], host + (sp0 - host_p0) * py * pz, (size_t)((sp1 - sp0) * py * pz) * sizeof(double),
-                               cudaMemcpyHostToDevice, ctx->s_copy));
-            CK(cudaEventRecord(ctx->ev_stg_full[b], ctx->s_copy));
-            CK(cudaStreamWaitEvent(ctx->s_main, ctx->ev_stg_full[b], 0));
-        }
-        const int grid = (int)std::min<long long>((long long)(i1 - i0) * g.yp, (long long)ctx->sm_count * 16);
-        if (check_ring) unpack_kernel<true><<<grid, 256, 0, ctx->s_main>>>(ctx->stg[b], dst, g, i0, i1, sp0, std::max(sp0, sp1), worksized ? 1 : 0, ctx->ring_flag);
-        else unpack_kernel<false><<<grid, 256, 0, ctx->s_main>>>(ctx->stg[b], dst, g, i0, i1, sp0, std::max(sp0, sp1), worksized ? 1 : 0, ctx->ring_flag);
-        TRY(post_launch(ctx));
-        CK(cudaEventRecord(ctx->ev_stg_free[b], ctx->s_main));
+        const size_t n = sp1 > sp0 ? (size_t)((sp1 - sp0) * py * pz) * sizeof(double) : 0;
+        TRY(ring_in(ctx, k & 1, host + (sp0 - host_p0) * py * pz, n, [&](void* slot) -> int {
+            const int grid = (int)std::min<long long>((long long)(i1 - i0) * g.yp, (long long)ctx->sm_count * 16);
+            if (check_ring) unpack_kernel<true><<<grid, 256, 0, ctx->s_main>>>((const double*)slot, dst, g, i0, i1, sp0, std::max(sp0, sp1), worksized ? 1 : 0, ctx->ring_flag);
+            else unpack_kernel<false><<<grid, 256, 0, ctx->s_main>>>((const double*)slot, dst, g, i0, i1, sp0, std::max(sp0, sp1), worksized ? 1 : 0, ctx->ring_flag);
+            return post_launch(ctx);
+        }));
     }
     if (check_ring) {
         int flag = 0;
@@ -1140,25 +1215,19 @@ int upload(wafer_ctx* ctx, const double* host, long long host_p0, long long hp0,
 int download(wafer_ctx* ctx, const double* src, double* host, long long host_p0, long long hp0, long long hp1) {
     const Geom& g = ctx->g;
     const long long py = g.ny + 2 * g.e, pz = g.nz + 2 * g.e;
-    TRY(ensure_staging(ctx));
-    CK(cudaEventRecord(ctx->ev_stg_free[0], ctx->s_main));
-    CK(cudaEventRecord(ctx->ev_stg_free[1], ctx->s_main));
+    TRY(ring_reserve(ctx, 0, false));
+    const long long planes = ring_planes(ctx);
+    TRY(ring_start(ctx));
     int k = 0;
-    for (long long sp0 = hp0; sp0 < hp1; sp0 += ctx->stg_planes, ++k) {
-        const long long sp1 = std::min(hp1, sp0 + ctx->stg_planes);
-        const int b = k & 1;
-        CK(cudaStreamWaitEvent(ctx->s_main, ctx->ev_stg_free[b], 0));
-        const int grid = (int)std::min<long long>((sp1 - sp0) * py, (long long)ctx->sm_count * 16);
-        pack_kernel<<<grid, 256, 0, ctx->s_main>>>(src, ctx->stg[b], g, sp0, sp1, 0);
-        TRY(post_launch(ctx));
-        CK(cudaEventRecord(ctx->ev_stg_full[b], ctx->s_main));
-        CK(cudaStreamWaitEvent(ctx->s_copy, ctx->ev_stg_full[b], 0));
-        CK(cudaMemcpyAsync(host + (sp0 - host_p0) * py * pz, ctx->stg[b], (size_t)((sp1 - sp0) * py * pz) * sizeof(double),
-                           cudaMemcpyDeviceToHost, ctx->s_copy));
-        CK(cudaEventRecord(ctx->ev_stg_free[b], ctx->s_copy));
+    for (long long sp0 = hp0; sp0 < hp1; sp0 += planes, ++k) {
+        const long long sp1 = std::min(hp1, sp0 + planes);
+        TRY(ring_out(ctx, k & 1, host + (sp0 - host_p0) * py * pz, (size_t)((sp1 - sp0) * py * pz) * sizeof(double), [&](void* slot) -> int {
+            const int grid = (int)std::min<long long>((sp1 - sp0) * py, (long long)ctx->sm_count * 16);
+            pack_kernel<<<grid, 256, 0, ctx->s_main>>>(src, (double*)slot, g, sp0, sp1, 0);
+            return post_launch(ctx);
+        }));
     }
-    CK(cudaStreamSynchronize(ctx->s_copy));
-    CK(cudaStreamSynchronize(ctx->s_main));
+    CK(ring_drain(ctx));
     return WAFER_OK;
 }
 
@@ -1190,9 +1259,9 @@ int ensure_ab(wafer_ctx* ctx) {
 }
 
 // fill_data / read_csv on the device (resample.cuh) into the work area of `dst`: only the source x-planes this rank's
-// planes need are copied, run by run, through two device staging buffers (the bounce buffers when two source planes
-// fit one, else two of at most 128 MB); the copy of one run overlaps the kernel of the other.  Synchronises.
-constexpr long long RS_MAX_STG = (128ll << 20) / (long long)sizeof(double);  // doubles in one 128 MB staging buffer
+// planes need are copied, run by run, through the staging ring (grown, to at most 128 MB a slot, when two source planes
+// do not fit the padded planes a slot carries); the copy of one run overlaps the kernel of the other.  Synchronises.
+constexpr long long RS_MAX_STG = RING_MAX / (long long)sizeof(double);  // doubles in one 128 MB slot
 
 bool resample_copies(const wafer_ctx* ctx, uint64_t sx, uint64_t sy, uint64_t sz, uint32_t from_csv) {
     return from_csv && sx == (uint64_t)ctx->g.gnx && sy == (uint64_t)ctx->g.gny && sz == (uint64_t)ctx->g.gnz;
@@ -1252,44 +1321,23 @@ void rs_launch(wafer_ctx* ctx, const RsPlan& pl, double* dst, const double* src,
 
 // the arguments passed resample_args
 int resample_into(wafer_ctx* ctx, const RsPlan& pl, const double* src, uint64_t sx, uint64_t sy, uint64_t sz, double* dst) {
-    const Geom& g = ctx->g;
     const long long splane = (long long)(sy * sz), need = pl.copy ? 1 : 2;
     auto lo = [&](long long gi) { return rs_lo(ctx, pl, sx, gi); };
     const long long ga = pl.ga, gb = pl.gb;
-    TRY(ensure_staging(ctx));
-    double* buf[2] = {ctx->stg[0], ctx->stg[1]};
-    long long cap = ctx->stg_planes * (long long)(g.ny + 2 * g.e) * (g.nz + 2 * g.e) / splane;  // source planes per buffer
-    if (cap < need) {
-        cap = std::min<long long>(RS_MAX_STG / splane, pl.sp1 - pl.sp0);
-        if (ctx->rs_cap < cap * splane) {  // the last call that used them synchronised before returning
-            for (int b = 0; b < 2; ++b) {
-                cudaFree(ctx->rs_stg[b]);
-                ctx->rs_stg[b] = nullptr;
-            }
-            ctx->rs_cap = 0;
-            for (int b = 0; b < 2; ++b) CK(cudaMalloc(&ctx->rs_stg[b], (size_t)(cap * splane) * sizeof(double)));
-            ctx->rs_cap = cap * splane;
-        }
-        buf[0] = ctx->rs_stg[0];
-        buf[1] = ctx->rs_stg[1];
-    }
-    CK(cudaEventRecord(ctx->ev_stg_free[0], ctx->s_main));  // everything queued so far precedes the first refill
-    CK(cudaEventRecord(ctx->ev_stg_free[1], ctx->s_main));
+    long long cap = ring_planes(ctx) * host_plane(ctx->g) / splane;  // source planes per run
+    if (cap < need) cap = std::min<long long>(RS_MAX_STG / splane, pl.sp1 - pl.sp0);
+    TRY(ring_reserve(ctx, (size_t)(cap * splane) * sizeof(double), false));
+    TRY(ring_start(ctx));
     int k = 0;
     for (long long a = ga; a < gb; ++k) {
         const long long s0 = lo(a);
         long long b = a + 1;
         while (b < gb && lo(b) + need - s0 <= cap) ++b;  // lo() is non-decreasing: the run's planes are [s0, lo(b-1)+need)
         const long long s1 = lo(b - 1) + need;
-        const int nb = k & 1;
-        CK(cudaStreamWaitEvent(ctx->s_copy, ctx->ev_stg_free[nb], 0));
-        CK(cudaMemcpyAsync(buf[nb], src + s0 * splane, (size_t)((s1 - s0) * splane) * sizeof(double), cudaMemcpyHostToDevice,
-                           ctx->s_copy));
-        CK(cudaEventRecord(ctx->ev_stg_full[nb], ctx->s_copy));
-        CK(cudaStreamWaitEvent(ctx->s_main, ctx->ev_stg_full[nb], 0));
-        rs_launch(ctx, pl, dst, buf[nb], s0, sx, sy, sz, a, b);
-        TRY(post_launch(ctx));
-        CK(cudaEventRecord(ctx->ev_stg_free[nb], ctx->s_main));
+        TRY(ring_in(ctx, k & 1, src + s0 * splane, (size_t)((s1 - s0) * splane) * sizeof(double), [&](void* slot) -> int {
+            rs_launch(ctx, pl, dst, (const double*)slot, s0, sx, sy, sz, a, b);
+            return post_launch(ctx);
+        }));
         a = b;
     }
     CK(cudaStreamSynchronize(ctx->s_main));  // the caller may free `src` on return
@@ -1298,8 +1346,8 @@ int resample_into(wafer_ctx* ctx, const RsPlan& pl, const double* src, uint64_t 
 
 enum { RS_PHI = 0, RS_POTENTIAL, RS_LOWER };
 
-// the effects of wafer_set_phi (which = RS_PHI), wafer_set_potential or wafer_push_lower, with fill(dst) writing the
-// work area of the field
+// what setting psi (which = RS_PHI), V (RS_POTENTIAL) or a new lower state (RS_LOWER) changes, for every entry that
+// sets one; fill(dst) writes the work area of the field (an upload, a generator, a resample)
 template <class Fill>
 int set_input(wafer_ctx* ctx, int which, Fill fill) {
     if (which == RS_PHI) {  // the ring is +0 by construction
@@ -1455,17 +1503,10 @@ int wafer_destroy(wafer_ctx* ctx) {
     for (double* q : ctx->lowers) cudaFree(q);
     cudaFree(ctx->hfield);
     cudaFree(ctx->psi[0]); cudaFree(ctx->psi[1]); cudaFree(ctx->v); cudaFree(ctx->a); cudaFree(ctx->b);
-    for (int b = 0; b < 2; ++b) {
-        cudaFree(ctx->stg[b]);
-        cudaFree(ctx->rs_stg[b]);
-        if (ctx->ev_stg_free[b]) cudaEventDestroy(ctx->ev_stg_free[b]);
-        if (ctx->ev_stg_full[b]) cudaEventDestroy(ctx->ev_stg_full[b]);
-    }
-    if (ctx->s_copy) cudaStreamDestroy(ctx->s_copy);
-    for (int b = 0; b < 2; ++b)
-        if (ctx->wr_host[b]) cudaFreeHost(ctx->wr_host[b]);
+    ring_free(ctx->ring, true);
+    cudaFree(ctx->pow10);
     cudaFree(ctx->wr_btot); cudaFree(ctx->wr_boff); cudaFree(ctx->wr_flags); cudaFree(ctx->wr_txt); cudaFree(ctx->wr_count);
-    cudaFree(ctx->wr_red); cudaFree(ctx->wr_pow10);
+    cudaFree(ctx->wr_red);
     for (int b = 0; b < 2; ++b) {
         cudaFree(ctx->rd_bcount[b]); cudaFree(ctx->rd_boff[b]); cudaFree(ctx->rd_flags[b]);
     }
@@ -1539,14 +1580,9 @@ int wafer_slab(const wafer_ctx* ctx, uint64_t* x0, uint64_t* x1) {
 // ---- state in / out ------------------------------------------------------------------------------------------
 int wafer_set_potential(wafer_ctx* ctx, const double* v_padded) {
     if (!ctx) return WAFER_ERR_INVALID;
-    ctx->chk_valid = false;  // psi (or what the check sums depend on) changes
     REQUIRE(v_padded, "v_padded is NULL");
     CK(cudaSetDevice(ctx->dev));
-    ctx->h_valid = false;
-    TRY(upload_global(ctx, v_padded, ctx->v, false, false));
-    TRY(ensure_ab(ctx));
-    ctx->have_v = true;
-    return WAFER_OK;
+    return set_input(ctx, RS_POTENTIAL, [&](double* dst) { return upload_global(ctx, v_padded, dst, false, false); });
 }
 
 int wafer_get_potential(wafer_ctx* ctx, double* v_padded) {
@@ -1579,12 +1615,9 @@ int wafer_set_pot_sub_array(wafer_ctx* ctx, const double* work) {
 
 int wafer_set_phi(wafer_ctx* ctx, const double* phi_padded) {
     if (!ctx) return WAFER_ERR_INVALID;
-    ctx->chk_valid = false;  // psi (or what the check sums depend on) changes
     REQUIRE(phi_padded, "phi_padded is NULL");
     CK(cudaSetDevice(ctx->dev));
-    const int rc = upload_global(ctx, phi_padded, ctx->psi[ctx->cur], false, true);
-    ctx->have_phi = rc == WAFER_OK;
-    return rc;
+    return set_input(ctx, RS_PHI, [&](double* dst) { return upload_global(ctx, phi_padded, dst, false, true); });
 }
 
 int wafer_get_phi(wafer_ctx* ctx, double* phi_padded) {
@@ -1607,26 +1640,20 @@ int wafer_slab_planes(const wafer_ctx* ctx, int32_t which, uint64_t* p0, uint64_
 
 int wafer_set_phi_slab(wafer_ctx* ctx, const double* chunk) {
     if (!ctx) return WAFER_ERR_INVALID;
-    ctx->chk_valid = false;  // psi (or what the check sums depend on) changes
     REQUIRE(chunk, "chunk is NULL");
     CK(cudaSetDevice(ctx->dev));
     long long hp0, hp1;
     chunk_range(ctx, false, &hp0, &hp1);
-    const int rc = upload(ctx, chunk, hp0, hp0, hp1, ctx->psi[ctx->cur], false, true);
-    ctx->have_phi = rc == WAFER_OK;
-    return rc;
+    return set_input(ctx, RS_PHI, [&](double* dst) { return upload(ctx, chunk, hp0, hp0, hp1, dst, false, true); });
 }
 
 int wafer_set_phi_owned(wafer_ctx* ctx, const double* chunk) {
     if (!ctx) return WAFER_ERR_INVALID;
-    ctx->chk_valid = false;  // psi (or what the check sums depend on) changes
     REQUIRE(chunk, "chunk is NULL");
     CK(cudaSetDevice(ctx->dev));
     long long hp0, hp1;
     owned_range(ctx, &hp0, &hp1);
-    const int rc = upload(ctx, chunk, hp0, hp0, hp1, ctx->psi[ctx->cur], false, true);
-    ctx->have_phi = rc == WAFER_OK;
-    if (rc != WAFER_OK) return rc;
+    TRY(set_input(ctx, RS_PHI, [&](double* dst) { return upload(ctx, chunk, hp0, hp0, hp1, dst, false, true); }));
     return exchange(ctx, ctx->psi[ctx->cur], ctx->s_main);  // ghost planes come from the neighbours (collective)
 }
 
@@ -1643,14 +1670,8 @@ int wafer_get_phi_slab(wafer_ctx* ctx, double* chunk) {
 static int wafer_push_lower_impl(wafer_ctx* ctx, const double* q_padded) {
     if (!ctx) return WAFER_ERR_INVALID;
     REQUIRE(q_padded, "q_padded is NULL");
-    REQUIRE(ctx->lowers.size() < 255, "at most 255 lower states (wavenum is a u8, config.rs:308)");
     CK(cudaSetDevice(ctx->dev));
-    double* q = nullptr;
-    TRY(alloc_field(ctx, &q));
-    int rc = upload_global(ctx, q_padded, q, false, true);
-    if (rc == WAFER_OK) rc = register_lower(ctx, q);
-    if (rc != WAFER_OK) cudaFree(q);
-    return rc;
+    return set_input(ctx, RS_LOWER, [&](double* dst) { return upload_global(ctx, q_padded, dst, false, true); });
 }
 
 static int wafer_push_lower_from_phi_impl(wafer_ctx* ctx) {
@@ -1710,17 +1731,14 @@ uint32_t wafer_num_lowers(const wafer_ctx* ctx) { return ctx ? (uint32_t)ctx->lo
 
 int wafer_generate_potential(wafer_ctx* ctx, int32_t kind, double sig) {
     if (!ctx) return WAFER_ERR_INVALID;
-    ctx->chk_valid = false;  // psi (or what the check sums depend on) changes
     CK(cudaSetDevice(ctx->dev));
     GenParams gp = make_gen_params(ctx->p.dn, ctx->p.mass, sig);
     REQUIRE(potential_kind_supported(kind), "PotentialNotAvailable: no formula for this potential kind (potential.rs:315-317)");
     const long long rows = (long long)(ctx->g.L + 2 * ctx->g.gx) * ctx->g.ny;
-    ctx->h_valid = false;
-    gen_potential_kernel<<<(int)std::min<long long>(rows, (long long)ctx->sm_count * 32), 128, 0, ctx->s_main>>>(ctx->v, ctx->g, kind, gp);
-    TRY(post_launch(ctx));
-    TRY(ensure_ab(ctx));
-    ctx->have_v = true;
-    return WAFER_OK;
+    return set_input(ctx, RS_POTENTIAL, [&](double* dst) {
+        gen_potential_kernel<<<(int)std::min<long long>(rows, (long long)ctx->sm_count * 32), 128, 0, ctx->s_main>>>(dst, ctx->g, kind, gp);
+        return post_launch(ctx);
+    });
 }
 
 int wafer_generate_initial_condition(wafer_ctx* ctx, int32_t kind) {
@@ -1814,24 +1832,29 @@ static int ready(wafer_ctx* ctx, bool need_v) {
 // Two passes over this rank's work sites.  Pass 1 measures: block totals of the certified sites, the refused sites
 // formatted on the host (their lengths added), an exclusive scan into block offsets.  The ranks then exchange their
 // byte counts in one all-reduce, so each knows where its planes start in the file.  Pass 2 encodes chunk after
-// chunk into a bounce buffer (as many whole blocks as fit), copies it to a pinned host buffer on s_copy and writes it
-// with pwrite while the next chunk is encoded.  Refused sites are collected again per piece of a chunk (a run of
+// chunk into a slot of the staging ring (as many whole blocks as fit), copies it to the slot's pinned half and writes
+// it with pwrite while the next chunk is encoded.  Refused sites are collected again per piece of a chunk (a run of
 // blocks with at most ENC_FLAG_CAP of them) rather than kept from pass 1: host memory stays bounded whatever the field.
-static constexpr size_t WR_MIN_STG = 2 * (size_t)ENC_BS * enc::SITE_MAX;  // two blocks of the longest Csv rows
+// the ring's slots for the array files, written or read: at least two blocks of the longest Csv rows
+static constexpr size_t FILE_MIN_STG = 2 * (size_t)ENC_BS * enc::SITE_MAX;
+
+// the 128-bit power table of encode.cuh / decode.cuh
+static int pow10_table(wafer_ctx* ctx) {
+    if (ctx->pow10) return WAFER_OK;
+    EncTable h;
+    const enc::Pow10 t = enc::host_pow10();
+    memcpy(h.hilo, t.hilo, sizeof h.hilo);
+    memcpy(h.shift, t.shift, sizeof h.shift);
+    EncTable* p = nullptr;
+    CK(cudaMalloc(&p, sizeof(EncTable)));
+    CK(cudaMemcpy(p, &h, sizeof(EncTable), cudaMemcpyHostToDevice));
+    ctx->pow10 = p;
+    return WAFER_OK;
+}
 
 static int wr_buffers(wafer_ctx* ctx, long long nblocks) {
-    TRY(ensure_staging(ctx));
-    if (ctx->stg_bytes < WR_MIN_STG) {  // a small lattice's bounce buffers; upload / download use stg_planes of them
-        for (int b = 0; b < 2; ++b) {
-            double* p = nullptr;
-            CK(cudaMalloc(&p, WR_MIN_STG));
-            cudaFree(ctx->stg[b]);
-            ctx->stg[b] = p;
-        }
-        ctx->stg_bytes = WR_MIN_STG;
-    }
-    for (int b = 0; b < 2; ++b)
-        if (!ctx->wr_host[b]) CK(cudaMallocHost(&ctx->wr_host[b], ctx->stg_bytes));
+    TRY(ring_reserve(ctx, FILE_MIN_STG, true));
+    TRY(pow10_table(ctx));
     if (ctx->wr_blocks < nblocks) {
         cudaFree(ctx->wr_btot);
         cudaFree(ctx->wr_boff);
@@ -1843,12 +1866,6 @@ static int wr_buffers(wafer_ctx* ctx, long long nblocks) {
         ctx->wr_blocks = nblocks;
     }
     if (!ctx->wr_count) {
-        EncTable h;
-        const enc::Pow10 t = enc::host_pow10();
-        memcpy(h.hilo, t.hilo, sizeof h.hilo);
-        memcpy(h.shift, t.shift, sizeof h.shift);
-        CK(cudaMalloc(&ctx->wr_pow10, sizeof(EncTable)));
-        CK(cudaMemcpy(ctx->wr_pow10, &h, sizeof(EncTable), cudaMemcpyHostToDevice));
         CK(cudaMalloc(&ctx->wr_flags, ENC_FLAG_CAP * sizeof(EncFlagIn)));
         CK(cudaMalloc(&ctx->wr_txt, ENC_FLAG_CAP * sizeof(EncFlagStr)));
         CK(cudaMalloc(&ctx->wr_count, 2 * sizeof(unsigned long long)));
@@ -1883,9 +1900,9 @@ static int wr_collect(wafer_ctx* ctx, const WrJob& job, long long b0, long long 
     CK(cudaMemsetAsync(ctx->wr_count, 0, sizeof(unsigned long long), ctx->s_main));
     const unsigned grid = (unsigned)(b1 - b0);
     if (job.fmt == enc::FMT_CSV)
-        encode_len_kernel<enc::FMT_CSV><<<grid, ENC_THREADS, 0, ctx->s_main>>>(job.f, g, b0, job.nsites, ctx->wr_pow10, ctx->wr_btot, ctx->wr_flags, ctx->wr_count);
+        encode_len_kernel<enc::FMT_CSV><<<grid, ENC_THREADS, 0, ctx->s_main>>>(job.f, g, b0, job.nsites, ctx->pow10, ctx->wr_btot, ctx->wr_flags, ctx->wr_count);
     else
-        encode_len_kernel<enc::FMT_JSON><<<grid, ENC_THREADS, 0, ctx->s_main>>>(job.f, g, b0, job.nsites, ctx->wr_pow10, ctx->wr_btot, ctx->wr_flags, ctx->wr_count);
+        encode_len_kernel<enc::FMT_JSON><<<grid, ENC_THREADS, 0, ctx->s_main>>>(job.f, g, b0, job.nsites, ctx->pow10, ctx->wr_btot, ctx->wr_flags, ctx->wr_count);
     TRY(post_launch(ctx));
     CK(cudaMemcpyAsync(n, ctx->wr_count, sizeof(unsigned long long), cudaMemcpyDeviceToHost, ctx->s_main));
     if (bt) {
@@ -1964,54 +1981,52 @@ static int wr_emit(wafer_ctx* ctx, const WrJob& job, const std::vector<unsigned 
                    unsigned long long data_off, bool* ok, std::string* io_err) {
     const Geom& g = ctx->g;
     CK(cudaMemsetAsync(ctx->wr_count + 1, 0, sizeof(unsigned long long), ctx->s_main));
-    CK(cudaEventRecord(ctx->ev_stg_free[0], ctx->s_main));
-    CK(cudaEventRecord(ctx->ev_stg_free[1], ctx->s_main));
+    const size_t cap = ctx->ring.bytes;
+    TRY(ring_start(ctx));
     unsigned long long pend_bytes = 0, pend_off = 0;
     int k = 0;
     for (long long cb = 0; cb < job.nblocks; ++k) {
         long long ce = cb + 1;
-        while (ce < job.nblocks && boff[ce + 1] - boff[cb] <= ctx->stg_bytes) ++ce;
+        while (ce < job.nblocks && boff[ce + 1] - boff[cb] <= cap) ++ce;
         const int buf = k & 1;
-        unsigned char* out = (unsigned char*)ctx->stg[buf];
-        CK(cudaStreamWaitEvent(ctx->s_main, ctx->ev_stg_free[buf], 0));  // the copy of chunk k - 2 has left it
-        for (long long pb = cb; pb < ce;) {
-            long long pe = pb;
-            unsigned long long nf = 0;
-            while (pe < ce && nf + job.bflag[pe] <= ENC_FLAG_CAP) nf += job.bflag[pe++];
-            int ntxt = 0;
-            if (nf > 0) {
-                std::vector<EncFlagStr> txt;
-                unsigned long long n = 0;
-                TRY(wr_collect(ctx, job, pb, pe, &txt, &n, nullptr));
-                if (n != nf) { ctx->err = "wafer_write_array: the refused sites differ between the passes"; return WAFER_ERR_CUDA; }
-                CK(cudaMemcpyAsync(ctx->wr_txt, txt.data(), txt.size() * sizeof(EncFlagStr), cudaMemcpyHostToDevice, ctx->s_main));
-                CK(cudaStreamSynchronize(ctx->s_main));
-                ntxt = (int)n;
-            }
-            const unsigned grid = (unsigned)(pe - pb);
-            switch (job.fmt) {
-                case enc::FMT_MPK: encode_emit_kernel<enc::FMT_MPK><<<grid, ENC_THREADS, 0, ctx->s_main>>>(job.f, g, pb, job.nsites, ctx->wr_pow10, ctx->wr_boff, boff[cb], ctx->wr_txt, ntxt, out, ctx->wr_count + 1); break;
-                case enc::FMT_CSV: encode_emit_kernel<enc::FMT_CSV><<<grid, ENC_THREADS, 0, ctx->s_main>>>(job.f, g, pb, job.nsites, ctx->wr_pow10, ctx->wr_boff, boff[cb], ctx->wr_txt, ntxt, out, ctx->wr_count + 1); break;
-                default: encode_emit_kernel<enc::FMT_JSON><<<grid, ENC_THREADS, 0, ctx->s_main>>>(job.f, g, pb, job.nsites, ctx->wr_pow10, ctx->wr_boff, boff[cb], ctx->wr_txt, ntxt, out, ctx->wr_count + 1); break;
-            }
-            TRY(post_launch(ctx));
-            pb = pe;
-        }
         const unsigned long long bytes = boff[ce] - boff[cb];
-        CK(cudaEventRecord(ctx->ev_stg_full[buf], ctx->s_main));
-        CK(cudaStreamWaitEvent(ctx->s_copy, ctx->ev_stg_full[buf], 0));
-        CK(cudaMemcpyAsync(ctx->wr_host[buf], out, bytes, cudaMemcpyDeviceToHost, ctx->s_copy));
-        CK(cudaEventRecord(ctx->ev_stg_free[buf], ctx->s_copy));
+        TRY(ring_out(ctx, buf, ctx->ring.host[buf], bytes, [&](void* slot) -> int {
+            unsigned char* out = (unsigned char*)slot;
+            for (long long pb = cb; pb < ce;) {
+                long long pe = pb;
+                unsigned long long nf = 0;
+                while (pe < ce && nf + job.bflag[pe] <= ENC_FLAG_CAP) nf += job.bflag[pe++];
+                int ntxt = 0;
+                if (nf > 0) {
+                    std::vector<EncFlagStr> txt;
+                    unsigned long long n = 0;
+                    TRY(wr_collect(ctx, job, pb, pe, &txt, &n, nullptr));
+                    if (n != nf) { ctx->err = "wafer_write_array: the refused sites differ between the passes"; return WAFER_ERR_CUDA; }
+                    CK(cudaMemcpyAsync(ctx->wr_txt, txt.data(), txt.size() * sizeof(EncFlagStr), cudaMemcpyHostToDevice, ctx->s_main));
+                    CK(cudaStreamSynchronize(ctx->s_main));
+                    ntxt = (int)n;
+                }
+                const unsigned grid = (unsigned)(pe - pb);
+                switch (job.fmt) {
+                    case enc::FMT_MPK: encode_emit_kernel<enc::FMT_MPK><<<grid, ENC_THREADS, 0, ctx->s_main>>>(job.f, g, pb, job.nsites, ctx->pow10, ctx->wr_boff, boff[cb], ctx->wr_txt, ntxt, out, ctx->wr_count + 1); break;
+                    case enc::FMT_CSV: encode_emit_kernel<enc::FMT_CSV><<<grid, ENC_THREADS, 0, ctx->s_main>>>(job.f, g, pb, job.nsites, ctx->pow10, ctx->wr_boff, boff[cb], ctx->wr_txt, ntxt, out, ctx->wr_count + 1); break;
+                    default: encode_emit_kernel<enc::FMT_JSON><<<grid, ENC_THREADS, 0, ctx->s_main>>>(job.f, g, pb, job.nsites, ctx->pow10, ctx->wr_boff, boff[cb], ctx->wr_txt, ntxt, out, ctx->wr_count + 1); break;
+                }
+                TRY(post_launch(ctx));
+                pb = pe;
+            }
+            return WAFER_OK;
+        }));
         if (k > 0) {  // chunk k - 1 is written while chunk k is encoded and copied
-            CK(cudaEventSynchronize(ctx->ev_stg_free[buf ^ 1]));
-            if (*ok) *ok = wr_pwrite(fd, ctx->wr_host[buf ^ 1], pend_bytes, data_off + pend_off, io_err);
+            TRY(ring_wait(ctx, buf ^ 1));
+            if (*ok) *ok = wr_pwrite(fd, ctx->ring.host[buf ^ 1], pend_bytes, data_off + pend_off, io_err);
         }
         pend_bytes = bytes;
         pend_off = boff[cb];
         cb = ce;
     }
-    CK(cudaEventSynchronize(ctx->ev_stg_free[(k - 1) & 1]));
-    if (*ok) *ok = wr_pwrite(fd, ctx->wr_host[(k - 1) & 1], pend_bytes, data_off + pend_off, io_err);
+    TRY(ring_wait(ctx, (k - 1) & 1));
+    if (*ok) *ok = wr_pwrite(fd, ctx->ring.host[(k - 1) & 1], pend_bytes, data_off + pend_off, io_err);
     unsigned long long missing = 0;
     CK(cudaMemcpyAsync(&missing, ctx->wr_count + 1, sizeof(missing), cudaMemcpyDeviceToHost, ctx->s_main));
     CK(cudaStreamSynchronize(ctx->s_main));
@@ -2126,14 +2141,15 @@ int wafer_write_array(wafer_ctx* ctx, int32_t what, int32_t file_type, const cha
 // ---- array files decoded on the device (decode.cuh) -----------------------------------------------------------
 // The preamble (and Json's trailer, a Csv file's last record) is read on the host; the shape rules give the source
 // planes this rank needs, converted into one device buffer.  The body is then read with pread into the two pinned
-// buffers, chunk after chunk; each goes to the device through a bounce buffer on s_copy and is decoded on s_main
+// halves of the staging ring, chunk after chunk; each goes to the device through its slot and is decoded on s_main
 // while the next one is read.  A chunk ends after its last separator, the rest is carried into the next.  Once a
 // chunk's kernels are done its uncertified numbers are converted with strtod from the pinned buffer it is still in.
 // The field changes only after the whole file has been read and found canonical: then resample_kernel reads the
 // buffer.
 static int dec_buffers(wafer_ctx* ctx) {
-    TRY(wr_buffers(ctx, 1));  // bounce buffers of at least two blocks of Csv rows, pinned host buffers, the power table
-    const long long nb = (long long)(ctx->stg_bytes / DEC_SEG) + 1;
+    TRY(ring_reserve(ctx, FILE_MIN_STG, true));
+    TRY(pow10_table(ctx));
+    const long long nb = (long long)(ctx->ring.bytes / DEC_SEG) + 1;
     if (ctx->rd_blocks < nb) {
         for (int b = 0; b < 2; ++b) {
             cudaFree(ctx->rd_bcount[b]);
@@ -2174,6 +2190,7 @@ static bool rd_pread(int fd, void* p, size_t n, unsigned long long off, std::str
 
 struct RdChunk {
     int buf;
+    const unsigned char* c;  // the slot it was copied to
     unsigned long long len;  // bytes of whole records
     long long nblocks;
 };
@@ -2186,12 +2203,11 @@ struct RdJob {
 
 static int rd_launch_text(wafer_ctx* ctx, const RdJob& job, const RdChunk& ch, long long b0, long long b1) {
     unsigned long long* st = ctx->rd_st + DEC_WORDS * ch.buf;
-    const unsigned char* c = (const unsigned char*)ctx->stg[ch.buf];
     CK(cudaMemsetAsync(st + DEC_NFLAG, 0, sizeof(unsigned long long), ctx->s_main));
     if (job.fmt == enc::FMT_CSV)
-        dec_text_kernel<enc::FMT_CSV><<<(unsigned)(b1 - b0), DEC_THREADS, 0, ctx->s_main>>>(c, ch.len, b0, ctx->rd_boff[ch.buf], ctx->wr_pow10, job.d, ctx->rd_flags[ch.buf], st);
+        dec_text_kernel<enc::FMT_CSV><<<(unsigned)(b1 - b0), DEC_THREADS, 0, ctx->s_main>>>(ch.c, ch.len, b0, ctx->rd_boff[ch.buf], ctx->pow10, job.d, ctx->rd_flags[ch.buf], st);
     else
-        dec_text_kernel<enc::FMT_JSON><<<(unsigned)(b1 - b0), DEC_THREADS, 0, ctx->s_main>>>(c, ch.len, b0, ctx->rd_boff[ch.buf], ctx->wr_pow10, job.d, ctx->rd_flags[ch.buf], st);
+        dec_text_kernel<enc::FMT_JSON><<<(unsigned)(b1 - b0), DEC_THREADS, 0, ctx->s_main>>>(ch.c, ch.len, b0, ctx->rd_boff[ch.buf], ctx->pow10, job.d, ctx->rd_flags[ch.buf], st);
     TRY(post_launch(ctx));
     CK(cudaMemcpyAsync(ctx->rd_hst + DEC_WORDS * ch.buf, st, DEC_WORDS * sizeof(unsigned long long), cudaMemcpyDeviceToHost,
                        ctx->s_main));
@@ -2216,7 +2232,7 @@ static int rd_host_convert(wafer_ctx* ctx, RdJob& job, const RdChunk& ch, long l
     std::vector<DecFlag> list(n);
     CK(cudaMemcpyAsync(list.data(), ctx->rd_flags[ch.buf], n * sizeof(DecFlag), cudaMemcpyDeviceToHost, ctx->s_main));
     CK(cudaStreamSynchronize(ctx->s_main));
-    const char* hb = (const char*)ctx->wr_host[ch.buf];
+    const char* hb = (const char*)ctx->ring.host[ch.buf];
     std::string tok;
     for (DecFlag& f : list) {
         if ((unsigned long long)f.at + f.len > ch.len) { ctx->err = "wafer_load_array: a listed number lies outside its chunk"; return WAFER_ERR_CUDA; }
@@ -2235,7 +2251,7 @@ static int rd_host_convert(wafer_ctx* ctx, RdJob& job, const RdChunk& ch, long l
 
 // a chunk whose kernels are queued: wait for them, then its status and its uncertified numbers
 static int rd_finish(wafer_ctx* ctx, RdJob& job, const RdChunk& ch) {
-    CK(cudaEventSynchronize(ctx->ev_stg_free[ch.buf]));
+    TRY(ring_wait(ctx, ch.buf));
     if (ctx->rd_hst[DEC_WORDS * ch.buf + DEC_ERR]) return WAFER_ERR_FORMAT;
     if (job.fmt == enc::FMT_MPK) return WAFER_OK;
     return rd_host_convert(ctx, job, ch, 0, ch.nblocks);
@@ -2244,17 +2260,16 @@ static int rd_finish(wafer_ctx* ctx, RdJob& job, const RdChunk& ch) {
 // bytes [b0, b1) of the file: every chunk decoded into job.d
 static int rd_stream(wafer_ctx* ctx, RdJob& job, int fd, unsigned long long b0, unsigned long long b1, std::string* io) {
     const unsigned char sep = job.fmt == enc::FMT_CSV ? '\n' : ',';
-    const unsigned long long cap = job.fmt == enc::FMT_MPK ? ctx->stg_bytes / 9 * 9 : ctx->stg_bytes;
+    const unsigned long long cap = job.fmt == enc::FMT_MPK ? ctx->ring.bytes / 9 * 9 : ctx->ring.bytes;
     unsigned long long off = b0, carry = 0;
-    RdChunk prev{0, 0, 0};
+    RdChunk prev{0, nullptr, 0, 0};
     CK(cudaMemsetAsync(ctx->rd_st, 0, (2 * DEC_WORDS + 1) * sizeof(unsigned long long), ctx->s_main));
-    CK(cudaEventRecord(ctx->ev_stg_free[0], ctx->s_main));
-    CK(cudaEventRecord(ctx->ev_stg_free[1], ctx->s_main));
+    TRY(ring_start(ctx));
     for (int k = 0; off < b1; ++k) {
         const int buf = k & 1;
-        unsigned char* hb = ctx->wr_host[buf];
+        unsigned char* hb = ctx->ring.host[buf];
         const unsigned long long e0 = (off - b0) / 9;  // Messagepack: the chunk's first element
-        if (carry) memcpy(hb, ctx->wr_host[buf ^ 1] + prev.len, carry);  // chunk k - 1's split record
+        if (carry) memcpy(hb, ctx->ring.host[buf ^ 1] + prev.len, carry);  // chunk k - 1's split record
         const unsigned long long n = std::min(cap - carry, b1 - off);
         if (!rd_pread(fd, hb + carry, n, off, io)) return WAFER_ERR_IO;
         off += n;
@@ -2263,32 +2278,29 @@ static int rd_stream(wafer_ctx* ctx, RdJob& job, int fd, unsigned long long b0, 
         if (off < b1 && job.fmt != enc::FMT_MPK) {  // end the chunk after its last separator
             unsigned long long cut = len;
             while (cut > 0 && hb[cut - 1] != sep) --cut;
-            if (cut == 0) return WAFER_ERR_FORMAT;  // a record longer than a bounce buffer
+            if (cut == 0) return WAFER_ERR_FORMAT;  // a record longer than a slot
             carry = len - cut;
             len = cut;
         }
-        RdChunk ch{buf, len, (long long)((len + DEC_SEG - 1) / DEC_SEG)};
-        unsigned char* db = (unsigned char*)ctx->stg[buf];
-        CK(cudaStreamWaitEvent(ctx->s_copy, ctx->ev_stg_free[buf], 0));  // chunk k - 2's kernels are done with it
-        CK(cudaMemcpyAsync(db, hb, len, cudaMemcpyHostToDevice, ctx->s_copy));
-        CK(cudaEventRecord(ctx->ev_stg_full[buf], ctx->s_copy));
-        CK(cudaStreamWaitEvent(ctx->s_main, ctx->ev_stg_full[buf], 0));
-        unsigned long long* st = ctx->rd_st + DEC_WORDS * buf;
-        if (job.fmt == enc::FMT_MPK) {
-            const unsigned long long nel = len / 9;
-            dec_mpk_kernel<<<(unsigned)std::min<unsigned long long>((nel + DEC_THREADS - 1) / DEC_THREADS, (unsigned long long)ctx->sm_count * 16),
-                             DEC_THREADS, 0, ctx->s_main>>>(db, nel, e0, job.d, st);
-            TRY(post_launch(ctx));
-            CK(cudaMemcpyAsync(ctx->rd_hst + DEC_WORDS * buf, st, DEC_WORDS * sizeof(unsigned long long), cudaMemcpyDeviceToHost,
-                               ctx->s_main));
-        } else {
-            dec_count_kernel<<<(unsigned)ch.nblocks, DEC_THREADS, 0, ctx->s_main>>>(db, len, sep, ctx->rd_bcount[buf]);
+        RdChunk ch{buf, nullptr, len, (long long)((len + DEC_SEG - 1) / DEC_SEG)};
+        TRY(ring_in(ctx, buf, hb, len, [&](void* slot) -> int {
+            ch.c = (const unsigned char*)slot;
+            unsigned long long* st = ctx->rd_st + DEC_WORDS * buf;
+            if (job.fmt == enc::FMT_MPK) {
+                const unsigned long long nel = len / 9;
+                dec_mpk_kernel<<<(unsigned)std::min<unsigned long long>((nel + DEC_THREADS - 1) / DEC_THREADS, (unsigned long long)ctx->sm_count * 16),
+                                 DEC_THREADS, 0, ctx->s_main>>>(ch.c, nel, e0, job.d, st);
+                TRY(post_launch(ctx));
+                CK(cudaMemcpyAsync(ctx->rd_hst + DEC_WORDS * buf, st, DEC_WORDS * sizeof(unsigned long long), cudaMemcpyDeviceToHost,
+                                   ctx->s_main));
+                return WAFER_OK;
+            }
+            dec_count_kernel<<<(unsigned)ch.nblocks, DEC_THREADS, 0, ctx->s_main>>>(ch.c, len, sep, ctx->rd_bcount[buf]);
             dec_offsets_kernel<<<1, 1024, 0, ctx->s_main>>>(ctx->rd_bcount[buf], (int)ch.nblocks, ctx->rd_boff[buf],
                                                             ctx->rd_st + 2 * DEC_WORDS);
             TRY(post_launch(ctx, 2));
-            TRY(rd_launch_text(ctx, job, ch, 0, ch.nblocks));
-        }
-        CK(cudaEventRecord(ctx->ev_stg_free[buf], ctx->s_main));
+            return rd_launch_text(ctx, job, ch, 0, ch.nblocks);
+        }));
         if (k > 0) TRY(rd_finish(ctx, job, prev));  // chunk k - 1, while chunk k is decoded
         prev = ch;
     }
@@ -2307,8 +2319,7 @@ struct DevBuf {  // the converted source planes; freed once the work queued on t
     wafer_ctx* ctx;
     double* p = nullptr;
     ~DevBuf() {
-        cudaStreamSynchronize(ctx->s_copy);
-        cudaStreamSynchronize(ctx->s_main);
+        ring_drain(ctx);
         cudaFree(p);
     }
 };
